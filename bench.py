@@ -2,7 +2,7 @@
 """Headline benchmark: randsvd (K=200, p=10, q=2) of a matrix-free covariance operator.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c5|c5s|small|dense]
-                    [--impl reference] [--generation table|arithmetic]
+                    [--impl reference] [--generation table|arithmetic] [--dump-outputs DIR]
 
 One "step" = one complete randsvd(A, K, p, q) of the workload (sketch GEMM, 2q power
 products with pivot-faithful LU normalisation, final Householder QR, projection, TSQR +
@@ -19,6 +19,10 @@ metric  = randsvd throughput in FP64 TFLOP/s, F = (2q+2)*2*n^2*(K+p) algorithmic
 value   : Omega already resident in HBM, Z left in HBM.
 e2e     : through the public API with HOST buffers -- Omega uploaded from pinned host
           memory and Z downloaded to pinned host memory inside the timed region.
+dump    : `--dump-outputs DIR` writes what the last timed step returned: DIR/S.npy (the l singular
+          values) and DIR/Z.npy (rows of Z, float64; all n rows when they fit in 64 MB, otherwise the
+          rows `dump_rows(n, l)` picks, a fixed seeded sample in ascending order).  Omega and the
+          operator are seeded, so two builds run with the same arguments can be compared file by file.
 parity  : BEFORE the timed region, at every N, the reduced workload (17 472-point Gaussian,
           same K, p, q; dense: n = 4096) is factored row-sharded over the N ranks; rank 0 compares
           it with the CPU oracle (singular values, subspace sine, exact-zero tail) after the ranks
@@ -85,6 +89,16 @@ CPU_SAMPLE = {"c3": (28, 26, 24), "small": (20, 18, 16), "c5": (132, 132), "c5s"
 # reduced workload of the pre-run parity check
 PARITY_GRID = {"c3": (28, 26, 24), "small": (20, 18, 16), "c5": (132, 132), "c5s": (132, 132), "dense": (64, 64)}
 KIND_ID = {"exponential": 0, "gaussian": 1, "powerlaw": 2}
+DUMP_BYTES = 64_000_000        # what --dump-outputs may write in all, .npy headers included
+
+
+def dump_rows(n, l):
+    """Row indices of Z that --dump-outputs writes: every row if Z and S fit in DUMP_BYTES, else a
+    sample drawn from a fixed seed, so that every run with the same n and l writes the same rows."""
+    k = min(n, (DUMP_BYTES - 8 * l - 4096) // (8 * l))
+    if k == n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
 
 
 def grid_coords(shape):
@@ -218,7 +232,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip extra.arith_tflops and (N = 8) extra.c5")
     ap.add_argument("--generation", default="table", choices=["table", "arithmetic"],
                     help="kernel values: lattice-table look-up (structured grid) or exp/sqrt arithmetic from coordinates")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write Z (rows, see dump_rows) and S of the last timed step as DIR/Z.npy, DIR/S.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -230,9 +248,11 @@ def main():
     if args.impl == "reference":
         # The reference (pure Julia) cannot run here: its CPU algorithm restated on
         # SciPy/OpenBLAS is timed on the host cores; rank 0 only, same thread count at every N.
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs the CUDA path (--impl gsi)")
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 3))
+        steps = args.steps
         cb = cpu_oracle_run(args.workload, steps, 1)
         print(json.dumps({
             "impl": "reference", "metric": "randsvd_fp64_tflops", "value": cb["value"], "unit": "TFLOP/s",
@@ -309,11 +329,14 @@ def main():
     Omega_d = gsi.DeviceMatrix.from_host(ctx, Omega_h)
     stream = torch.cuda.ExternalStream(ctx.stream(), device=torch.device("cuda", local_rank))
     sigma_head = []
+    last = {}                   # Z (on the device) and S of the latest step_resident, for --dump-outputs
 
     def step_resident():
+        if last:
+            last.pop("Z").free()        # back to the library's pool before this step allocates its Z
         Z, S = gsi.randsvd(op, K, p, q, Omega=Omega_d, device_out=True, return_singular_values=True)
         sigma_head[:] = [float(s) for s in S[:5]]
-        Z.free()
+        last.update(Z=Z, S=S)
 
     def step_e2e():
         Z = gsi.randsvd(op, K, p, q, Omega=Omega_h, device_out=True)     # uploads Omega from pinned host memory
@@ -352,6 +375,21 @@ def main():
     for _ in range(args.warmup):
         step_resident()
     ms, launches, gemm, clocks, phases = timed(step_resident, args.steps, True)
+    if args.dump_outputs:
+        # each rank holds the rows of its own block of Z (a dense operator's Z is replicated): gather the sample on rank 0
+        rows = dump_rows(n, l)
+        z0 = 0 if dense else row0
+        mine = rows[(rows >= z0) & (rows < z0 + zrows)]
+        Zs = last["Z"].numpy()[mine - z0]
+        if dist is not None and not dense:
+            parts = [None] * world if rank == 0 else None
+            dist.gather_object(Zs, parts, dst=0)
+            Zs = np.concatenate(parts) if rank == 0 else None
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "Z.npy"), Zs)
+            np.save(os.path.join(args.dump_outputs, "S.npy"), last["S"])
+    last.pop("Z").free()
     ms_per_step = ms / args.steps
     F = randsvd_flops(n, l, q)
     value = F / (ms_per_step * 1e-3) * 1e-12

@@ -8,7 +8,7 @@ CPU fallback: importing works anywhere, creating a Context needs a B200.
 from . import _lib
 from ._lib import (GsiError, SingularException, PosDefException, DimensionMismatch, NoDeviceError,
                    LAYOUT_TALL, LAYOUT_COLMAJOR, KERNEL_EXPONENTIAL, KERNEL_GAUSSIAN, KERNEL_POWERLAW,
-                   NORMALISER_LU_REF, NORMALISER_QR)
+                   KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SPHERICAL, NORMALISER_LU_REF, NORMALISER_QR)
 from .core import (Context, DeviceMatrix, DenseMatrix, LowRankCovMatrix, KernelCovMatrix, GridKernelCovMatrix, default_context,
                    set_default_context, as_operator, partition_rows)
 from . import randmatfact as RandMatFact

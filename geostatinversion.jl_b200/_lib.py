@@ -28,6 +28,9 @@ LAYOUT_COLMAJOR = 1
 KERNEL_EXPONENTIAL = 0
 KERNEL_GAUSSIAN = 1
 KERNEL_POWERLAW = 2
+KERNEL_MATERN32 = 3
+KERNEL_MATERN52 = 4
+KERNEL_SPHERICAL = 5
 NORMALISER_LU_REF = 0
 NORMALISER_QR = 1
 

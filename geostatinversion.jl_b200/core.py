@@ -8,11 +8,13 @@ import numpy as np
 
 from . import _lib
 from ._lib import (LAYOUT_TALL, LAYOUT_COLMAJOR, KERNEL_EXPONENTIAL, KERNEL_GAUSSIAN, KERNEL_POWERLAW,
-                   NORMALISER_LU_REF, NORMALISER_QR, check)
+                   KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SPHERICAL, NORMALISER_LU_REF, NORMALISER_QR, check)
 
 _KINDS = {"exponential": KERNEL_EXPONENTIAL, "gaussian": KERNEL_GAUSSIAN, "powerlaw": KERNEL_POWERLAW,
+          "matern32": KERNEL_MATERN32, "matern52": KERNEL_MATERN52, "spherical": KERNEL_SPHERICAL,
           KERNEL_EXPONENTIAL: KERNEL_EXPONENTIAL, KERNEL_GAUSSIAN: KERNEL_GAUSSIAN,
-          KERNEL_POWERLAW: KERNEL_POWERLAW}
+          KERNEL_POWERLAW: KERNEL_POWERLAW, KERNEL_MATERN32: KERNEL_MATERN32,
+          KERNEL_MATERN52: KERNEL_MATERN52, KERNEL_SPHERICAL: KERNEL_SPHERICAL}
 
 
 def _f64_colmajor(a):
@@ -358,6 +360,8 @@ class LowRankCovMatrix(_Operator):
 class KernelCovMatrix(_Operator):
     """Matrix-free covariance operator C[i,j] = sigma2*k(|(x_i-x_j)./ell|) + nugget*(i==j)
     (NEW operator type with LowRankCovMatrix's method set; SURVEY.md F4).
+    kind: "exponential", "gaussian", "powerlaw", "matern32", "matern52" or "spherical" (or its
+    KERNEL_* code; formulas in include/gsi_b200.h).
     coords: d x n (point j = coords[:, j]).  On a multi-rank context this rank applies
     rows [row0, row0+mloc)."""
     symmetric = True

@@ -509,7 +509,8 @@ GSI_API int32_t gsi_op_kernelcov(gsi_ctx* ctx, int32_t kind, int32_t d, int64_t 
         use(ctx);
         GSI_REQUIRE(coords && ell && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
         GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov: d must be 1, 2 or 3");
-        GSI_REQUIRE(kind >= 0 && kind <= 2, GSI_ERR_INVALID_ARGUMENT, "kernelcov: unknown kernel kind");
+        GSI_REQUIRE(kind >= GSI_KERNEL_EXPONENTIAL && kind <= GSI_KERNEL_SPHERICAL, GSI_ERR_INVALID_ARGUMENT,
+                    "kernelcov: unknown kernel kind");
         GSI_REQUIRE(n >= 1 && row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov: bad row block");
         for (int k = 0; k < d; ++k) GSI_REQUIRE(ell[k] > 0.0, GSI_ERR_INVALID_ARGUMENT, "kernelcov: length scales must be positive");
         std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
@@ -518,8 +519,12 @@ GSI_API int32_t gsi_op_kernelcov(gsi_ctx* ctx, int32_t kind, int32_t d, int64_t 
         op->sigma2 = sigma2; op->nugget = nugget; op->beta = beta;
         op->n_pad = round_up(n, kRowPad);
         // scaled SoA coordinates u[k][j] = x_j[k] / ell[k]; padding repeats the last point.
-        // Gaussian: an extra 1/sqrt(2) folds the factor 1/2 of exp(-r2/2) into r2.
-        const double pre = (kind == GSI_KERNEL_GAUSSIAN) ? 0.70710678118654752440 : 1.0;
+        // Gaussian: an extra 1/sqrt(2) folds the factor 1/2 of exp(-r2/2) into r2; Matern nu = 3/2 / 5/2: an extra
+        // sqrt(3) / sqrt(5), so the kernel's sqrt(r2) is the argument sqrt(2 nu) r of exp and of the polynomial.
+        const double pre = kind == GSI_KERNEL_GAUSSIAN   ? 0.70710678118654752440
+                           : kind == GSI_KERNEL_MATERN32 ? 1.73205080756887729353
+                           : kind == GSI_KERNEL_MATERN52 ? 2.23606797749978969641
+                                                         : 1.0;
         std::vector<double> u((size_t)3 * op->n_pad, 0.0);
         for (int k = 0; k < d; ++k) {
             double* uk = u.data() + (size_t)k * op->n_pad;
@@ -542,7 +547,8 @@ GSI_API int32_t gsi_op_kernelcov_grid(gsi_ctx* ctx, int32_t kind, int32_t d, con
         use(ctx);
         GSI_REQUIRE(dims && spacing && ell && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
         GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov_grid: d must be 1, 2 or 3");
-        GSI_REQUIRE(kind >= 0 && kind <= 2, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: unknown kernel kind");
+        GSI_REQUIRE(kind >= GSI_KERNEL_EXPONENTIAL && kind <= GSI_KERNEL_SPHERICAL, GSI_ERR_INVALID_ARGUMENT,
+                    "kernelcov_grid: unknown kernel kind");
         int64_t nd[3] = {1, 1, 1};
         double h[3] = {1, 1, 1}, el[3] = {1, 1, 1};
         int64_t n = 1;
@@ -571,7 +577,16 @@ GSI_API int32_t gsi_op_kernelcov_grid(gsi_ctx* ctx, int32_t kind, int32_t d, con
                     double v;
                     if (kind == GSI_KERNEL_EXPONENTIAL) v = std::exp(-std::sqrt(r2));
                     else if (kind == GSI_KERNEL_GAUSSIAN) v = std::exp(-0.5 * r2);
-                    else v = std::exp(-beta * std::log1p(r2));
+                    else if (kind == GSI_KERNEL_MATERN32) {
+                        const double s = std::sqrt(3.0 * r2);
+                        v = (1.0 + s) * std::exp(-s);
+                    } else if (kind == GSI_KERNEL_MATERN52) {
+                        const double s = std::sqrt(5.0 * r2);
+                        v = (1.0 + s + s * s / 3.0) * std::exp(-s);
+                    } else if (kind == GSI_KERNEL_SPHERICAL) {
+                        const double r = std::sqrt(r2);
+                        v = r < 1.0 ? 0.5 * (1.0 - r) * (1.0 - r) * (2.0 + r) : 0.0;   // = 1 - 1.5 r + 0.5 r^3, no cancellation
+                    } else v = std::exp(-beta * std::log1p(r2));
                     tab[(size_t)(dx + nd[0] * (dy + nd[1] * dz))] = v;
                 }
         // lattice indices of every point (SoA, padding repeats the last point)

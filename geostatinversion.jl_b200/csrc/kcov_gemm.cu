@@ -33,7 +33,8 @@ constexpr int KC_AP = KC_BK + 4;   // pitch of the generated A tile (4 mod 16 do
 constexpr int KC_WARPS = 16;
 constexpr int KC_THREADS = KC_WARPS * 32;
 constexpr int KC_CG = 4;           // column groups (warps sharing one row group)
-constexpr int KC_KIND_TABLE = 3;   // internal kind: stationary kernel on a structured grid, values from a lattice table
+constexpr int KC_KIND_TABLE = 15;  // internal kind: stationary kernel on a structured grid, values from a lattice table
+                                   // (outside the public GSI_KERNEL_* range)
 constexpr long long KC_SPIN_LIMIT = 400000;   // cycles (~0.2 ms) a producer waits on the sweep window before giving it up
 
 struct KcovParams {
@@ -131,12 +132,52 @@ __device__ __forceinline__ double fast_sqrt_pos(double x) {
     return g;
 }
 
+// kinds whose value is a function of sqrt(r2): r2 gets a 1e-300 offset so that fast_sqrt_pos stays finite
+// on the diagonal (sqrt(1e-300) = 1e-150 leaves every one of these values at exactly 1)
+template <int KIND>
+__device__ __forceinline__ constexpr bool kind_takes_sqrt() {
+    return KIND == GSI_KERNEL_EXPONENTIAL || KIND == GSI_KERNEL_MATERN32 || KIND == GSI_KERNEL_MATERN52 ||
+           KIND == GSI_KERNEL_SPHERICAL;
+}
+
 // kind-specific value from r2.  For the Gaussian kernel the coordinates handed to the
-// kernel are pre-scaled by 1/sqrt(2) so that r2 already carries the factor 1/2.
+// kernel are pre-scaled by 1/sqrt(2) so that r2 already carries the factor 1/2; for the Matern
+// kernels by sqrt(3) / sqrt(5), so that s = sqrt(r2) is the argument sqrt(2 nu) r of the Matern form.
+// Relative error, in units of 2^-52 (measured in ulps of the exact value of the device's r2 this is at most twice
+// as much, as a value and its rounding error can sit at opposite ends of a binade), with k = the conditioning
+// |s k'(s) / k(s)| and 2 ulp of s from fast_sqrt_pos (each contributing at most 2 k * 2^-52):
+//   matern32   fma(s, e, e) = RN(e (1 + s)):     2.5 (fast_exp_neg) + 0.5 (fma)                       = 3    + 2 k
+//   matern52   RN(RN(fma(r2, RN(1/3), RN(s + 1))) e): 2.5 + 0.5 (s + 1) + 0.25 (1/3) + 0.5 (fma) + 0.5 = 4.25 + 2 k
+//   spherical  RN(RN(0.5 t * t) RN(2 + s)), t = 1 - s (exact for s >= 0.5, 2^-53 relative below,
+//              doubled by the square): 1 + 0.5 + 0.5 + 0.5                                            = 2.5  + 2 k
+// tests/test_gpu_matern.py asserts 6 + 4 k, 8.5 + 4 k and 5 + 4 k ulp.  Largest errors measured on a B200
+// (1000 W), d = 1..3, about 4200 arguments each: matern32 2.31 ulp for s < 1 (worst against the bound 2.05 of
+// 6.25 ulp), matern52 3.07 ulp for s < 1 (3.07 of 8.71), spherical 4.15 ulp for s < 0.5 (worst against the bound
+// 2.40 of 5.09).  Every term of the Matern polynomials is positive (no cancellation); the clamp of matern52
+// to 1 only moves a value towards the exact one (<= 1).  The spherical form 0.5 (1 - s)^2 (2 + s) avoids the
+// cancellation of 1 - 1.5 s + 0.5 s^3 as s -> 1.  The Matern values are flushed to zero with their exp factor
+// (below 2^-1000).
 template <int KIND>
 __device__ __forceinline__ double kern_eval(double r2, double beta, const double* __restrict__ tab) {
     if (KIND == GSI_KERNEL_EXPONENTIAL) return fast_exp_neg(fast_sqrt_pos(r2), tab);
     if (KIND == GSI_KERNEL_GAUSSIAN) return fast_exp_neg(r2, tab);
+    if (KIND == GSI_KERNEL_MATERN32) {
+        const double s = fast_sqrt_pos(r2);
+        const double e = fast_exp_neg(s, tab);
+        return fma(s, e, e);                                   // (1 + s) e^-s
+    }
+    if (KIND == GSI_KERNEL_MATERN52) {
+        const double s = fast_sqrt_pos(r2);
+        const double e = fast_exp_neg(s, tab);
+        // (1 + s + s^2/3) e^-s.  For s around 2e-8 the exact value is 1 - s^3/30 and the rounding errors of e and
+        // of the product can leave 1 + 2^-52 (host emulation of this sequence), so the value is clamped to 1
+        return fmin(fma(r2, 1.0 / 3.0, s + 1.0) * e, 1.0);
+    }
+    if (KIND == GSI_KERNEL_SPHERICAL) {
+        const double s = fast_sqrt_pos(r2);
+        const double t = 1.0 - s;
+        return s < 1.0 ? (0.5 * t) * t * (2.0 + s) : 0.0;      // 0.5 (1 - s)^2 (2 + s)
+    }
     if (KIND == KC_KIND_TABLE) return 0.0;
     return exp(-beta * log1p(r2));
 }
@@ -387,7 +428,7 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
     auto gen4 = [&](const double (&ui)[DIM], const double* u0, int64_t ustride, double (&v)[4]) {
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
-            double r2 = (KIND == GSI_KERNEL_EXPONENTIAL) ? 1e-300 : 0.0;
+            double r2 = kind_takes_sqrt<KIND>() ? 1e-300 : 0.0;
 #pragma unroll
             for (int k = 0; k < DIM; ++k) {
                 const double dk = ui[k] - u0[k * ustride + gcol(e)];
@@ -491,7 +532,7 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
                 // is live at a time and its DFMAs interleave with this step's DMMAs
                 if (KIND != KC_KIND_TABLE && (ks & 1) == 0 && gen_next) {
                     const int e = ks >> 1;
-                    double r2 = (KIND == GSI_KERNEL_EXPONENTIAL) ? 1e-300 : 0.0;
+                    double r2 = kind_takes_sqrt<KIND>() ? 1e-300 : 0.0;
 #pragma unroll
                     for (int k = 0; k < DIM; ++k) {
                         const double dk = ui[k] - us[k * KC_BK + gcol(e)];
@@ -674,6 +715,9 @@ static void dispatch_kind(gsi_ctx* ctx, const KcovParams& p, int kind, int dim) 
         case GSI_KERNEL_EXPONENTIAL: dispatch_dim<NB, GSI_KERNEL_EXPONENTIAL>(ctx, p, dim); break;
         case GSI_KERNEL_GAUSSIAN: dispatch_dim<NB, GSI_KERNEL_GAUSSIAN>(ctx, p, dim); break;
         case GSI_KERNEL_POWERLAW: dispatch_dim<NB, GSI_KERNEL_POWERLAW>(ctx, p, dim); break;
+        case GSI_KERNEL_MATERN32: dispatch_dim<NB, GSI_KERNEL_MATERN32>(ctx, p, dim); break;
+        case GSI_KERNEL_MATERN52: dispatch_dim<NB, GSI_KERNEL_MATERN52>(ctx, p, dim); break;
+        case GSI_KERNEL_SPHERICAL: dispatch_dim<NB, GSI_KERNEL_SPHERICAL>(ctx, p, dim); break;
         case KC_KIND_TABLE: dispatch_dim<NB, KC_KIND_TABLE>(ctx, p, dim); break;
         default: throw Error(GSI_ERR_INVALID_ARGUMENT, "unknown covariance kernel kind");
     }

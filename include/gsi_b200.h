@@ -65,6 +65,12 @@ extern "C" {
 #define GSI_KERNEL_EXPONENTIAL 0 /* sigma2 * exp(-sqrt(r2))                                    */
 #define GSI_KERNEL_GAUSSIAN 1    /* sigma2 * exp(-0.5 * r2)                                    */
 #define GSI_KERNEL_POWERLAW 2    /* sigma2 * (1 + r2)^(-beta)                                  */
+/* Matern nu = 3/2 and 5/2 (Rasmussen-Williams convention, r = sqrt(r2); exponential is nu = 1/2,
+ * Gaussian the limit nu -> infinity) and the spherical model (ell is its range; positive definite
+ * for d <= 3).  beta is ignored by these kinds.                                                    */
+#define GSI_KERNEL_MATERN32 3    /* sigma2 * (1 + sqrt(3) r) * exp(-sqrt(3) r)                 */
+#define GSI_KERNEL_MATERN52 4    /* sigma2 * (1 + sqrt(5) r + 5 r2 / 3) * exp(-sqrt(5) r)       */
+#define GSI_KERNEL_SPHERICAL 5   /* sigma2 * (1 - 1.5 r + 0.5 r^3) for r < 1, else 0            */
 
 /* normaliser used between power iterations */
 #define GSI_NORMALISER_LU_REF 0 /* partial-pivot LU, unit-lower L kept in LAPACK row order

@@ -27,6 +27,9 @@ const GSI_NORMALISER_LU_REF = Int32(0)
 const GSI_KERNEL_EXPONENTIAL = Int32(0)
 const GSI_KERNEL_GAUSSIAN = Int32(1)
 const GSI_KERNEL_POWERLAW = Int32(2)
+const GSI_KERNEL_MATERN32 = Int32(3)
+const GSI_KERNEL_MATERN52 = Int32(4)
+const GSI_KERNEL_SPHERICAL = Int32(5)
 
 lasterror() = unsafe_string(ccall((:gsi_last_error_string, LIB), Cstring, ()))
 
@@ -155,7 +158,8 @@ function DenseOperator(A::Matrix{Float64}; ctx::Context=context(), rows::UnitRan
 	return op
 end
 
-"kind: 0 exponential, 1 gaussian, 2 powerlaw; coords d x n; ell d.  Multi-GPU: `rows` = this worker's rows of C."
+"kind: 0 exponential, 1 gaussian, 2 powerlaw, 3 matern32, 4 matern52, 5 spherical (GSI_KERNEL_*; ell is the spherical
+model's range); coords d x n; ell d.  Multi-GPU: `rows` = this worker's rows of C."
 function KernelCovMatrix(kind::Integer, coords::Matrix{Float64}, ell::Vector{Float64}; sigma2=1.0, nugget=0.0, beta=1.0,
 		ctx::Context=context(), rows::UnitRange{Int}=partitionrows(size(coords, 2), ctx.world, ctx.rank))
 	d, n = size(coords)
@@ -168,7 +172,7 @@ function KernelCovMatrix(kind::Integer, coords::Matrix{Float64}, ell::Vector{Flo
 	return op
 end
 
-"structured grid variant: dims[1] fastest (Julia linear index), coordinates idx .* spacing"
+"structured grid variant (same kinds): dims[1] fastest (Julia linear index), coordinates idx .* spacing"
 function KernelCovGrid(kind::Integer, dims::Vector{Int}, spacing::Vector{Float64}, ell::Vector{Float64}; sigma2=1.0, nugget=0.0, beta=1.0,
 		ctx::Context=context(), rows::UnitRange{Int}=partitionrows(prod(dims), ctx.world, ctx.rank))
 	d = length(dims)

@@ -8,9 +8,11 @@ CPU fallback: importing works anywhere, creating a Context needs a B200.
 from . import _lib
 from ._lib import (GsiError, SingularException, PosDefException, DimensionMismatch, NoDeviceError,
                    LAYOUT_TALL, LAYOUT_COLMAJOR, KERNEL_EXPONENTIAL, KERNEL_GAUSSIAN, KERNEL_POWERLAW,
-                   KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SPHERICAL, NORMALISER_LU_REF, NORMALISER_QR)
+                   KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SPHERICAL, MODEL_MAX_STRUCTURES, NORMALISER_LU_REF,
+                   NORMALISER_QR)
 from .core import (Context, DeviceMatrix, DenseMatrix, LowRankCovMatrix, KernelCovMatrix, GridKernelCovMatrix, default_context,
-                   set_default_context, as_operator, partition_rows)
+                   set_default_context, as_operator, partition_rows, CovStructure, rotation_matrix, KernelCovModelMatrix,
+                   GridKernelCovModelMatrix)
 from . import randmatfact as RandMatFact
 from .randmatfact import randsvd, rangefinder, eig_nystrom
 from . import dist

@@ -31,6 +31,7 @@ KERNEL_POWERLAW = 2
 KERNEL_MATERN32 = 3
 KERNEL_MATERN52 = 4
 KERNEL_SPHERICAL = 5
+MODEL_MAX_STRUCTURES = 4
 NORMALISER_LU_REF = 0
 NORMALISER_QR = 1
 
@@ -71,6 +72,9 @@ SIGNATURES = {
     "gsi_op_lowrankcov_sharded": (_i32, [_p, _p, _i32, _i64, _i64, _pp]),
     "gsi_op_kernelcov": (_i32, [_p, _i32, _i32, _i64, _pd, _pd, _f64, _f64, _f64, _i64, _i64, _pp]),
     "gsi_op_kernelcov_grid": (_i32, [_p, _i32, _i32, _pi64, _pd, _pd, _f64, _f64, _f64, _i64, _i64, _pp]),
+    "gsi_op_kernelcov_model": (_i32, [_p, _i32, _i64, _pd, _i32, _pi32, _pd, _pd, _pd, _pd, _f64, _i64, _i64, _pp]),
+    "gsi_op_kernelcov_model_grid": (_i32, [_p, _i32, _pi64, _pd, _i32, _pi32, _pd, _pd, _pd, _pd, _f64, _i64, _i64,
+                                           _pp]),
     "gsi_op_free": (_i32, [_p]),
     "gsi_op_size": (_i32, [_p, _pi64, _pi64]),
     "gsi_op_apply": (_i32, [_p, _i32, _p, _p]),

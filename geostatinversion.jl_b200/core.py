@@ -8,7 +8,8 @@ import numpy as np
 
 from . import _lib
 from ._lib import (LAYOUT_TALL, LAYOUT_COLMAJOR, KERNEL_EXPONENTIAL, KERNEL_GAUSSIAN, KERNEL_POWERLAW,
-                   KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SPHERICAL, NORMALISER_LU_REF, NORMALISER_QR, check)
+                   KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_SPHERICAL, MODEL_MAX_STRUCTURES, NORMALISER_LU_REF,
+                   NORMALISER_QR, check)
 
 _KINDS = {"exponential": KERNEL_EXPONENTIAL, "gaussian": KERNEL_GAUSSIAN, "powerlaw": KERNEL_POWERLAW,
           "matern32": KERNEL_MATERN32, "matern52": KERNEL_MATERN52, "spherical": KERNEL_SPHERICAL,
@@ -399,6 +400,95 @@ class GridKernelCovMatrix(_Operator):
         self.kind = _KINDS[kind]
         check(self._lib.gsi_op_kernelcov_grid(self.ctx._h, self.kind, d, dims, _pd(spacing), _pd(ell), float(sigma2),
                                               float(nugget), float(beta), self.row0, self.mloc, C.byref(self._h)))
+
+
+def rotation_matrix(angles):
+    """Rotation R (u = R x) onto the principal axes of an anisotropic structure.  2-D: one angle in radians,
+    counter-clockwise from the x axis to the first principal axis.  3-D: three intrinsic z-y-x angles (the first
+    about z, the second about the new y, the third about the newest x).  The rows of R are the principal axes."""
+    a = np.atleast_1d(np.asarray(angles, dtype=np.float64))
+    if a.size == 1:
+        c, s = np.cos(a[0]), np.sin(a[0])
+        return np.array([[c, s], [-s, c]])
+    if a.size != 3:
+        raise ValueError("rotation_matrix: one angle (2-D) or three z-y-x angles (3-D)")
+    cz, sz = np.cos(a[0]), np.sin(a[0])
+    cy, sy = np.cos(a[1]), np.sin(a[1])
+    cx, sx = np.cos(a[2]), np.sin(a[2])
+    rz = np.array([[cz, -sz, 0.0], [sz, cz, 0.0], [0.0, 0.0, 1.0]])
+    ry = np.array([[cy, 0.0, sy], [0.0, 1.0, 0.0], [-sy, 0.0, cy]])
+    rx = np.array([[1.0, 0.0, 0.0], [0.0, cx, -sx], [0.0, sx, cx]])
+    return (rz @ ry @ rx).T                # columns of rz ry rx: the principal axes in world coordinates
+
+
+class CovStructure:
+    """One structure of a nested covariance model: sill * k_kind(r2), r2 = |(R x_i - R x_j) ./ ranges|^2 (with the
+    kind's scaling, include/gsi_b200.h).  rotation: d x d orthonormal R (u = R x, see rotation_matrix) or None."""
+
+    def __init__(self, kind, sill, ranges, rotation=None, beta=1.0):
+        self.kind = _KINDS[kind]
+        self.sill = float(sill)
+        self.ranges = np.atleast_1d(np.asarray(ranges, dtype=np.float64))
+        self.rotation = None if rotation is None else np.asarray(rotation, dtype=np.float64)
+        self.beta = float(beta)
+
+
+def _model_args(structures, d):
+    """ctypes arguments (nstruct, kinds, sills, ranges, rotations or None, betas) of the gsi_op_kernelcov_model* calls;
+    the arrays are returned too, to keep them alive through the call."""
+    structures = list(structures)
+    ns = len(structures)
+    kinds = (C.c_int32 * max(ns, 1))(*[s.kind for s in structures])
+    sills = np.array([s.sill for s in structures], dtype=np.float64)
+    ranges = np.concatenate([np.broadcast_to(s.ranges, (d,)) for s in structures]) if ns else np.zeros(1)
+    ranges = np.ascontiguousarray(ranges, dtype=np.float64)
+    betas = np.array([s.beta for s in structures], dtype=np.float64)
+    rot = None
+    if any(s.rotation is not None for s in structures):
+        rot = np.concatenate([(np.eye(d) if s.rotation is None else s.rotation.reshape(d, d)).ravel(order="F")
+                              for s in structures])
+        rot = np.ascontiguousarray(rot, dtype=np.float64)
+    keep = (kinds, sills, ranges, betas, rot)
+    args = [ns, kinds, _pd(sills) if ns else None, _pd(ranges), None if rot is None else _pd(rot),
+            _pd(betas) if ns else None]
+    return args, keep
+
+
+class KernelCovModelMatrix(_Operator):
+    """Matrix-free covariance operator of a nested model (gsi_op_kernelcov_model):
+    C[i,j] = sum_s sill_s k_s(x_i, x_j) + nugget (i == j), 1 to MODEL_MAX_STRUCTURES CovStructure terms, each with its
+    own kind, ranges and rotation.  coords: d x n.  Several structures are summed inside the product kernel, so the
+    model costs one operator application."""
+    symmetric = True
+
+    def __init__(self, structures, coords, nugget=0.0, ctx=None, row0=0, mloc=None):
+        super().__init__(ctx or default_context())
+        coords = _f64_colmajor(coords)
+        d, n = coords.shape
+        self.row0 = int(row0)
+        self.mloc = int(n - row0 if mloc is None else mloc)
+        args, self._keep = _model_args(structures, d)
+        check(self._lib.gsi_op_kernelcov_model(self.ctx._h, d, n, _pd(coords), *args, float(nugget), self.row0,
+                                               self.mloc, C.byref(self._h)))
+
+
+class GridKernelCovModelMatrix(_Operator):
+    """KernelCovModelMatrix for points on a structured grid (as GridKernelCovMatrix): the whole model is tabulated once
+    per lattice offset (signed offsets when a structure is rotated)."""
+    symmetric = True
+
+    def __init__(self, structures, shape, spacing=None, nugget=0.0, ctx=None, row0=0, mloc=None):
+        super().__init__(ctx or default_context())
+        shape = [int(s) for s in shape]
+        d = len(shape)
+        n = int(np.prod(shape))
+        dims = (C.c_int64 * d)(*shape)
+        spacing = np.ascontiguousarray(np.broadcast_to(np.asarray(1.0 if spacing is None else spacing, dtype=np.float64), (d,)))
+        self.row0 = int(row0)
+        self.mloc = int(n - row0 if mloc is None else mloc)
+        args, self._keep = _model_args(structures, d)
+        check(self._lib.gsi_op_kernelcov_model_grid(self.ctx._h, d, dims, _pd(spacing), *args, float(nugget), self.row0,
+                                                    self.mloc, C.byref(self._h)))
 
 
 def as_operator(A, ctx=None):

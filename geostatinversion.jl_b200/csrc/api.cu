@@ -502,6 +502,221 @@ GSI_API int32_t gsi_op_lowrankcov_sharded(gsi_ctx* ctx, gsi_buf* samples_local, 
     return guarded([&] { make_lowrankcov(ctx, samples_local, remove_mean, row0, n_global, out); });
 }
 
+namespace gsi {
+// A covariance model: nstruct structures, each a kind, a sill, d ranges, an optional rotation (column-major d x d,
+// u = R x) and a power-law exponent.  gsi_op_kernelcov / _grid are the one-structure, unrotated case.
+struct CovModel {
+    int d = 1, nstruct = 1;
+    int kinds[GSI_MODEL_MAX_STRUCTURES] = {};
+    double sills[GSI_MODEL_MAX_STRUCTURES] = {}, betas[GSI_MODEL_MAX_STRUCTURES] = {};
+    double ranges[GSI_MODEL_MAX_STRUCTURES][3] = {};
+    double rot[GSI_MODEL_MAX_STRUCTURES][9] = {};
+    bool rotated[GSI_MODEL_MAX_STRUCTURES] = {};
+    bool any_rotated() const {
+        for (int s = 0; s < nstruct; ++s)
+            if (rotated[s]) return true;
+        return false;
+    }
+};
+
+static CovModel single_structure(int32_t kind, int32_t d, const double* ell, double sigma2, double beta) {
+    CovModel m;
+    m.d = d; m.nstruct = 1; m.kinds[0] = kind; m.sills[0] = sigma2; m.betas[0] = beta;
+    for (int k = 0; k < d; ++k) m.ranges[0][k] = ell[k];
+    return m;
+}
+
+// the public model arguments, checked (d was checked by the caller)
+static CovModel model_from_args(int32_t d, int32_t nstruct, const int32_t* kinds, const double* sills,
+                                const double* ranges, const double* rotations, const double* betas) {
+    GSI_REQUIRE(nstruct >= 1 && nstruct <= GSI_MODEL_MAX_STRUCTURES, GSI_ERR_INVALID_ARGUMENT,
+                "kernelcov_model: nstruct must be in 1..GSI_MODEL_MAX_STRUCTURES");
+    CovModel m;
+    m.d = d; m.nstruct = nstruct;
+    for (int s = 0; s < nstruct; ++s) {
+        GSI_REQUIRE(kinds[s] >= GSI_KERNEL_EXPONENTIAL && kinds[s] <= GSI_KERNEL_SPHERICAL, GSI_ERR_INVALID_ARGUMENT,
+                    "kernelcov_model: unknown kernel kind");
+        GSI_REQUIRE(std::isfinite(sills[s]) && sills[s] > 0.0, GSI_ERR_INVALID_ARGUMENT,
+                    "kernelcov_model: sills must be positive and finite");
+        m.kinds[s] = kinds[s]; m.sills[s] = sills[s]; m.betas[s] = betas ? betas[s] : 1.0;
+        for (int k = 0; k < d; ++k) {
+            GSI_REQUIRE(ranges[s * d + k] > 0.0, GSI_ERR_INVALID_ARGUMENT, "kernelcov_model: ranges must be positive");
+            m.ranges[s][k] = ranges[s * d + k];
+        }
+        if (!rotations) continue;
+        const double* R = rotations + (size_t)s * d * d;
+        double dev = 0.0;
+        for (int a = 0; a < d; ++a)
+            for (int b = 0; b < d; ++b) {
+                GSI_REQUIRE(std::isfinite(R[a + d * b]), GSI_ERR_INVALID_ARGUMENT, "kernelcov_model: rotation not finite");
+                double rr = 0.0;                                   // (R'R)[a, b]
+                for (int k = 0; k < d; ++k) rr += R[k + d * a] * R[k + d * b];
+                dev = std::fmax(dev, std::fabs(rr - (a == b ? 1.0 : 0.0)));
+            }
+        GSI_REQUIRE(dev <= 1e-12, GSI_ERR_INVALID_ARGUMENT, "kernelcov_model: rotation is not orthonormal");
+        for (int q = 0; q < d * d; ++q) m.rot[s][q] = R[q];
+        m.rotated[s] = true;
+    }
+    return m;
+}
+
+// coordinate scaling of the kinds: Gaussian: an extra 1/sqrt(2) folds the factor 1/2 of exp(-r2/2) into r2; Matern
+// nu = 3/2 / 5/2: an extra sqrt(3) / sqrt(5), so the kernel's sqrt(r2) is the argument sqrt(2 nu) r of exp and of the
+// polynomial
+static double kind_pre(int kind) {
+    return kind == GSI_KERNEL_GAUSSIAN   ? 0.70710678118654752440
+           : kind == GSI_KERNEL_MATERN32 ? 1.73205080756887729353
+           : kind == GSI_KERNEL_MATERN52 ? 2.23606797749978969641
+                                         : 1.0;
+}
+
+// u[k] = ((sum_j R[k,j] x_j) / range[k]) * pre of structure s; without a rotation (x[k] / range[k]) * pre
+static void structure_coords(const CovModel& m, int s, const double* x, double pre, double* u) {
+    for (int k = 0; k < m.d; ++k) {
+        double y = x[k];
+        if (m.rotated[s]) {
+            y = 0.0;
+            for (int j = 0; j < m.d; ++j) y += m.rot[s][k + m.d * j] * x[j];
+        }
+        u[k] = (y / m.ranges[s][k]) * pre;
+    }
+}
+
+// k(r2) with libm, r2 in unscaled coordinates (x / range): the value of every lattice-table entry
+static double kern_host(int kind, double r2, double beta) {
+    if (kind == GSI_KERNEL_EXPONENTIAL) return std::exp(-std::sqrt(r2));
+    if (kind == GSI_KERNEL_GAUSSIAN) return std::exp(-0.5 * r2);
+    if (kind == GSI_KERNEL_MATERN32) {
+        const double s = std::sqrt(3.0 * r2);
+        return (1.0 + s) * std::exp(-s);
+    }
+    if (kind == GSI_KERNEL_MATERN52) {
+        const double s = std::sqrt(5.0 * r2);
+        return (1.0 + s + s * s / 3.0) * std::exp(-s);
+    }
+    if (kind == GSI_KERNEL_SPHERICAL) {
+        const double r = std::sqrt(r2);
+        return r < 1.0 ? 0.5 * (1.0 - r) * (1.0 - r) * (2.0 + r) : 0.0;   // = 1 - 1.5 r + 0.5 r^3, no cancellation
+    }
+    return std::exp(-beta * std::log1p(r2));
+}
+
+// the table value of the offset x (one structure: k, scaled by sigma2 = its sill in the epilogue; several: the sum)
+static double model_host(const CovModel& m, const double* x) {
+    double v = 0.0;
+    for (int s = 0; s < m.nstruct; ++s) {
+        double u[3];
+        structure_coords(m, s, x, 1.0, u);
+        double r2 = u[0] * u[0];
+        if (m.d > 1) r2 += u[1] * u[1];
+        if (m.d > 2) r2 += u[2] * u[2];
+        const double k = kern_host(m.kinds[s], r2, m.betas[s]);
+        if (m.nstruct == 1) return k;
+        v += m.sills[s] * k;
+    }
+    return v;
+}
+
+// the operator's model parameters: one structure is the specialised KIND kernel with sigma2 = its sill; several are
+// KC_KIND_MODEL (arithmetic) or a table of the sum (grid), both with sigma2 = 1
+static void set_model(gsi_op* op, const CovModel& m, double nugget, bool generated) {
+    op->type = OP_KERNELCOV; op->dim = m.d; op->nugget = nugget;
+    op->kind = m.kinds[0]; op->sigma2 = m.sills[0]; op->beta = m.betas[0];
+    if (m.nstruct == 1) return;
+    op->sigma2 = 1.0; op->beta = 1.0;
+    if (!generated) return;
+    op->kind = KC_KIND_MODEL;
+    op->nstruct = m.nstruct;
+    for (int s = 0; s < m.nstruct; ++s) {
+        op->mkinds[s] = m.kinds[s]; op->msills[s] = m.sills[s]; op->mbetas[s] = m.betas[s];
+    }
+}
+
+static void make_kernelcov(gsi_ctx* ctx, int64_t n, const double* coords, const CovModel& m, double nugget, int64_t row0,
+                           int64_t mloc, gsi_op** out) {
+    GSI_REQUIRE(n >= 1 && row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov: bad row block");
+    const int d = m.d;
+    std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
+    op->ctx = ctx;
+    set_model(op.get(), m, nugget, true);
+    op->m = op->n = n; op->row0 = row0; op->mloc = mloc;
+    op->n_pad = round_up(n, kRowPad);
+    // scaled SoA coordinates u[s][k][j] of every structure (one structure: u[k][j]); padding repeats the last point
+    std::vector<double> u((size_t)m.nstruct * 3 * op->n_pad, 0.0);
+    for (int s = 0; s < m.nstruct; ++s) {
+        const double pre = kind_pre(m.kinds[s]);
+        double* us = u.data() + (size_t)s * 3 * op->n_pad;
+        for (int64_t j = 0; j < n; ++j) {
+            double uj[3];
+            structure_coords(m, s, coords + j * d, pre, uj);
+            for (int k = 0; k < d; ++k) us[(size_t)k * op->n_pad + j] = uj[k];
+        }
+        for (int k = 0; k < d; ++k)
+            for (int64_t j = n; j < op->n_pad; ++j) us[(size_t)k * op->n_pad + j] = us[(size_t)k * op->n_pad + n - 1];
+    }
+    GSI_CUDA(cudaMalloc(&op->ucoords, u.size() * sizeof(double)));
+    GSI_CUDA(cudaMemcpyAsync(op->ucoords, u.data(), u.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
+    set_partition(op.get());
+    ctx_retain(ctx);
+    *out = op.release();
+}
+
+static void make_kernelcov_grid(gsi_ctx* ctx, const int64_t* dims, const double* spacing, const CovModel& m, double nugget,
+                                int64_t row0, int64_t mloc, gsi_op** out) {
+    const int d = m.d;
+    int64_t nd[3] = {1, 1, 1};
+    double h[3] = {1, 1, 1};
+    int64_t n = 1;
+    for (int k = 0; k < d; ++k) {
+        GSI_REQUIRE(dims[k] >= 1, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad dims / length scales");
+        nd[k] = dims[k]; h[k] = spacing[k];
+        n *= dims[k];
+    }
+    GSI_REQUIRE(n < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: more than 2^31 points");
+    GSI_REQUIRE(row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad row block");
+    // a rotated model is not symmetric in each axis: its table covers signed offsets, folded by k(delta) = k(-delta)
+    // (the last axis as |delta|, the others from -(n - 1) to n - 1).  d = 1 is symmetric whatever the rotation (+-1)
+    const bool sgn = m.any_rotated() && d >= 2;
+    const int64_t ex = sgn ? 2 * nd[0] - 1 : nd[0];
+    const int64_t ey = sgn && d == 3 ? 2 * nd[1] - 1 : nd[1];
+    const int64_t tsize = ex * ey * nd[2];
+    GSI_REQUIRE(tsize < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: lattice table of 2^31 entries or more");
+    std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
+    op->ctx = ctx;
+    set_model(op.get(), m, nugget, false);
+    op->m = op->n = n; op->row0 = row0; op->mloc = mloc;
+    op->n_pad = round_up(n, kRowPad);
+    op->grid_nx = (int)nd[0]; op->grid_ny = (int)nd[1]; op->grid_nz = (int)nd[2];
+    op->table_signed = sgn;
+    // kernel value of every lattice offset (libm, same formula as the dense definition)
+    const int64_t ox = sgn ? nd[0] - 1 : 0, oy = sgn && d == 3 ? nd[1] - 1 : 0;
+    std::vector<double> tab((size_t)tsize);
+    for (int64_t iz = 0; iz < nd[2]; ++iz)
+        for (int64_t iy = 0; iy < ey; ++iy)
+            for (int64_t ix = 0; ix < ex; ++ix) {
+                const double x[3] = {(double)(ix - ox) * h[0], (double)(iy - oy) * h[1], (double)iz * h[2]};
+                tab[(size_t)(ix + ex * (iy + ey * iz))] = model_host(m, x);
+            }
+    // lattice indices of every point (SoA, padding repeats the last point)
+    std::vector<int> lat((size_t)3 * op->n_pad, 0);
+    for (int64_t j = 0; j < op->n_pad; ++j) {
+        const int64_t jj = j < n ? j : n - 1;
+        lat[(size_t)0 * op->n_pad + j] = (int)(jj % nd[0]);
+        lat[(size_t)1 * op->n_pad + j] = (int)((jj / nd[0]) % nd[1]);
+        lat[(size_t)2 * op->n_pad + j] = (int)(jj / (nd[0] * nd[1]));
+    }
+    GSI_CUDA(cudaMalloc(&op->table, tab.size() * sizeof(double)));
+    GSI_CUDA(cudaMalloc(&op->lattice, lat.size() * sizeof(int)));
+    GSI_CUDA(cudaMemcpyAsync(op->table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    GSI_CUDA(cudaMemcpyAsync(op->lattice, lat.data(), lat.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
+    set_partition(op.get());
+    ctx_retain(ctx);
+    *out = op.release();
+}
+}  // namespace gsi
+
 GSI_API int32_t gsi_op_kernelcov(gsi_ctx* ctx, int32_t kind, int32_t d, int64_t n, const double* coords,
                                  const double* ell, double sigma2, double nugget, double beta, int64_t row0,
                                  int64_t mloc, gsi_op** out) {
@@ -513,30 +728,7 @@ GSI_API int32_t gsi_op_kernelcov(gsi_ctx* ctx, int32_t kind, int32_t d, int64_t 
                     "kernelcov: unknown kernel kind");
         GSI_REQUIRE(n >= 1 && row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov: bad row block");
         for (int k = 0; k < d; ++k) GSI_REQUIRE(ell[k] > 0.0, GSI_ERR_INVALID_ARGUMENT, "kernelcov: length scales must be positive");
-        std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
-        op->ctx = ctx; op->type = OP_KERNELCOV; op->kind = kind; op->dim = d;
-        op->m = op->n = n; op->row0 = row0; op->mloc = mloc;
-        op->sigma2 = sigma2; op->nugget = nugget; op->beta = beta;
-        op->n_pad = round_up(n, kRowPad);
-        // scaled SoA coordinates u[k][j] = x_j[k] / ell[k]; padding repeats the last point.
-        // Gaussian: an extra 1/sqrt(2) folds the factor 1/2 of exp(-r2/2) into r2; Matern nu = 3/2 / 5/2: an extra
-        // sqrt(3) / sqrt(5), so the kernel's sqrt(r2) is the argument sqrt(2 nu) r of exp and of the polynomial.
-        const double pre = kind == GSI_KERNEL_GAUSSIAN   ? 0.70710678118654752440
-                           : kind == GSI_KERNEL_MATERN32 ? 1.73205080756887729353
-                           : kind == GSI_KERNEL_MATERN52 ? 2.23606797749978969641
-                                                         : 1.0;
-        std::vector<double> u((size_t)3 * op->n_pad, 0.0);
-        for (int k = 0; k < d; ++k) {
-            double* uk = u.data() + (size_t)k * op->n_pad;
-            for (int64_t j = 0; j < n; ++j) uk[j] = (coords[j * d + k] / ell[k]) * pre;
-            for (int64_t j = n; j < op->n_pad; ++j) uk[j] = uk[n - 1];
-        }
-        GSI_CUDA(cudaMalloc(&op->ucoords, u.size() * sizeof(double)));
-        GSI_CUDA(cudaMemcpyAsync(op->ucoords, u.data(), u.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        GSI_CUDA(cudaStreamSynchronize(ctx->stream));
-        set_partition(op.get());
-        ctx_retain(ctx);
-        *out = op.release();
+        make_kernelcov(ctx, n, coords, single_structure(kind, d, ell, sigma2, beta), nugget, row0, mloc, out);
     });
 }
 
@@ -549,62 +741,35 @@ GSI_API int32_t gsi_op_kernelcov_grid(gsi_ctx* ctx, int32_t kind, int32_t d, con
         GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov_grid: d must be 1, 2 or 3");
         GSI_REQUIRE(kind >= GSI_KERNEL_EXPONENTIAL && kind <= GSI_KERNEL_SPHERICAL, GSI_ERR_INVALID_ARGUMENT,
                     "kernelcov_grid: unknown kernel kind");
-        int64_t nd[3] = {1, 1, 1};
-        double h[3] = {1, 1, 1}, el[3] = {1, 1, 1};
-        int64_t n = 1;
-        for (int k = 0; k < d; ++k) {
+        for (int k = 0; k < d; ++k)
             GSI_REQUIRE(dims[k] >= 1 && ell[k] > 0.0, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad dims / length scales");
-            nd[k] = dims[k]; h[k] = spacing[k]; el[k] = ell[k];
-            n *= dims[k];
-        }
-        GSI_REQUIRE(n < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: more than 2^31 points");
-        GSI_REQUIRE(row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad row block");
-        std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
-        op->ctx = ctx; op->type = OP_KERNELCOV; op->kind = kind; op->dim = d;
-        op->m = op->n = n; op->row0 = row0; op->mloc = mloc;
-        op->sigma2 = sigma2; op->nugget = nugget; op->beta = beta;
-        op->n_pad = round_up(n, kRowPad);
-        op->grid_nx = (int)nd[0]; op->grid_ny = (int)nd[1]; op->grid_nz = (int)nd[2];
-        // kernel value of every lattice offset (libm, same formula as the dense definition)
-        std::vector<double> tab((size_t)n);
-        for (int64_t dz = 0; dz < nd[2]; ++dz)
-            for (int64_t dy = 0; dy < nd[1]; ++dy)
-                for (int64_t dx = 0; dx < nd[0]; ++dx) {
-                    const double ux = (dx * h[0]) / el[0], uy = (dy * h[1]) / el[1], uz = (dz * h[2]) / el[2];
-                    double r2 = ux * ux;
-                    if (d > 1) r2 += uy * uy;
-                    if (d > 2) r2 += uz * uz;
-                    double v;
-                    if (kind == GSI_KERNEL_EXPONENTIAL) v = std::exp(-std::sqrt(r2));
-                    else if (kind == GSI_KERNEL_GAUSSIAN) v = std::exp(-0.5 * r2);
-                    else if (kind == GSI_KERNEL_MATERN32) {
-                        const double s = std::sqrt(3.0 * r2);
-                        v = (1.0 + s) * std::exp(-s);
-                    } else if (kind == GSI_KERNEL_MATERN52) {
-                        const double s = std::sqrt(5.0 * r2);
-                        v = (1.0 + s + s * s / 3.0) * std::exp(-s);
-                    } else if (kind == GSI_KERNEL_SPHERICAL) {
-                        const double r = std::sqrt(r2);
-                        v = r < 1.0 ? 0.5 * (1.0 - r) * (1.0 - r) * (2.0 + r) : 0.0;   // = 1 - 1.5 r + 0.5 r^3, no cancellation
-                    } else v = std::exp(-beta * std::log1p(r2));
-                    tab[(size_t)(dx + nd[0] * (dy + nd[1] * dz))] = v;
-                }
-        // lattice indices of every point (SoA, padding repeats the last point)
-        std::vector<int> lat((size_t)3 * op->n_pad, 0);
-        for (int64_t j = 0; j < op->n_pad; ++j) {
-            const int64_t jj = j < n ? j : n - 1;
-            lat[(size_t)0 * op->n_pad + j] = (int)(jj % nd[0]);
-            lat[(size_t)1 * op->n_pad + j] = (int)((jj / nd[0]) % nd[1]);
-            lat[(size_t)2 * op->n_pad + j] = (int)(jj / (nd[0] * nd[1]));
-        }
-        GSI_CUDA(cudaMalloc(&op->table, tab.size() * sizeof(double)));
-        GSI_CUDA(cudaMalloc(&op->lattice, lat.size() * sizeof(int)));
-        GSI_CUDA(cudaMemcpyAsync(op->table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-        GSI_CUDA(cudaMemcpyAsync(op->lattice, lat.data(), lat.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-        GSI_CUDA(cudaStreamSynchronize(ctx->stream));
-        set_partition(op.get());
-        ctx_retain(ctx);
-        *out = op.release();
+        make_kernelcov_grid(ctx, dims, spacing, single_structure(kind, d, ell, sigma2, beta), nugget, row0, mloc, out);
+    });
+}
+
+GSI_API int32_t gsi_op_kernelcov_model(gsi_ctx* ctx, int32_t d, int64_t n, const double* coords, int32_t nstruct,
+                                       const int32_t* kinds, const double* sills, const double* ranges,
+                                       const double* rotations, const double* betas, double nugget, int64_t row0,
+                                       int64_t mloc, gsi_op** out) {
+    return guarded([&] {
+        use(ctx);
+        GSI_REQUIRE(coords && kinds && sills && ranges && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov_model: d must be 1, 2 or 3");
+        const CovModel m = model_from_args(d, nstruct, kinds, sills, ranges, rotations, betas);
+        make_kernelcov(ctx, n, coords, m, nugget, row0, mloc, out);
+    });
+}
+
+GSI_API int32_t gsi_op_kernelcov_model_grid(gsi_ctx* ctx, int32_t d, const int64_t* dims, const double* spacing,
+                                            int32_t nstruct, const int32_t* kinds, const double* sills,
+                                            const double* ranges, const double* rotations, const double* betas,
+                                            double nugget, int64_t row0, int64_t mloc, gsi_op** out) {
+    return guarded([&] {
+        use(ctx);
+        GSI_REQUIRE(dims && spacing && kinds && sills && ranges && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov_model_grid: d must be 1, 2 or 3");
+        const CovModel m = model_from_args(d, nstruct, kinds, sills, ranges, rotations, betas);
+        make_kernelcov_grid(ctx, dims, spacing, m, nugget, row0, mloc, out);
     });
 }
 

@@ -128,6 +128,11 @@ struct gsi_buf {
     }
 };
 
+// internal covariance kinds of the matrix-free product kernel (outside the public GSI_KERNEL_* range 0..5)
+constexpr int KC_KIND_MODEL = 13;         // nested model: sum of structures, each with its own kind and coordinates
+constexpr int KC_KIND_TABLE_SIGNED = 14;  // structured grid, table over signed lattice offsets (rotated anisotropy)
+constexpr int KC_KIND_TABLE = 15;         // structured grid, table over |lattice offsets|
+
 enum OpType { OP_DENSE = 0, OP_LOWRANKCOV = 1, OP_KERNELCOV = 2 };
 
 struct gsi_op {
@@ -147,6 +152,11 @@ struct gsi_op {
     int* lattice = nullptr;              // structured grid: [3][n_pad] lattice indices
     double* table = nullptr;             // structured grid: kernel value per lattice offset
     int grid_nx = 1, grid_ny = 1, grid_nz = 1;
+    bool table_signed = false;           // structured grid: the table covers signed offsets (rotated model)
+    // nested model generated in the kernel (kind == KC_KIND_MODEL): ucoords is [nstruct][3][n_pad]
+    int32_t nstruct = 1;
+    int32_t mkinds[GSI_MODEL_MAX_STRUCTURES] = {0, 0, 0, 0};
+    double msills[GSI_MODEL_MAX_STRUCTURES] = {0, 0, 0, 0}, mbetas[GSI_MODEL_MAX_STRUCTURES] = {1, 1, 1, 1};
     std::vector<int64_t> part;           // row partition over ranks: part[r] .. part[r+1]
 };
 

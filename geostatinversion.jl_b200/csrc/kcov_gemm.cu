@@ -33,11 +33,9 @@ constexpr int KC_AP = KC_BK + 4;   // pitch of the generated A tile (4 mod 16 do
 constexpr int KC_WARPS = 16;
 constexpr int KC_THREADS = KC_WARPS * 32;
 constexpr int KC_CG = 4;           // column groups (warps sharing one row group)
-constexpr int KC_KIND_TABLE = 15;  // internal kind: stationary kernel on a structured grid, values from a lattice table
-                                   // (outside the public GSI_KERNEL_* range)
 constexpr long long KC_SPIN_LIMIT = 400000;   // cycles (~0.2 ms) a producer waits on the sweep window before giving it up
 
-struct KcovParams {
+struct KcovBase {
     const double* X;       // TALL, all n rows (zero padded), pitch ld
     double* W;             // TALL, local rows, pitch ldw
     const double* u;       // scaled coordinates [3][n_pad]              (arithmetic generation)
@@ -60,6 +58,19 @@ struct KcovParams {
     int64_t tail_u;        // k-tiles of tail work per CTA (0: no tail)
     double* partial;       // [2 * grid][KC_BM][ldw] raw accumulators of the tail segments (slot 2b + s)
 };
+// the product kernel's parameters: KcovBase (all the tail fix-up reads) with the nested model appended
+struct KcovParams : KcovBase {
+    // nested model (KC_KIND_MODEL): u is [nstruct][3][n_pad], value = sum_s sill_s * k_{kind_s}(r2_s)
+    int nstruct;
+    int mkinds[GSI_MODEL_MAX_STRUCTURES];
+    double msills[GSI_MODEL_MAX_STRUCTURES], mbetas[GSI_MODEL_MAX_STRUCTURES];
+};
+
+template <int KIND>
+__host__ __device__ constexpr bool kind_is_table() { return KIND == KC_KIND_TABLE || KIND == KC_KIND_TABLE_SIGNED; }
+// coordinate doubles of one k-tile in a pipeline stage (the model carries up to GSI_MODEL_MAX_STRUCTURES sets)
+template <int KIND>
+__host__ __device__ constexpr int kc_coord_doubles() { return (KIND == KC_KIND_MODEL ? GSI_MODEL_MAX_STRUCTURES : 1) * 3 * KC_BK; }
 
 // 2^(j/64), j = 0..63, correctly rounded (generated with 200-bit arithmetic)
 __constant__ double kExp2Table[64] = {
@@ -178,8 +189,47 @@ __device__ __forceinline__ double kern_eval(double r2, double beta, const double
         const double t = 1.0 - s;
         return s < 1.0 ? (0.5 * t) * t * (2.0 + s) : 0.0;      // 0.5 (1 - s)^2 (2 + s)
     }
-    if (KIND == KC_KIND_TABLE) return 0.0;
+    if (kind_is_table<KIND>() || KIND == KC_KIND_MODEL) return 0.0;
     return exp(-beta * log1p(r2));
+}
+
+// Nested model (KC_KIND_MODEL): v = sum_s fma(c_s, kern_eval<kind_s>(r2_s), v), s = 0..nstruct-1, the kind decided at run
+// time (warp-uniform: one model per launch).  r2_s = sum_k (ui[s][k] - uj[s][k])^2 by the same fma chain as the single
+// kinds.  Error bound: every term is >= 0 (c_s > 0, k >= 0), so nothing cancels.  With b_s the bound of kind_s in ulps of
+// its own exact value k_s (above; 2.5 + 4 y exponential, 2.5 Gaussian, 2 + 4 |z| power law, 6 / 8.5 / 5 + 4 k Matern 3/2,
+// 5/2, spherical) each term carries a relative error b_s 2^-52 and the S roundings of the fma chain add gamma_S <= S 2^-53
+// relative to the sum v:  |v_hat - v| <= 2^-52 sum_s c_s k_s b_s + gamma_S v,  i.e. in ulps of v at most
+// 2 sum_s (c_s k_s / v) b_s + S <= 2 max_s b_s + S.  tests/test_gpu_kcov_model.py asserts the weighted form value by value.
+// Two identical structures with c = 0.5 give 0.5 k + 0.5 k = k exactly, the single kind's value bit for bit.
+__device__ __forceinline__ double kern_eval_runtime(int kind, double r2, double beta, const double* __restrict__ tab) {
+    switch (kind) {
+        case GSI_KERNEL_EXPONENTIAL: return kern_eval<GSI_KERNEL_EXPONENTIAL>(r2, beta, tab);
+        case GSI_KERNEL_GAUSSIAN: return kern_eval<GSI_KERNEL_GAUSSIAN>(r2, beta, tab);
+        case GSI_KERNEL_MATERN32: return kern_eval<GSI_KERNEL_MATERN32>(r2, beta, tab);
+        case GSI_KERNEL_MATERN52: return kern_eval<GSI_KERNEL_MATERN52>(r2, beta, tab);
+        case GSI_KERNEL_SPHERICAL: return kern_eval<GSI_KERNEL_SPHERICAL>(r2, beta, tab);
+        default: return kern_eval<GSI_KERNEL_POWERLAW>(r2, beta, tab);
+    }
+}
+__device__ __forceinline__ bool kind_takes_sqrt_runtime(int kind) { return kind != GSI_KERNEL_GAUSSIAN && kind != GSI_KERNEL_POWERLAW; }
+
+// ui: the row's coordinates [nstruct][DIM] (shared memory); uj: column point of structure 0, coordinate k, at
+// uj[k * kstride], structure s at + s * sstride
+template <int DIM>
+__device__ __forceinline__ double model_value(const KcovParams& p, const double* ui, const double* uj, int64_t kstride,
+                                              int64_t sstride, const double* __restrict__ tab) {
+    double v = 0.0;
+    for (int s = 0; s < p.nstruct; ++s) {
+        const int kind = p.mkinds[s];
+        double r2 = kind_takes_sqrt_runtime(kind) ? 1e-300 : 0.0;
+#pragma unroll
+        for (int k = 0; k < DIM; ++k) {
+            const double dk = ui[s * DIM + k] - uj[s * sstride + k * kstride];
+            r2 = fma(dk, dk, r2);
+        }
+        v = fma(p.msills[s], kern_eval_runtime(kind, r2, p.mbetas[s], tab), v);
+    }
+    return v;
 }
 
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
@@ -195,12 +245,30 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
 // (sweep window) hammer the same L2 lines in the same order -- made every schedule slower (windowed front 563 ->
 // 623 / 652 / 836 ms, default 516 -> 559 ms: the per-copy cost outweighs any spreading; gpurun_out r03_chunks.log);
 // removed as well.)
+// Signed lattice table (KC_KIND_TABLE_SIGNED): index of the offset li - lj, folded by central symmetry -- the last axis
+// stored as |delta|, every component negated when that delta is negative, the other axes shifted by n - 1 into
+// 0 .. 2n - 2.  Integer ALU only; unsigned because 2 n - 1 may reach 2^31 - 1 (the index itself is < 2^31).  Column
+// point c: lattice index k at col[k * stride + c]
+template <int DIM>
+__device__ __forceinline__ int signed_table_index(const int (&li)[DIM], const int* col, int64_t stride, int c, int nx, int ny) {
+    const int dl = li[DIM - 1] - col[(DIM - 1) * stride + c];
+    const bool neg = dl < 0;
+    unsigned idx = (unsigned)(neg ? -dl : dl);
+#pragma unroll
+    for (int k = DIM - 2; k >= 0; --k) {
+        const int dk = li[k] - col[k * stride + c];
+        const unsigned nk = (unsigned)(k == 0 ? nx : ny);
+        idx = idx * (2u * nk - 1u) + (unsigned)(neg ? -dk : dk) + (nk - 1u);
+    }
+    return (int)idx;
+}
+
 template <int NB, int KIND, int DIM>
 __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_constant__ KcovParams p) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int ld = NB * 8 + 4;
     constexpr int NBW = (NB + KC_CG - 1) / KC_CG;                // n-blocks per warp
-    constexpr int stage_doubles = KC_BK * ld + 3 * KC_BK;        // X tile + coordinate tile
+    constexpr int stage_doubles = KC_BK * ld + kc_coord_doubles<KIND>();   // X tile + coordinate tile
     constexpr int a_doubles = KC_BM * KC_AP;
     double* smem = reinterpret_cast<double*>(smem_raw);
     double* a_tiles = smem + (size_t)p.stages * stage_doubles;   // [2][KC_BM][KC_AP]
@@ -318,8 +386,9 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
     };
     bool window_on = p.win_epochs > 0;            // thread 0 only
     const uint64_t xpolicy = l2_policy_evict_last();
-    constexpr uint32_t stage_bytes = (uint32_t)(KC_BK * ld * sizeof(double) +
-                                                DIM * KC_BK * (KIND == KC_KIND_TABLE ? sizeof(int) : sizeof(double)));
+    const uint32_t stage_bytes = (uint32_t)(KC_BK * ld * sizeof(double) +
+                                            (KIND == KC_KIND_MODEL ? p.nstruct : 1) * DIM * KC_BK *
+                                                (kind_is_table<KIND>() ? sizeof(int) : sizeof(double)));
 
     // ---------------- producer (thread 0): streams X / coordinate tiles ----------------------
     const int64_t total_it = full_it + (u1 - u0);
@@ -374,10 +443,14 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
         mbar_expect_tx(&full[p_s], stage_bytes);
         if (p.l2_hint) bulk_g2s_hint(xs, p.X + kt * KC_BK * p.ld, KC_BK * ld * 8, &full[p_s], xpolicy);
         else bulk_g2s(xs, p.X + kt * KC_BK * p.ld, KC_BK * ld * 8, &full[p_s]);
-        if (KIND == KC_KIND_TABLE) {
+        if (kind_is_table<KIND>()) {
             int* usi = reinterpret_cast<int*>(us);
             for (int k = 0; k < DIM; ++k)
                 bulk_g2s(usi + k * KC_BK, p.lat + k * p.n_pad + ktn * KC_BK, KC_BK * 4, &full[p_s]);
+        } else if (KIND == KC_KIND_MODEL) {
+            for (int s = 0; s < p.nstruct; ++s)
+                for (int k = 0; k < DIM; ++k)
+                    bulk_g2s(us + (s * DIM + k) * KC_BK, p.u + (s * 3 + k) * p.n_pad + ktn * KC_BK, KC_BK * 8, &full[p_s]);
         } else {
             for (int k = 0; k < DIM; ++k)
                 bulk_g2s(us + k * KC_BK, p.u + k * p.n_pad + ktn * KC_BK, KC_BK * 8, &full[p_s]);
@@ -408,12 +481,25 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
     auto row_coords = [&](int64_t base_rg, double (&ui)[DIM]) {
         int64_t gpt = p.row0 + base_rg * 16 + grow_in_tile;           // global point of my generated row
         if (gpt > p.n - 1) gpt = p.n - 1;                             // tail rows: clamp (never stored)
+        if constexpr (KIND == KC_KIND_MODEL) {
+            // the row's nstruct * DIM coordinates go to shared memory, [KC_BM][GSI_MODEL_MAX_STRUCTURES * DIM] after
+            // etab (they do not fit the register budget): the 8 threads of a row, all in this warp, load them
+            // together; only this warp reads them
+            __syncwarp();
+            for (int q = gtid & 7; q < p.nstruct * DIM; q += 8) {
+                const int s = q / DIM, k = q - s * DIM;
+                etab[64 + grow_in_tile * (GSI_MODEL_MAX_STRUCTURES * DIM) + q] = p.u[(s * 3 + k) * p.n_pad + gpt];
+            }
+            __syncwarp();
+        } else {
 #pragma unroll
-        for (int k = 0; k < DIM; ++k) {
-            if (KIND == KC_KIND_TABLE) li[k] = p.lat[k * p.n_pad + gpt];
-            else ui[k] = p.u[k * p.n_pad + gpt];
+            for (int k = 0; k < DIM; ++k) {
+                if (kind_is_table<KIND>()) li[k] = p.lat[k * p.n_pad + gpt];
+                else ui[k] = p.u[k * p.n_pad + gpt];
+            }
         }
     };
+
     // table variant: lattice offset of (my row, column point e of the tile) -> table index
     auto table_index = [&](const int* usi, int e) -> int {
         int idx = 0;
@@ -466,6 +552,15 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
                     }
                     v[e] = __ldg(p.table + idx);
                 }
+            } else if constexpr (KIND == KC_KIND_TABLE_SIGNED) {
+#pragma unroll
+                for (int e = 0; e < 4; ++e)
+                    v[e] = __ldg(p.table + signed_table_index<DIM>(li, p.lat + ktf * KC_BK, p.n_pad, gcol(e), p.nx, p.ny));
+            } else if constexpr (KIND == KC_KIND_MODEL) {
+                const double* urow = etab + 64 + grow_in_tile * (GSI_MODEL_MAX_STRUCTURES * DIM);
+#pragma unroll
+                for (int e = 0; e < 4; ++e)
+                    v[e] = model_value<DIM>(p, urow, p.u + ktf * KC_BK + gcol(e), p.n_pad, 3 * p.n_pad, etab);
             } else {
                 gen4(ui, p.u + ktf * KC_BK, p.n_pad, v);
             }
@@ -513,12 +608,17 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
             }
             double* anext = a_tiles + (size_t)(par ^ 1) * a_doubles + grow_in_tile * KC_AP + gj0;
             double tv[4] = {0.0, 0.0, 0.0, 0.0};
-            if (KIND == KC_KIND_TABLE && gen_next) {
+            if (kind_is_table<KIND>() && gen_next) {
                 // structured grid: the four kernel values are table look-ups (L1/L2 hits, no FP64 pipe
                 // work); issued now, consumed after the MMA loop
                 const int* usi = reinterpret_cast<const int*>(us);
 #pragma unroll
-                for (int e = 0; e < 4; ++e) tv[e] = __ldg(p.table + table_index(usi, e));
+                for (int e = 0; e < 4; ++e) {
+                    if constexpr (KIND == KC_KIND_TABLE_SIGNED)
+                        tv[e] = __ldg(p.table + signed_table_index<DIM>(li, usi, KC_BK, gcol(e), p.nx, p.ny));
+                    else
+                        tv[e] = __ldg(p.table + table_index(usi, e));
+                }
             }
             // ---- tensor-core phase on the current k-tile: wait until the whole row group has
             //      published this block (and has stopped reading the other buffer)
@@ -530,7 +630,14 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
             for (int ks = 0; ks < KC_BK / 4; ++ks) {
                 // one kernel value of the NEXT block every second k-step: a single exp chain
                 // is live at a time and its DFMAs interleave with this step's DMMAs
-                if (KIND != KC_KIND_TABLE && (ks & 1) == 0 && gen_next) {
+                if constexpr (KIND == KC_KIND_MODEL) {
+                    if ((ks & 1) == 0 && gen_next) {
+                        const int e = ks >> 1;
+                        const double* urow = etab + 64 + grow_in_tile * (GSI_MODEL_MAX_STRUCTURES * DIM);
+                        anext[(e & 1) + ((e >> 1) << 4)] = model_value<DIM>(p, urow, us + gcol(e), KC_BK, DIM * KC_BK, etab);
+                    }
+                }
+                if (!kind_is_table<KIND>() && KIND != KC_KIND_MODEL && (ks & 1) == 0 && gen_next) {
                     const int e = ks >> 1;
                     double r2 = kind_takes_sqrt<KIND>() ? 1e-300 : 0.0;
 #pragma unroll
@@ -554,7 +661,7 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
                     }
                 }
             }
-            if (KIND == KC_KIND_TABLE && gen_next) {
+            if (kind_is_table<KIND>() && gen_next) {
                 double2* dst = reinterpret_cast<double2*>(anext);
                 dst[0] = make_double2(tv[0], tv[1]);
                 dst[8] = make_double2(tv[2], tv[3]);
@@ -611,7 +718,7 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
 // round-2 version divided 64-bit integers per piece and element on 9 CTAs: 141 us for 9 tiles at n = 10 000).
 constexpr int KF_ROWS = 8;
 constexpr int KF_MAX_PIECES = 160;     // pieces of one tile <= CTAs of the main grid (<= SMs, checked at launch)
-__global__ void kcov_tail_fixup_kernel(KcovParams p, int64_t nkt, int64_t tail_rg0, int grid_main, int cols) {
+__global__ void kcov_tail_fixup_kernel(KcovBase p, int64_t nkt, int64_t tail_rg0, int grid_main, int cols) {
     __shared__ int s_slot[KF_MAX_PIECES];
     const int64_t tile = blockIdx.x;
     const int64_t ulo = tile * nkt, uhi = ulo + nkt;                  // this tile's units
@@ -644,13 +751,14 @@ template <int NB, int KIND, int DIM>
 static void launch_kcov(gsi_ctx* ctx, const KcovParams& p0) {
     KcovParams p = p0;
     const int ld = NB * 8 + 4;
-    const size_t stage_bytes = (size_t)(KC_BK * ld + 3 * KC_BK) * sizeof(double);
+    const size_t stage_bytes = (size_t)(KC_BK * ld + kc_coord_doubles<KIND>()) * sizeof(double);
     const size_t a_bytes = (size_t)2 * KC_BM * KC_AP * sizeof(double);
     int stages = (int)((224 * 1024 - a_bytes - 1024) / stage_bytes);
     if (stages > 4) stages = 4;
     if (stages < 2) stages = 2;
     p.stages = stages;
-    const size_t smem = stages * stage_bytes + a_bytes + (2 * stages + 4) * sizeof(uint64_t) + 64 * sizeof(double);
+    const size_t urow_bytes = KIND == KC_KIND_MODEL ? (size_t)KC_BM * GSI_MODEL_MAX_STRUCTURES * DIM * sizeof(double) : 0;
+    const size_t smem = stages * stage_bytes + a_bytes + (2 * stages + 4) * sizeof(uint64_t) + 64 * sizeof(double) + urow_bytes;
     auto kfn = kcov_gemm_kernel<NB, KIND, DIM>;
     GSI_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
@@ -719,6 +827,8 @@ static void dispatch_kind(gsi_ctx* ctx, const KcovParams& p, int kind, int dim) 
         case GSI_KERNEL_MATERN52: dispatch_dim<NB, GSI_KERNEL_MATERN52>(ctx, p, dim); break;
         case GSI_KERNEL_SPHERICAL: dispatch_dim<NB, GSI_KERNEL_SPHERICAL>(ctx, p, dim); break;
         case KC_KIND_TABLE: dispatch_dim<NB, KC_KIND_TABLE>(ctx, p, dim); break;
+        case KC_KIND_TABLE_SIGNED: dispatch_dim<NB, KC_KIND_TABLE_SIGNED>(ctx, p, dim); break;
+        case KC_KIND_MODEL: dispatch_dim<NB, KC_KIND_MODEL>(ctx, p, dim); break;
         default: throw Error(GSI_ERR_INVALID_ARGUMENT, "unknown covariance kernel kind");
     }
 }
@@ -752,8 +862,13 @@ void kcov_apply(gsi_op* op, const gsi_buf* X, gsi_buf* W) {
     p.ld = X->ld; p.ldw = W->ld;
     p.sigma2 = op->sigma2; p.nugget = op->nugget; p.beta = op->beta;
     p.stages = 0;
+    p.nstruct = op->nstruct;
+    for (int s = 0; s < GSI_MODEL_MAX_STRUCTURES; ++s) {
+        p.mkinds[s] = op->mkinds[s]; p.msills[s] = op->msills[s]; p.mbetas[s] = op->mbetas[s];
+    }
+    const int kind = op->table ? (op->table_signed ? KC_KIND_TABLE_SIGNED : KC_KIND_TABLE) : op->kind;
     switch (nb) {
-#define GSI_CASE(N) case N: dispatch_kind<N>(ctx, p, op->table ? KC_KIND_TABLE : op->kind, op->dim); break;
+#define GSI_CASE(N) case N: dispatch_kind<N>(ctx, p, kind, op->dim); break;
         GSI_NB_LIST(GSI_CASE)
 #undef GSI_CASE
         default: throw Error(GSI_ERR_UNSUPPORTED, "kernelcov apply: unsupported column-block count");

@@ -178,6 +178,34 @@ int32_t gsi_op_kernelcov(gsi_ctx* ctx, int32_t kind, int32_t d, int64_t n, const
 int32_t gsi_op_kernelcov_grid(gsi_ctx* ctx, int32_t kind, int32_t d, const int64_t* dims,
                               const double* spacing, const double* ell, double sigma2, double nugget,
                               double beta, int64_t row0, int64_t mloc, gsi_op** out);
+/* Nested covariance models with rotated (geometric) anisotropy: the same operator for a sum of
+ * 1 <= nstruct <= GSI_MODEL_MAX_STRUCTURES structures (e.g. nugget + spherical + exponential, as GSLIB,
+ * gstools and SGeMS model a fitted variogram).  Structure s has kinds[s] (GSI_KERNEL_*), a sill
+ * sills[s] > 0, ranges ranges[s*d .. s*d+d) > 0 along its principal axes, an orthonormal d x d
+ * rotation R_s = rotations + s*d*d (column-major; rotations == NULL: every R_s = I) and betas[s]
+ * (power law only; betas == NULL: 1).  With pre(kind) the coordinate scaling of gsi_op_kernelcov
+ * (1/sqrt(2) Gaussian, sqrt(3) / sqrt(5) Matern, else 1):
+ *   u_s,k(x)  = ((sum_j R_s[k,j] x_j) / ranges[s*d+k]) * pre(kinds[s])       (j = 0..d-1 in order)
+ *   r2_s(i,j) = sum_k (u_s,k(x_i) - u_s,k(x_j))^2
+ *   C[i,j]    = sum_s sills[s] * k_kinds[s](r2_s) + nugget * (i == j)
+ * With R_s = I the coordinates are bit-identical to gsi_op_kernelcov's (x / ell) * pre, and one
+ * structure gives gsi_op_kernelcov's operator with sigma2 = sills[0].  Invalid nstruct, kinds,
+ * sills (<= 0 or not finite), ranges (<= 0) or rotations (not finite, or max |R'R - I| > 1e-12):
+ * GSI_ERR_INVALID_ARGUMENT; d outside 1..3: GSI_ERR_UNSUPPORTED.                                */
+#define GSI_MODEL_MAX_STRUCTURES 4
+int32_t gsi_op_kernelcov_model(gsi_ctx* ctx, int32_t d, int64_t n, const double* coords, int32_t nstruct,
+                               const int32_t* kinds, const double* sills, const double* ranges,
+                               const double* rotations, const double* betas, double nugget,
+                               int64_t row0, int64_t mloc, gsi_op** out);
+/* The nested model on a structured grid (dims / spacing as gsi_op_kernelcov_grid): the whole model is
+ * tabulated once on the host.  Without rotations (or d = 1) the table is indexed by |lattice offset|;
+ * a rotated model is not symmetric in each axis, so its table covers the signed offsets, folded by
+ * k(delta) = k(-delta): (2 dims[0] - 1) (2 dims[1] - 1) dims[2] entries in 3-D, (2 dims[0] - 1) dims[1]
+ * in 2-D (GSI_ERR_UNSUPPORTED at 2^31 entries or more).                                           */
+int32_t gsi_op_kernelcov_model_grid(gsi_ctx* ctx, int32_t d, const int64_t* dims, const double* spacing,
+                                    int32_t nstruct, const int32_t* kinds, const double* sills,
+                                    const double* ranges, const double* rotations, const double* betas,
+                                    double nugget, int64_t row0, int64_t mloc, gsi_op** out);
 int32_t gsi_op_free(gsi_op* op);
 /* size(A) (src/RandMatFact.jl:52-53, src/lowrank.jl:50-60)                           */
 int32_t gsi_op_size(const gsi_op* op, int64_t* m, int64_t* n);

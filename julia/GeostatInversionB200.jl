@@ -187,6 +187,47 @@ function KernelCovGrid(kind::Integer, dims::Vector{Int}, spacing::Vector{Float64
 	return op
 end
 
+"""Nested covariance model (gsi_op_kernelcov_model): C = sum_s sills[s] k_{kinds[s]} + nugget I, 1 to
+GSI_MODEL_MAX_STRUCTURES structures.  ranges d x nstruct; rotations d x d x nstruct (u = R x, orthonormal) or
+`nothing` (no rotation); betas (power law) or `nothing` (1)."""
+function KernelCovModel(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, coords::Matrix{Float64};
+		rotations::Union{Nothing, Array{Float64, 3}}=nothing, betas::Union{Nothing, Vector{Float64}}=nothing, nugget=0.0,
+		ctx::Context=context(), rows::UnitRange{Int}=partitionrows(size(coords, 2), ctx.world, ctx.rank))
+	d, n = size(coords)
+	kinds32 = Int32.(kinds)
+	rot = rotations === nothing ? Ptr{Float64}(C_NULL) : pointer(rotations)
+	bet = betas === nothing ? Ptr{Float64}(C_NULL) : pointer(betas)
+	out = Ref{Ptr{Cvoid}}(C_NULL)
+	GC.@preserve coords kinds32 sills ranges rotations betas check(ccall((:gsi_op_kernelcov_model, LIB), Int32,
+		(Ptr{Cvoid}, Int32, Int64, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+		 Float64, Int64, Int64, Ref{Ptr{Cvoid}}),
+		ctx.h, d, n, coords, length(kinds32), kinds32, sills, ranges, rot, bet, nugget, first(rows) - 1, length(rows), out))
+	op = KernelCovMatrix(out[], n, ctx, rows)
+	finalizer(freeop, op)
+	return op
+end
+
+"structured grid variant of KernelCovModel (the model is tabulated once per lattice offset)"
+function KernelCovModelGrid(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, dims::Vector{Int},
+		spacing::Vector{Float64}; rotations::Union{Nothing, Array{Float64, 3}}=nothing,
+		betas::Union{Nothing, Vector{Float64}}=nothing, nugget=0.0,
+		ctx::Context=context(), rows::UnitRange{Int}=partitionrows(prod(dims), ctx.world, ctx.rank))
+	d = length(dims)
+	n = prod(dims)
+	dims64 = Int64.(dims)
+	kinds32 = Int32.(kinds)
+	rot = rotations === nothing ? Ptr{Float64}(C_NULL) : pointer(rotations)
+	bet = betas === nothing ? Ptr{Float64}(C_NULL) : pointer(betas)
+	out = Ref{Ptr{Cvoid}}(C_NULL)
+	GC.@preserve dims64 spacing kinds32 sills ranges rotations betas check(ccall((:gsi_op_kernelcov_model_grid, LIB), Int32,
+		(Ptr{Cvoid}, Int32, Ptr{Int64}, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+		 Float64, Int64, Int64, Ref{Ptr{Cvoid}}),
+		ctx.h, d, dims64, spacing, length(kinds32), kinds32, sills, ranges, rot, bet, nugget, first(rows) - 1, length(rows), out))
+	op = KernelCovMatrix(out[], n, ctx, rows)
+	finalizer(freeop, op)
+	return op
+end
+
 "LowRankCovMatrix(samples) -- src/lowrank.jl:14-30 (the mean is removed on the device)"
 function LowRankCovMatrix(samples::Vector{Vector{Float64}}; ctx::Context=context())
 	S = reduce(hcat, samples)

@@ -12,7 +12,7 @@ from ._lib import (GsiError, SingularException, PosDefException, DimensionMismat
                    NORMALISER_QR)
 from .core import (Context, DeviceMatrix, DenseMatrix, LowRankCovMatrix, KernelCovMatrix, GridKernelCovMatrix, default_context,
                    set_default_context, as_operator, partition_rows, CovStructure, rotation_matrix, KernelCovModelMatrix,
-                   GridKernelCovModelMatrix)
+                   GridKernelCovModelMatrix, KernelCrossCovMatrix, GridKernelCrossCovMatrix)
 from . import randmatfact as RandMatFact
 from .randmatfact import randsvd, rangefinder, eig_nystrom
 from . import dist

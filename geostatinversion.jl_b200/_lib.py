@@ -75,6 +75,9 @@ SIGNATURES = {
     "gsi_op_kernelcov_model": (_i32, [_p, _i32, _i64, _pd, _i32, _pi32, _pd, _pd, _pd, _pd, _f64, _i64, _i64, _pp]),
     "gsi_op_kernelcov_model_grid": (_i32, [_p, _i32, _pi64, _pd, _i32, _pi32, _pd, _pd, _pd, _pd, _f64, _i64, _i64,
                                            _pp]),
+    "gsi_op_kernelcov_cross": (_i32, [_p, _i32, _i64, _pd, _i64, _pd, _i32, _pi32, _pd, _pd, _pd, _pd, _i64, _i64, _pp]),
+    "gsi_op_kernelcov_cross_grid": (_i32, [_p, _i32, _pi64, _pd, _i64, _pi64, _i64, _pi64, _i32, _pi32, _pd, _pd, _pd,
+                                           _pd, _i64, _i64, _pp]),
     "gsi_op_free": (_i32, [_p]),
     "gsi_op_size": (_i32, [_p, _pi64, _pi64]),
     "gsi_op_apply": (_i32, [_p, _i32, _p, _p]),

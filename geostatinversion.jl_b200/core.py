@@ -491,6 +491,62 @@ class GridKernelCovModelMatrix(_Operator):
                                                     self.mloc, C.byref(self._h)))
 
 
+class KernelCrossCovMatrix(_Operator):
+    """Matrix-free cross-covariance C(T, S) of a nested model between targets T (d x m) and sources S (d x n)
+    (gsi_op_kernelcov_cross): C[i,j] = sum_s sill_s k_s(t_i, s_j), no nugget.  Kriging / conditioning is C(T, S) w;
+    with point observations H, Q H' = C(grid, obs).  Not symmetric: A.T @ X (or X' @ A) is C(S, T) X, on a multi-rank
+    context summed over the ranks, each of which owns the target rows [row0, row0 + mloc)."""
+    symmetric = False
+
+    def __init__(self, structures, targets, sources, ctx=None, row0=0, mloc=None):
+        super().__init__(ctx or default_context())
+        targets, sources = _f64_colmajor(targets), _f64_colmajor(sources)
+        d, m = targets.shape
+        if sources.shape[0] != d:
+            raise ValueError(f"KernelCrossCovMatrix: targets are {d}-D, sources {sources.shape[0]}-D")
+        n = sources.shape[1]
+        self.row0 = int(row0)
+        self.mloc = int(m - row0 if mloc is None else mloc)
+        args, self._keep = _model_args(structures, d)
+        check(self._lib.gsi_op_kernelcov_cross(self.ctx._h, d, m, _pd(targets), n, _pd(sources), *args, self.row0,
+                                               self.mloc, C.byref(self._h)))
+
+
+def _index_array(idx):
+    """(count, ctypes int64 array or None) of a list of 0-based linear grid indices (None: every node in order)."""
+    if idx is None:
+        return None, None
+    a = np.ascontiguousarray(np.asarray(idx, dtype=np.int64).ravel())
+    return a.size, a
+
+
+class GridKernelCrossCovMatrix(_Operator):
+    """KernelCrossCovMatrix for points that are nodes of one structured grid (as GridKernelCovModelMatrix), given by
+    0-based linear indices (shape[0] fastest); targets / sources None: every node in order.  The model is tabulated
+    once per lattice offset."""
+    symmetric = False
+
+    def __init__(self, structures, shape, targets=None, sources=None, spacing=None, ctx=None, row0=0, mloc=None):
+        super().__init__(ctx or default_context())
+        shape = [int(s) for s in shape]
+        d = len(shape)
+        nodes = int(np.prod(shape))
+        dims = (C.c_int64 * d)(*shape)
+        spacing = np.ascontiguousarray(np.broadcast_to(np.asarray(1.0 if spacing is None else spacing, dtype=np.float64), (d,)))
+        m, ti = _index_array(targets)
+        n, si = _index_array(sources)
+        m = nodes if m is None else m
+        n = nodes if n is None else n
+        pi64 = C.POINTER(C.c_int64)
+        self.row0 = int(row0)
+        self.mloc = int(m - row0 if mloc is None else mloc)
+        args, keep = _model_args(structures, d)
+        self._keep = (keep, ti, si)
+        check(self._lib.gsi_op_kernelcov_cross_grid(
+            self.ctx._h, d, dims, _pd(spacing), m, None if ti is None else ti.ctypes.data_as(pi64), n,
+            None if si is None else si.ctypes.data_as(pi64), *args, self.row0, self.mloc, C.byref(self._h)))
+
+
 def as_operator(A, ctx=None):
     if isinstance(A, _Operator):
         return A

@@ -80,14 +80,34 @@ void resolve_gemm_timing(gsi_ctx* ctx) {
 
 // Y = op(A) X.   X: all rows of the operand on this rank.  Output distribution:
 //   kernelcov / lowrankcov (symmetric): this rank's row block (SHARDED when world > 1)
-//   dense, trans = 0: this rank's row block;  trans = 1: all n rows, summed over ranks
+//   dense and cross-covariance, trans = 0: this rank's row block;  trans = 1: all n rows, summed over ranks
 void op_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* Y) {
     gsi_ctx* ctx = op->ctx;
     switch (op->type) {
         case OP_KERNELCOV: {
             timed_begin(ctx);
-            kcov_apply(op, X, Y);
+            kcov_apply(op, 0, X, Y);
             timed_end(ctx, 2.0 * (double)op->mloc * (double)op->n * (double)X->cols, 1);
+            break;
+        }
+        case OP_KERNELCROSS: {
+            // trans = 1 on several ranks: this rank's operand rows go to a zero-padded buffer of their own -- in a view
+            // into the full operand, the rows past mloc that the last k-tile's padded columns multiply are the next
+            // rank's data
+            BufPtr xl;
+            const gsi_buf* Xk = X;
+            if (trans && ctx->world > 1) {
+                GSI_REQUIRE(X->rows == op->m, GSI_ERR_DIMENSION_MISMATCH, "cross-covariance C'X: X must hold all m rows");
+                xl = make_buf(ctx, GSI_LAYOUT_TALL, op->mloc, X->cols);
+                GSI_REQUIRE(xl->ld == X->ld, GSI_ERR_INVALID_ARGUMENT, "cross-covariance C'X: bad pitch");
+                GSI_CUDA(cudaMemcpyAsync(xl->d, X->d + op->row0 * X->ld, (size_t)op->mloc * X->ld * 8,
+                                         cudaMemcpyDeviceToDevice, ctx->stream));
+                Xk = xl.get();
+            }
+            timed_begin(ctx);
+            kcov_apply(op, trans, Xk, Y);
+            timed_end(ctx, 2.0 * (double)op->mloc * (double)op->n * (double)X->cols, 1);
+            if (trans && ctx->world > 1) comm_allreduce_sum(ctx, Y->d, (size_t)Y->rows_alloc * Y->ld);
             break;
         }
         case OP_DENSE: {
@@ -152,7 +172,7 @@ static void gather_rows(gsi_op* op, const gsi_buf* loc, gsi_buf* full) {
     }
 }
 
-static bool op_symmetric(const gsi_op* op) { return op->type != OP_DENSE; }
+bool op_symmetric(const gsi_op* op) { return op->type != OP_DENSE && op->type != OP_KERNELCROSS; }
 
 // In-place LU normalisation of an iterate all of whose rows are on this device.
 static void normalise_lu(gsi_op* op, gsi_buf* Y) {

@@ -9,6 +9,7 @@ typedef std::unique_ptr<gsi_buf, BufDeleter> BufPtr;
 
 BufPtr make_buf(gsi_ctx* ctx, int32_t layout, int64_t rows, int64_t cols);
 void op_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* Y);
+bool op_symmetric(const gsi_op* op);
 void resolve_gemm_timing(gsi_ctx* ctx);
 BufPtr X_view_for_dense(gsi_op* op, int trans, const gsi_buf* X);
 void tsqr_thinQ(gsi_op* op, gsi_buf* Y, bool sharded, double* Rdev);

@@ -442,6 +442,8 @@ struct OpAbort {
         if (op->ucoords) cudaFree(op->ucoords);
         if (op->table) cudaFree(op->table);
         if (op->lattice) cudaFree(op->lattice);
+        if (op->ucoords_t) cudaFree(op->ucoords_t);
+        if (op->lattice_t) cudaFree(op->lattice_t);
         delete op;
     }
 };
@@ -632,85 +634,178 @@ static void set_model(gsi_op* op, const CovModel& m, double nugget, bool generat
     }
 }
 
+// scaled SoA coordinates u[s][k][j] of every structure (one structure: u[k][j]) of `count` points (point j at
+// coords + j * d) -> device array dst with pitch pad = round_up(count, kRowPad); the padding repeats the last point
+static void upload_coords(gsi_ctx* ctx, const CovModel& m, int64_t count, const double* coords, double*& dst,
+                          int64_t& pad) {
+    const int d = m.d;
+    pad = round_up(count, kRowPad);
+    if (count == 0) return;
+    std::vector<double> u((size_t)m.nstruct * 3 * pad, 0.0);
+    for (int s = 0; s < m.nstruct; ++s) {
+        const double pre = kind_pre(m.kinds[s]);
+        double* us = u.data() + (size_t)s * 3 * pad;
+        for (int64_t j = 0; j < count; ++j) {
+            double uj[3];
+            structure_coords(m, s, coords + j * d, pre, uj);
+            for (int k = 0; k < d; ++k) us[(size_t)k * pad + j] = uj[k];
+        }
+        for (int k = 0; k < d; ++k)
+            for (int64_t j = count; j < pad; ++j) us[(size_t)k * pad + j] = us[(size_t)k * pad + count - 1];
+    }
+    GSI_CUDA(cudaMalloc(&dst, u.size() * sizeof(double)));
+    GSI_CUDA(cudaMemcpyAsync(dst, u.data(), u.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
+}
+
 static void make_kernelcov(gsi_ctx* ctx, int64_t n, const double* coords, const CovModel& m, double nugget, int64_t row0,
                            int64_t mloc, gsi_op** out) {
     GSI_REQUIRE(n >= 1 && row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov: bad row block");
-    const int d = m.d;
     std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
     op->ctx = ctx;
     set_model(op.get(), m, nugget, true);
     op->m = op->n = n; op->row0 = row0; op->mloc = mloc;
-    op->n_pad = round_up(n, kRowPad);
-    // scaled SoA coordinates u[s][k][j] of every structure (one structure: u[k][j]); padding repeats the last point
-    std::vector<double> u((size_t)m.nstruct * 3 * op->n_pad, 0.0);
-    for (int s = 0; s < m.nstruct; ++s) {
-        const double pre = kind_pre(m.kinds[s]);
-        double* us = u.data() + (size_t)s * 3 * op->n_pad;
-        for (int64_t j = 0; j < n; ++j) {
-            double uj[3];
-            structure_coords(m, s, coords + j * d, pre, uj);
-            for (int k = 0; k < d; ++k) us[(size_t)k * op->n_pad + j] = uj[k];
-        }
-        for (int k = 0; k < d; ++k)
-            for (int64_t j = n; j < op->n_pad; ++j) us[(size_t)k * op->n_pad + j] = us[(size_t)k * op->n_pad + n - 1];
-    }
-    GSI_CUDA(cudaMalloc(&op->ucoords, u.size() * sizeof(double)));
-    GSI_CUDA(cudaMemcpyAsync(op->ucoords, u.data(), u.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
+    upload_coords(ctx, m, n, coords, op->ucoords, op->n_pad);
     set_partition(op.get());
     ctx_retain(ctx);
     *out = op.release();
 }
 
-static void make_kernelcov_grid(gsi_ctx* ctx, const int64_t* dims, const double* spacing, const CovModel& m, double nugget,
-                                int64_t row0, int64_t mloc, gsi_op** out) {
-    const int d = m.d;
+// a structured grid (dims / spacing of the public calls) and the size of the model's lattice table over it
+struct GridSpec {
     int64_t nd[3] = {1, 1, 1};
     double h[3] = {1, 1, 1};
-    int64_t n = 1;
+    int64_t n = 1;          // nodes
+    bool sgn = false;       // the table covers signed offsets
+    int64_t ex = 1, ey = 1, tsize = 1;
+};
+
+static GridSpec grid_spec(const int64_t* dims, const double* spacing, const CovModel& m) {
+    const int d = m.d;
+    GridSpec g;
     for (int k = 0; k < d; ++k) {
         GSI_REQUIRE(dims[k] >= 1, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad dims / length scales");
-        nd[k] = dims[k]; h[k] = spacing[k];
-        n *= dims[k];
+        g.nd[k] = dims[k]; g.h[k] = spacing[k];
+        g.n *= dims[k];
     }
-    GSI_REQUIRE(n < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: more than 2^31 points");
-    GSI_REQUIRE(row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad row block");
+    GSI_REQUIRE(g.n < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: more than 2^31 points");
     // a rotated model is not symmetric in each axis: its table covers signed offsets, folded by k(delta) = k(-delta)
     // (the last axis as |delta|, the others from -(n - 1) to n - 1).  d = 1 is symmetric whatever the rotation (+-1)
-    const bool sgn = m.any_rotated() && d >= 2;
-    const int64_t ex = sgn ? 2 * nd[0] - 1 : nd[0];
-    const int64_t ey = sgn && d == 3 ? 2 * nd[1] - 1 : nd[1];
-    const int64_t tsize = ex * ey * nd[2];
-    GSI_REQUIRE(tsize < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: lattice table of 2^31 entries or more");
+    g.sgn = m.any_rotated() && d >= 2;
+    g.ex = g.sgn ? 2 * g.nd[0] - 1 : g.nd[0];
+    g.ey = g.sgn && d == 3 ? 2 * g.nd[1] - 1 : g.nd[1];
+    g.tsize = g.ex * g.ey * g.nd[2];
+    return g;
+}
+
+static void check_table_size(const GridSpec& g) {
+    GSI_REQUIRE(g.tsize < ((int64_t)1 << 31), GSI_ERR_UNSUPPORTED, "kernelcov_grid: lattice table of 2^31 entries or more");
+}
+
+// the grid parameters of the operator and its lattice table: the model value of every lattice offset (libm, same
+// formula as the dense definition)
+static void upload_table(gsi_ctx* ctx, gsi_op* op, const CovModel& m, const GridSpec& g) {
+    op->grid_nx = (int)g.nd[0]; op->grid_ny = (int)g.nd[1]; op->grid_nz = (int)g.nd[2];
+    op->table_signed = g.sgn;
+    const int64_t ox = g.sgn ? g.nd[0] - 1 : 0, oy = g.sgn && m.d == 3 ? g.nd[1] - 1 : 0;
+    std::vector<double> tab((size_t)g.tsize);
+    for (int64_t iz = 0; iz < g.nd[2]; ++iz)
+        for (int64_t iy = 0; iy < g.ey; ++iy)
+            for (int64_t ix = 0; ix < g.ex; ++ix) {
+                const double x[3] = {(double)(ix - ox) * g.h[0], (double)(iy - oy) * g.h[1], (double)iz * g.h[2]};
+                tab[(size_t)(ix + g.ex * (iy + g.ey * iz))] = model_host(m, x);
+            }
+    GSI_CUDA(cudaMalloc(&op->table, tab.size() * sizeof(double)));
+    GSI_CUDA(cudaMemcpyAsync(op->table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
+}
+
+// lattice indices [3][pad] (SoA, pad = round_up(count, kRowPad)) of `count` grid nodes, node j at the linear index
+// idx[j] (idx == NULL: j), dims[0] fastest; the padding repeats the last node
+static void upload_lattice(gsi_ctx* ctx, const GridSpec& g, int64_t count, const int64_t* idx, int*& dst, int64_t& pad) {
+    pad = round_up(count, kRowPad);
+    if (count == 0) return;
+    std::vector<int> lat((size_t)3 * pad, 0);
+    for (int64_t j = 0; j < pad; ++j) {
+        const int64_t jc = j < count ? j : count - 1;
+        const int64_t jj = idx ? idx[jc] : jc;
+        lat[(size_t)0 * pad + j] = (int)(jj % g.nd[0]);
+        lat[(size_t)1 * pad + j] = (int)((jj / g.nd[0]) % g.nd[1]);
+        lat[(size_t)2 * pad + j] = (int)(jj / (g.nd[0] * g.nd[1]));
+    }
+    GSI_CUDA(cudaMalloc(&dst, lat.size() * sizeof(int)));
+    GSI_CUDA(cudaMemcpyAsync(dst, lat.data(), lat.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
+}
+
+static void make_kernelcov_grid(gsi_ctx* ctx, const int64_t* dims, const double* spacing, const CovModel& m, double nugget,
+                                int64_t row0, int64_t mloc, gsi_op** out) {
+    const GridSpec g = grid_spec(dims, spacing, m);
+    const int64_t n = g.n;
+    GSI_REQUIRE(row0 >= 0 && mloc >= 0 && row0 + mloc <= n, GSI_ERR_INVALID_ARGUMENT, "kernelcov_grid: bad row block");
+    check_table_size(g);
     std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
     op->ctx = ctx;
     set_model(op.get(), m, nugget, false);
     op->m = op->n = n; op->row0 = row0; op->mloc = mloc;
-    op->n_pad = round_up(n, kRowPad);
-    op->grid_nx = (int)nd[0]; op->grid_ny = (int)nd[1]; op->grid_nz = (int)nd[2];
-    op->table_signed = sgn;
-    // kernel value of every lattice offset (libm, same formula as the dense definition)
-    const int64_t ox = sgn ? nd[0] - 1 : 0, oy = sgn && d == 3 ? nd[1] - 1 : 0;
-    std::vector<double> tab((size_t)tsize);
-    for (int64_t iz = 0; iz < nd[2]; ++iz)
-        for (int64_t iy = 0; iy < ey; ++iy)
-            for (int64_t ix = 0; ix < ex; ++ix) {
-                const double x[3] = {(double)(ix - ox) * h[0], (double)(iy - oy) * h[1], (double)iz * h[2]};
-                tab[(size_t)(ix + ex * (iy + ey * iz))] = model_host(m, x);
-            }
-    // lattice indices of every point (SoA, padding repeats the last point)
-    std::vector<int> lat((size_t)3 * op->n_pad, 0);
-    for (int64_t j = 0; j < op->n_pad; ++j) {
-        const int64_t jj = j < n ? j : n - 1;
-        lat[(size_t)0 * op->n_pad + j] = (int)(jj % nd[0]);
-        lat[(size_t)1 * op->n_pad + j] = (int)((jj / nd[0]) % nd[1]);
-        lat[(size_t)2 * op->n_pad + j] = (int)(jj / (nd[0] * nd[1]));
+    upload_table(ctx, op.get(), m, g);
+    upload_lattice(ctx, g, n, nullptr, op->lattice, op->n_pad);
+    set_partition(op.get());
+    ctx_retain(ctx);
+    *out = op.release();
+}
+
+// Cross-covariance C(T, S): m targets (this rank: [row0, row0 + mloc), compacted), n sources, no nugget
+static void check_cross_rows(int64_t m, int64_t n, int64_t row0, int64_t mloc) {
+    GSI_REQUIRE(m >= 1 && n >= 1, GSI_ERR_INVALID_ARGUMENT, "kernelcov_cross: m and n must be at least 1");
+    GSI_REQUIRE(row0 >= 0 && mloc >= 0 && row0 + mloc <= m, GSI_ERR_INVALID_ARGUMENT, "kernelcov_cross: bad row block");
+}
+
+static void make_kernelcross(gsi_ctx* ctx, int64_t m, const double* targets, int64_t n, const double* sources,
+                             const CovModel& model, int64_t row0, int64_t mloc, gsi_op** out) {
+    check_cross_rows(m, n, row0, mloc);
+    std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
+    op->ctx = ctx;
+    set_model(op.get(), model, 0.0, true);
+    op->type = OP_KERNELCROSS;
+    op->m = m; op->n = n; op->row0 = row0; op->mloc = mloc;
+    upload_coords(ctx, model, n, sources, op->ucoords, op->n_pad);
+    upload_coords(ctx, model, mloc, targets + row0 * model.d, op->ucoords_t, op->nt_pad);
+    set_partition(op.get());
+    ctx_retain(ctx);
+    *out = op.release();
+}
+
+static void make_kernelcross_grid(gsi_ctx* ctx, const int64_t* dims, const double* spacing, int64_t m,
+                                  const int64_t* target_idx, int64_t n, const int64_t* source_idx,
+                                  const CovModel& model, int64_t row0, int64_t mloc, gsi_op** out) {
+    const GridSpec g = grid_spec(dims, spacing, model);
+    check_cross_rows(m, n, row0, mloc);
+    GSI_REQUIRE(target_idx || m == g.n, GSI_ERR_INVALID_ARGUMENT,
+                "kernelcov_cross_grid: without target indices m must be the number of grid nodes");
+    GSI_REQUIRE(source_idx || n == g.n, GSI_ERR_INVALID_ARGUMENT,
+                "kernelcov_cross_grid: without source indices n must be the number of grid nodes");
+    for (int64_t i = 0; target_idx && i < m; ++i)
+        GSI_REQUIRE(target_idx[i] >= 0 && target_idx[i] < g.n, GSI_ERR_INVALID_ARGUMENT,
+                    "kernelcov_cross_grid: target index outside the grid");
+    for (int64_t j = 0; source_idx && j < n; ++j)
+        GSI_REQUIRE(source_idx[j] >= 0 && source_idx[j] < g.n, GSI_ERR_INVALID_ARGUMENT,
+                    "kernelcov_cross_grid: source index outside the grid");
+    check_table_size(g);
+    std::unique_ptr<gsi_op, OpAbort> op(new gsi_op());
+    op->ctx = ctx;
+    set_model(op.get(), model, 0.0, false);
+    op->type = OP_KERNELCROSS;
+    op->m = m; op->n = n; op->row0 = row0; op->mloc = mloc;
+    upload_table(ctx, op.get(), model, g);
+    upload_lattice(ctx, g, n, source_idx, op->lattice, op->n_pad);
+    if (target_idx) {
+        upload_lattice(ctx, g, mloc, target_idx + row0, op->lattice_t, op->nt_pad);
+    } else {
+        std::vector<int64_t> rows((size_t)mloc);
+        for (int64_t i = 0; i < mloc; ++i) rows[(size_t)i] = row0 + i;
+        upload_lattice(ctx, g, mloc, rows.data(), op->lattice_t, op->nt_pad);
     }
-    GSI_CUDA(cudaMalloc(&op->table, tab.size() * sizeof(double)));
-    GSI_CUDA(cudaMalloc(&op->lattice, lat.size() * sizeof(int)));
-    GSI_CUDA(cudaMemcpyAsync(op->table, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    GSI_CUDA(cudaMemcpyAsync(op->lattice, lat.data(), lat.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-    GSI_CUDA(cudaStreamSynchronize(ctx->stream));
     set_partition(op.get());
     ctx_retain(ctx);
     *out = op.release();
@@ -773,6 +868,33 @@ GSI_API int32_t gsi_op_kernelcov_model_grid(gsi_ctx* ctx, int32_t d, const int64
     });
 }
 
+GSI_API int32_t gsi_op_kernelcov_cross(gsi_ctx* ctx, int32_t d, int64_t m, const double* targets, int64_t n,
+                                       const double* sources, int32_t nstruct, const int32_t* kinds, const double* sills,
+                                       const double* ranges, const double* rotations, const double* betas, int64_t row0,
+                                       int64_t mloc, gsi_op** out) {
+    return guarded([&] {
+        use(ctx);
+        GSI_REQUIRE(targets && sources && kinds && sills && ranges && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov_cross: d must be 1, 2 or 3");
+        const CovModel model = model_from_args(d, nstruct, kinds, sills, ranges, rotations, betas);
+        make_kernelcross(ctx, m, targets, n, sources, model, row0, mloc, out);
+    });
+}
+
+GSI_API int32_t gsi_op_kernelcov_cross_grid(gsi_ctx* ctx, int32_t d, const int64_t* dims, const double* spacing,
+                                            int64_t m, const int64_t* target_idx, int64_t n, const int64_t* source_idx,
+                                            int32_t nstruct, const int32_t* kinds, const double* sills,
+                                            const double* ranges, const double* rotations, const double* betas,
+                                            int64_t row0, int64_t mloc, gsi_op** out) {
+    return guarded([&] {
+        use(ctx);
+        GSI_REQUIRE(dims && spacing && kinds && sills && ranges && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        GSI_REQUIRE(d >= 1 && d <= 3, GSI_ERR_UNSUPPORTED, "kernelcov_cross_grid: d must be 1, 2 or 3");
+        const CovModel model = model_from_args(d, nstruct, kinds, sills, ranges, rotations, betas);
+        make_kernelcross_grid(ctx, dims, spacing, m, target_idx, n, source_idx, model, row0, mloc, out);
+    });
+}
+
 GSI_API int32_t gsi_op_free(gsi_op* op) {
     if (!op) return GSI_OK;
     return guarded([&] {
@@ -780,6 +902,8 @@ GSI_API int32_t gsi_op_free(gsi_op* op) {
         if (op->ucoords) cudaFree(op->ucoords);
         if (op->table) cudaFree(op->table);
         if (op->lattice) cudaFree(op->lattice);
+        if (op->ucoords_t) cudaFree(op->ucoords_t);
+        if (op->lattice_t) cudaFree(op->lattice_t);
         if (op->tmpT) BufDeleter()(op->tmpT);
         gsi_ctx* octx = op->ctx;
         delete op;
@@ -799,8 +923,7 @@ GSI_API int32_t gsi_op_apply(gsi_op* op, int32_t trans, const gsi_buf* X, gsi_bu
     return guarded([&] {
         GSI_REQUIRE(op && X && Y, GSI_ERR_INVALID_ARGUMENT, "null argument");
         use(op->ctx);
-        const bool sym = op->type != OP_DENSE;
-        op_apply(op, sym ? 0 : trans, X, Y);
+        op_apply(op, op_symmetric(op) ? 0 : trans, X, Y);
         GSI_CUDA(cudaStreamSynchronize(op->ctx->stream));
     });
 }

@@ -133,7 +133,7 @@ constexpr int KC_KIND_MODEL = 13;         // nested model: sum of structures, ea
 constexpr int KC_KIND_TABLE_SIGNED = 14;  // structured grid, table over signed lattice offsets (rotated anisotropy)
 constexpr int KC_KIND_TABLE = 15;         // structured grid, table over |lattice offsets|
 
-enum OpType { OP_DENSE = 0, OP_LOWRANKCOV = 1, OP_KERNELCOV = 2 };
+enum OpType { OP_DENSE = 0, OP_LOWRANKCOV = 1, OP_KERNELCOV = 2, OP_KERNELCROSS = 3 };
 
 struct gsi_op {
     gsi_ctx* ctx = nullptr;
@@ -157,6 +157,11 @@ struct gsi_op {
     int32_t nstruct = 1;
     int32_t mkinds[GSI_MODEL_MAX_STRUCTURES] = {0, 0, 0, 0};
     double msills[GSI_MODEL_MAX_STRUCTURES] = {0, 0, 0, 0}, mbetas[GSI_MODEL_MAX_STRUCTURES] = {1, 1, 1, 1};
+    // cross-covariance C(T, S) (OP_KERNELCROSS): ucoords / lattice hold the n source points, these this rank's mloc
+    // target points (compacted, so that bulk copies of them stay 16-byte aligned), same layouts with pitch nt_pad
+    double* ucoords_t = nullptr;
+    int* lattice_t = nullptr;
+    int64_t nt_pad = 0;
     std::vector<int64_t> part;           // row partition over ranks: part[r] .. part[r+1]
 };
 
@@ -176,8 +181,8 @@ void small_cm_to_tall(gsi_ctx*, const double* M, int64_t ldm, int64_t rows, int6
 void colmajor_upload(gsi_buf* b, const double* host, int64_t ldh);
 void colmajor_download(const gsi_buf* b, double* host, int64_t ldh);
 
-// ---- kcov_gemm.cu :  W[local rows] = C[rows, :] * X
-void kcov_apply(gsi_op* op, const gsi_buf* X, gsi_buf* W);
+// ---- kcov_gemm.cu :  W[local rows] = C[rows, :] * X  (cross-covariance: trans = 1 gives W = C' X, all n rows)
+void kcov_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* W);
 // ---- dense_gemm.cu : W = A X (trans=0) or A' X (trans=1); alpha scaling
 void dense_apply(gsi_ctx*, const gsi_buf* A, int trans, const gsi_buf* X, gsi_buf* W, double alpha);
 void tall_window_update(gsi_ctx*, const double* Pd, int64_t ldp, int64_t rows, int64_t kdim, const gsi_buf* X,

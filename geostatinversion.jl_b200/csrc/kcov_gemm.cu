@@ -64,6 +64,12 @@ struct KcovParams : KcovBase {
     int nstruct;
     int mkinds[GSI_MODEL_MAX_STRUCTURES];
     double msills[GSI_MODEL_MAX_STRUCTURES], mbetas[GSI_MODEL_MAX_STRUCTURES];
+    // row side: the points of the output rows, the same layouts as u / lat with their own stride.  A square operator
+    // passes u / lat themselves; a cross-covariance operator C(T, S) passes the other point set (row0 = 0 then)
+    const double* ur;      // scaled coordinates of the row points [nstruct][3][nr_pad]
+    const int* latr;       // lattice indices of the row points [3][nr_pad]
+    int64_t nr_pad;
+    int64_t nr;            // row points: a generated row beyond the last one is clamped to it (never stored)
 };
 
 template <int KIND>
@@ -479,8 +485,8 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
     auto gcol = [&](int e) -> int { return gj0 + (e & 1) + ((e >> 1) << 4); };
     int li[DIM];
     auto row_coords = [&](int64_t base_rg, double (&ui)[DIM]) {
-        int64_t gpt = p.row0 + base_rg * 16 + grow_in_tile;           // global point of my generated row
-        if (gpt > p.n - 1) gpt = p.n - 1;                             // tail rows: clamp (never stored)
+        int64_t gpt = p.row0 + base_rg * 16 + grow_in_tile;           // row point of my generated row
+        if (gpt > p.nr - 1) gpt = p.nr - 1;                           // tail rows: clamp (never stored)
         if constexpr (KIND == KC_KIND_MODEL) {
             // the row's nstruct * DIM coordinates go to shared memory, [KC_BM][GSI_MODEL_MAX_STRUCTURES * DIM] after
             // etab (they do not fit the register budget): the 8 threads of a row, all in this warp, load them
@@ -488,14 +494,14 @@ __global__ void __launch_bounds__(KC_THREADS, 1) kcov_gemm_kernel(const __grid_c
             __syncwarp();
             for (int q = gtid & 7; q < p.nstruct * DIM; q += 8) {
                 const int s = q / DIM, k = q - s * DIM;
-                etab[64 + grow_in_tile * (GSI_MODEL_MAX_STRUCTURES * DIM) + q] = p.u[(s * 3 + k) * p.n_pad + gpt];
+                etab[64 + grow_in_tile * (GSI_MODEL_MAX_STRUCTURES * DIM) + q] = p.ur[(s * 3 + k) * p.nr_pad + gpt];
             }
             __syncwarp();
         } else {
 #pragma unroll
             for (int k = 0; k < DIM; ++k) {
-                if (kind_is_table<KIND>()) li[k] = p.lat[k * p.n_pad + gpt];
-                else ui[k] = p.u[k * p.n_pad + gpt];
+                if (kind_is_table<KIND>()) li[k] = p.latr[k * p.nr_pad + gpt];
+                else ui[k] = p.ur[k * p.nr_pad + gpt];
             }
         }
     };
@@ -747,8 +753,14 @@ __global__ void kcov_tail_fixup_kernel(KcovBase p, int64_t nkt, int64_t tail_rg0
     }
 }
 
+// all_sms: the cross-covariance operator launches the full persistent grid even when the output has fewer than
+// 4 x grid row groups.  C(obs, grid) X has few rows and a long k range (200 x 200 704); a grid capped at its 13 row
+// groups would leave 135 of 148 SMs idle, while the stream-K tail spreads the k range over every CTA (CTAs past the
+// last unit own no work).  The tail invariants hold for any grid: tail tiles <= grid, so a share of
+// ceil(tiles * nkt / grid) <= nkt units spans at most two segments, and a tile's pieces <= grid <= KF_MAX_PIECES.
+// The square operators keep the capped grid (a different grid reorders their sums).
 template <int NB, int KIND, int DIM>
-static void launch_kcov(gsi_ctx* ctx, const KcovParams& p0) {
+static void launch_kcov(gsi_ctx* ctx, const KcovParams& p0, bool all_sms) {
     KcovParams p = p0;
     const int ld = NB * 8 + 4;
     const size_t stage_bytes = (size_t)(KC_BK * ld + kc_coord_doubles<KIND>()) * sizeof(double);
@@ -766,7 +778,7 @@ static void launch_kcov(gsi_ctx* ctx, const KcovParams& p0) {
     if (occ < 1) occ = 1;
     const int64_t total_rg = (p.mloc + 15) / 16;                 // 16-row groups; a CTA runs up to 4 at a time
     int64_t grid = (int64_t)ctx->num_sms * occ;
-    if (grid > total_rg) grid = total_rg;
+    if (!all_sms && grid > total_rg) grid = total_rg;
     if (grid < 1) grid = 1;
     p.pad0 = 0;
     p.win_epochs = ctx->kcov_window > 0 ? ctx->kcov_window : 0;
@@ -812,34 +824,47 @@ static void launch_kcov(gsi_ctx* ctx, const KcovParams& p0) {
 }
 
 template <int NB, int KIND>
-static void dispatch_dim(gsi_ctx* ctx, const KcovParams& p, int dim) {
-    if (dim <= 2) launch_kcov<NB, KIND, 2>(ctx, p);
-    else launch_kcov<NB, KIND, 3>(ctx, p);
+static void dispatch_dim(gsi_ctx* ctx, const KcovParams& p, int dim, bool all_sms) {
+    if (dim <= 2) launch_kcov<NB, KIND, 2>(ctx, p, all_sms);
+    else launch_kcov<NB, KIND, 3>(ctx, p, all_sms);
 }
 
 template <int NB>
-static void dispatch_kind(gsi_ctx* ctx, const KcovParams& p, int kind, int dim) {
+static void dispatch_kind(gsi_ctx* ctx, const KcovParams& p, int kind, int dim, bool all_sms) {
     switch (kind) {
-        case GSI_KERNEL_EXPONENTIAL: dispatch_dim<NB, GSI_KERNEL_EXPONENTIAL>(ctx, p, dim); break;
-        case GSI_KERNEL_GAUSSIAN: dispatch_dim<NB, GSI_KERNEL_GAUSSIAN>(ctx, p, dim); break;
-        case GSI_KERNEL_POWERLAW: dispatch_dim<NB, GSI_KERNEL_POWERLAW>(ctx, p, dim); break;
-        case GSI_KERNEL_MATERN32: dispatch_dim<NB, GSI_KERNEL_MATERN32>(ctx, p, dim); break;
-        case GSI_KERNEL_MATERN52: dispatch_dim<NB, GSI_KERNEL_MATERN52>(ctx, p, dim); break;
-        case GSI_KERNEL_SPHERICAL: dispatch_dim<NB, GSI_KERNEL_SPHERICAL>(ctx, p, dim); break;
-        case KC_KIND_TABLE: dispatch_dim<NB, KC_KIND_TABLE>(ctx, p, dim); break;
-        case KC_KIND_TABLE_SIGNED: dispatch_dim<NB, KC_KIND_TABLE_SIGNED>(ctx, p, dim); break;
-        case KC_KIND_MODEL: dispatch_dim<NB, KC_KIND_MODEL>(ctx, p, dim); break;
+        case GSI_KERNEL_EXPONENTIAL: dispatch_dim<NB, GSI_KERNEL_EXPONENTIAL>(ctx, p, dim, all_sms); break;
+        case GSI_KERNEL_GAUSSIAN: dispatch_dim<NB, GSI_KERNEL_GAUSSIAN>(ctx, p, dim, all_sms); break;
+        case GSI_KERNEL_POWERLAW: dispatch_dim<NB, GSI_KERNEL_POWERLAW>(ctx, p, dim, all_sms); break;
+        case GSI_KERNEL_MATERN32: dispatch_dim<NB, GSI_KERNEL_MATERN32>(ctx, p, dim, all_sms); break;
+        case GSI_KERNEL_MATERN52: dispatch_dim<NB, GSI_KERNEL_MATERN52>(ctx, p, dim, all_sms); break;
+        case GSI_KERNEL_SPHERICAL: dispatch_dim<NB, GSI_KERNEL_SPHERICAL>(ctx, p, dim, all_sms); break;
+        case KC_KIND_TABLE: dispatch_dim<NB, KC_KIND_TABLE>(ctx, p, dim, all_sms); break;
+        case KC_KIND_TABLE_SIGNED: dispatch_dim<NB, KC_KIND_TABLE_SIGNED>(ctx, p, dim, all_sms); break;
+        case KC_KIND_MODEL: dispatch_dim<NB, KC_KIND_MODEL>(ctx, p, dim, all_sms); break;
         default: throw Error(GSI_ERR_INVALID_ARGUMENT, "unknown covariance kernel kind");
     }
 }
 
-void kcov_apply(gsi_op* op, const gsi_buf* X, gsi_buf* W) {
+// Square operator (OP_KERNELCOV): W = C[row0 .. row0 + mloc, :] X, trans ignored (C is symmetric).
+// Cross-covariance operator (OP_KERNELCROSS, C = C(T, S), targets compacted to this rank's mloc points):
+//   trans = 0: W (mloc rows) = C X,  X: all n source rows   -- target rows x source columns
+//   trans = 1: W (n rows) = C' X,    X: this rank's mloc target rows (zero padded beyond them: the last k-tile's
+//              padded columns multiply them)                -- source rows x target columns
+void kcov_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* W) {
     gsi_ctx* ctx = op->ctx;
+    const bool cross = op->type == OP_KERNELCROSS;
+    const bool tr = cross && trans;
+    const int64_t krows = tr ? op->mloc : op->n;               // rows of X (the product's k range)
+    const int64_t orows = tr ? op->n : op->mloc;               // rows of W
     GSI_REQUIRE(X->layout == GSI_LAYOUT_TALL && W->layout == GSI_LAYOUT_TALL, GSI_ERR_INVALID_ARGUMENT,
                 "kernelcov apply needs TALL buffers");
-    GSI_REQUIRE(X->rows == op->n, GSI_ERR_DIMENSION_MISMATCH, "kernelcov apply: X must have n rows");
-    GSI_REQUIRE(W->rows == op->mloc, GSI_ERR_DIMENSION_MISMATCH, "kernelcov apply: W must have mloc rows");
+    GSI_REQUIRE(X->rows == krows, GSI_ERR_DIMENSION_MISMATCH, "kernelcov apply: X must have n rows");
+    GSI_REQUIRE(W->rows == orows, GSI_ERR_DIMENSION_MISMATCH, "kernelcov apply: W must have mloc rows");
     GSI_REQUIRE(X->cols == W->cols, GSI_ERR_DIMENSION_MISMATCH, "kernelcov apply: X/W column mismatch");
+    if (cross && (orows == 0 || krows == 0)) {                 // a rank without target rows: no rows, or C' X = 0
+        if (orows > 0) tall_zero(ctx, W);
+        return;
+    }
     if (X->cols > kMaxCols) {
         // wide iterate (K + p > 256): the product runs on 256-column chunks packed into compact buffers
         for (int64_t c0 = 0; c0 < X->cols; c0 += kMaxCols) {
@@ -847,7 +872,7 @@ void kcov_apply(gsi_op* op, const gsi_buf* X, gsi_buf* W) {
             BufPtr xc = make_buf(ctx, GSI_LAYOUT_TALL, X->rows, w);
             BufPtr wc = make_buf(ctx, GSI_LAYOUT_TALL, W->rows, w);
             tall_cols_copy(ctx, X->d + c0, X->ld, xc->d, xc->ld, X->rows, w);
-            kcov_apply(op, xc.get(), wc.get());
+            kcov_apply(op, trans, xc.get(), wc.get());
             tall_cols_copy(ctx, wc->d, wc->ld, W->d + c0, W->ld, W->rows, w);
         }
         return;
@@ -866,9 +891,20 @@ void kcov_apply(gsi_op* op, const gsi_buf* X, gsi_buf* W) {
     for (int s = 0; s < GSI_MODEL_MAX_STRUCTURES; ++s) {
         p.mkinds[s] = op->mkinds[s]; p.msills[s] = op->msills[s]; p.mbetas[s] = op->mbetas[s];
     }
+    p.ur = op->ucoords; p.latr = op->lattice; p.nr_pad = op->n_pad; p.nr = op->n;
+    if (cross) {
+        // sources: ucoords / lattice (n points); targets: ucoords_t / lattice_t (this rank's mloc points)
+        p.row0 = 0;
+        if (!tr) {
+            p.ur = op->ucoords_t; p.latr = op->lattice_t; p.nr_pad = op->nt_pad; p.nr = op->mloc;
+        } else {
+            p.u = op->ucoords_t; p.lat = op->lattice_t; p.n = op->mloc; p.n_pad = op->nt_pad;
+            p.mloc = op->n;
+        }
+    }
     const int kind = op->table ? (op->table_signed ? KC_KIND_TABLE_SIGNED : KC_KIND_TABLE) : op->kind;
     switch (nb) {
-#define GSI_CASE(N) case N: dispatch_kind<N>(ctx, p, kind, op->dim); break;
+#define GSI_CASE(N) case N: dispatch_kind<N>(ctx, p, kind, op->dim, cross); break;
         GSI_NB_LIST(GSI_CASE)
 #undef GSI_CASE
         default: throw Error(GSI_ERR_UNSUPPORTED, "kernelcov apply: unsupported column-block count");

@@ -206,13 +206,34 @@ int32_t gsi_op_kernelcov_model_grid(gsi_ctx* ctx, int32_t d, const int64_t* dims
                                     int32_t nstruct, const int32_t* kinds, const double* sills,
                                     const double* ranges, const double* rotations, const double* betas,
                                     double nugget, int64_t row0, int64_t mloc, gsi_op** out);
+/* Cross-covariance between two point sets (kriging C(T, S) w, Q H' = C(grid, obs) of point observations):
+ * m x n matrix C[i,j] = sum_s sills[s] k_kinds[s](r2_s(t_i, s_j)), t_i = targets[:, i], s_j = sources[:, j] (host,
+ * d x m and d x n column-major; model arguments and coordinate scaling exactly as gsi_op_kernelcov_model).  No nugget
+ * term: T and S are different sets.  This rank owns target rows [row0, row0 + mloc).  Not symmetric: gsi_op_apply
+ * trans = 0 gives this rank's rows of C X (X: all n rows), trans = 1 gives all n rows of C' X summed over ranks (X: all
+ * m rows), as for gsi_op_dense; gsi_op_size reports (m, n).  m < 1, n < 1, a bad row block or a missing pointer:
+ * GSI_ERR_INVALID_ARGUMENT; d outside 1..3: GSI_ERR_UNSUPPORTED.                                     */
+int32_t gsi_op_kernelcov_cross(gsi_ctx* ctx, int32_t d, int64_t m, const double* targets, int64_t n,
+                               const double* sources, int32_t nstruct, const int32_t* kinds, const double* sills,
+                               const double* ranges, const double* rotations, const double* betas,
+                               int64_t row0, int64_t mloc, gsi_op** out);
+/* The same for points that are nodes of one structured grid (dims / spacing as gsi_op_kernelcov_grid), given by
+ * 0-based linear indices (dims[0] fastest); target_idx == NULL: all prod(dims) nodes in order (m must equal it),
+ * likewise source_idx.  Same table as gsi_op_kernelcov_model_grid (signed offsets when a structure is rotated).
+ * An index outside 0 .. prod(dims) - 1, or a NULL index list with m (n) != prod(dims): GSI_ERR_INVALID_ARGUMENT;
+ * a table of 2^31 entries or more: GSI_ERR_UNSUPPORTED.                                             */
+int32_t gsi_op_kernelcov_cross_grid(gsi_ctx* ctx, int32_t d, const int64_t* dims, const double* spacing,
+                                    int64_t m, const int64_t* target_idx, int64_t n, const int64_t* source_idx,
+                                    int32_t nstruct, const int32_t* kinds, const double* sills, const double* ranges,
+                                    const double* rotations, const double* betas, int64_t row0, int64_t mloc,
+                                    gsi_op** out);
 int32_t gsi_op_free(gsi_op* op);
 /* size(A) (src/RandMatFact.jl:52-53, src/lowrank.jl:50-60)                           */
 int32_t gsi_op_size(const gsi_op* op, int64_t* m, int64_t* n);
 /* `A * X` (trans=0, src/RandMatFact.jl:55,70) or `A' * X` (trans=1, :67; and
  * `(Q' * A)' = A' * Q`, :85).  X: TALL, all n (resp. m) rows.  Y: TALL, this rank's
- * rows of the result (for trans=1 on a row-sharded dense A the partial products are
- * summed over ranks and every rank receives all n rows).                             */
+ * rows of the result (for trans=1 on a row-sharded dense A or cross-covariance the partial
+ * products are summed over ranks and every rank receives all n rows).                */
 int32_t gsi_op_apply(gsi_op* op, int32_t trans, const gsi_buf* X, gsi_buf* Y);
 
 /* ---- factorisation building blocks (exposed for tests and for the shim) ----------- */

@@ -9,7 +9,8 @@
 #   eig_nystrom(A, Q), getxis(Q, numxis, p, q, seed), getxis(samplefield, numfields, numxis, p, q, seed),
 #   getxis(Val{:iwantfields}, ...), pcgalsqr / pcgadirect / pcga / rga with the reference's
 #   positional and keyword arguments,
-# for A::Matrix{Float64}, A::KernelCovMatrix (new) and A::LowRankCovMatrix, whose method set is
+# for A::Matrix{Float64}, A::KernelCovMatrix (new), A::KernelCrossCovMatrix (new, not symmetric) and
+# A::LowRankCovMatrix, whose method set is
 # the one the reference's LowRankCovMatrix provides (src/lowrank.jl:38-60,115-139):
 #   size(A), size(A, i), A', A * Matrix, A * Vector, Adjoint{Matrix} * A.
 module GeostatInversionB200
@@ -139,7 +140,10 @@ abstract type Operator end
 mutable struct DenseOperator <: Operator; h::Ptr{Cvoid}; buf::DeviceMatrix; ctx::Context; rows::UnitRange{Int}; end
 mutable struct KernelCovMatrix <: Operator; h::Ptr{Cvoid}; n::Int; ctx::Context; rows::UnitRange{Int}; end
 mutable struct LowRankCovMatrix <: Operator; h::Ptr{Cvoid}; buf::DeviceMatrix; ctx::Context; rows::UnitRange{Int}; end
+# cross-covariance C(T, S): `rows` = this worker's block of target rows
+mutable struct KernelCrossCovMatrix <: Operator; h::Ptr{Cvoid}; n::Int; ctx::Context; rows::UnitRange{Int}; end
 issym(::DenseOperator) = false
+issym(::KernelCrossCovMatrix) = false
 issym(::Operator) = true
 
 freeop(o) = ccall((:gsi_op_free, LIB), Int32, (Ptr{Cvoid},), o.h)
@@ -228,6 +232,56 @@ function KernelCovModelGrid(kinds::Vector{<:Integer}, sills::Vector{Float64}, ra
 	return op
 end
 
+"""Cross-covariance C(T, S) of a nested model (gsi_op_kernelcov_cross) between targets d x m and sources d x n, no
+nugget: kriging `C(T, S) * w`, `Q H' = C(grid, obs)`.  Model arguments as KernelCovModel.  Not symmetric: `A' * X` is
+C(S, T) X (all n rows, summed over workers).  Multi-GPU: `rows` = this worker's target rows."""
+function KernelCrossCov(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, targets::Matrix{Float64},
+		sources::Matrix{Float64}; rotations::Union{Nothing, Array{Float64, 3}}=nothing,
+		betas::Union{Nothing, Vector{Float64}}=nothing,
+		ctx::Context=context(), rows::UnitRange{Int}=partitionrows(size(targets, 2), ctx.world, ctx.rank))
+	d, m = size(targets)
+	size(sources, 1) == d || throw(DimensionMismatch("KernelCrossCov: targets are $d-D, sources $(size(sources, 1))-D"))
+	n = size(sources, 2)
+	kinds32 = Int32.(kinds)
+	rot = rotations === nothing ? Ptr{Float64}(C_NULL) : pointer(rotations)
+	bet = betas === nothing ? Ptr{Float64}(C_NULL) : pointer(betas)
+	out = Ref{Ptr{Cvoid}}(C_NULL)
+	GC.@preserve targets sources kinds32 sills ranges rotations betas check(ccall((:gsi_op_kernelcov_cross, LIB), Int32,
+		(Ptr{Cvoid}, Int32, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+		 Ptr{Float64}, Int64, Int64, Ref{Ptr{Cvoid}}),
+		ctx.h, d, m, targets, n, sources, length(kinds32), kinds32, sills, ranges, rot, bet, first(rows) - 1, length(rows), out))
+	op = KernelCrossCovMatrix(out[], n, ctx, rows)
+	finalizer(freeop, op)
+	return op
+end
+
+"""structured grid variant of KernelCrossCov: targets / sources are 1-based linear indices of grid nodes (dims[1]
+fastest), `nothing` for every node in order"""
+function KernelCrossCovGrid(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, dims::Vector{Int},
+		spacing::Vector{Float64}, targets::Union{Nothing, AbstractVector{<:Integer}}, sources::Union{Nothing, AbstractVector{<:Integer}};
+		rotations::Union{Nothing, Array{Float64, 3}}=nothing, betas::Union{Nothing, Vector{Float64}}=nothing,
+		ctx::Context=context(), rows::UnitRange{Int}=partitionrows(targets === nothing ? prod(dims) : length(targets), ctx.world, ctx.rank))
+	d = length(dims)
+	dims64 = Int64.(dims)
+	tidx = targets === nothing ? nothing : Int64.(targets) .- 1                # 0-based for the library
+	sidx = sources === nothing ? nothing : Int64.(sources) .- 1
+	m = tidx === nothing ? prod(dims) : length(tidx)
+	n = sidx === nothing ? prod(dims) : length(sidx)
+	tp = tidx === nothing ? Ptr{Int64}(C_NULL) : pointer(tidx)
+	sp = sidx === nothing ? Ptr{Int64}(C_NULL) : pointer(sidx)
+	kinds32 = Int32.(kinds)
+	rot = rotations === nothing ? Ptr{Float64}(C_NULL) : pointer(rotations)
+	bet = betas === nothing ? Ptr{Float64}(C_NULL) : pointer(betas)
+	out = Ref{Ptr{Cvoid}}(C_NULL)
+	GC.@preserve dims64 spacing tidx sidx kinds32 sills ranges rotations betas check(ccall((:gsi_op_kernelcov_cross_grid, LIB), Int32,
+		(Ptr{Cvoid}, Int32, Ptr{Int64}, Ptr{Float64}, Int64, Ptr{Int64}, Int64, Ptr{Int64}, Int32, Ptr{Int32}, Ptr{Float64},
+		 Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int64, Int64, Ref{Ptr{Cvoid}}),
+		ctx.h, d, dims64, spacing, m, tp, n, sp, length(kinds32), kinds32, sills, ranges, rot, bet, first(rows) - 1, length(rows), out))
+	op = KernelCrossCovMatrix(out[], n, ctx, rows)
+	finalizer(freeop, op)
+	return op
+end
+
 "LowRankCovMatrix(samples) -- src/lowrank.jl:14-30 (the mean is removed on the device)"
 function LowRankCovMatrix(samples::Vector{Vector{Float64}}; ctx::Context=context())
 	S = reduce(hcat, samples)
@@ -249,9 +303,9 @@ Base.eltype(::Operator) = Float64
 Base.adjoint(op::Union{KernelCovMatrix, LowRankCovMatrix}) = op      # symmetric (src/lowrank.jl:38-44)
 Base.transpose(op::Union{KernelCovMatrix, LowRankCovMatrix}) = op
 
-"lazy adjoint of a dense operator, so that `A' * X` maps onto gsi_op_apply(trans = 1)"
-struct AdjointOperator; parent::DenseOperator; end
-Base.adjoint(op::DenseOperator) = AdjointOperator(op)
+"lazy adjoint of a non-symmetric operator (dense, cross-covariance), so that `A' * X` maps onto gsi_op_apply(trans = 1)"
+struct AdjointOperator{T<:Operator}; parent::T; end
+Base.adjoint(op::Union{DenseOperator, KernelCrossCovMatrix}) = AdjointOperator(op)
 Base.adjoint(a::AdjointOperator) = a.parent
 Base.size(a::AdjointOperator) = reverse(size(a.parent))
 Base.size(a::AdjointOperator, i::Int) = size(a)[i]
@@ -281,7 +335,7 @@ Base.:*(Bt::LinearAlgebra.Adjoint{Float64, Matrix{Float64}}, op::Operator) = Mat
 
 module RandMatFact
 import ..GeostatInversionB200: LIB, check, context, Operator, DenseOperator, DeviceMatrix, upload!, download,
-	GSI_LAYOUT_TALL, GSI_NORMALISER_LU_REF
+	GSI_LAYOUT_TALL, GSI_NORMALISER_LU_REF, issym
 import LinearAlgebra
 
 asoperator(A::Operator) = A
@@ -294,7 +348,7 @@ function randsvd(A, K::Int, p::Int, q::Int; full::Bool=false)
 	n = size(op, 2)
 	Omega = randn(n, K + p)                              # same host RNG stream as the reference
 	Om = upload!(DeviceMatrix(op.ctx, GSI_LAYOUT_TALL, n, K + p), Omega)
-	zrows = (full || op isa DenseOperator) ? n : length(op.rows)
+	zrows = (full || !issym(op)) ? n : length(op.rows)
 	Z = DeviceMatrix(op.ctx, GSI_LAYOUT_TALL, zrows, K + p)
 	check(ccall((:gsi_randsvd, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Int64, Int64, Int32, Ptr{Cvoid}, Ptr{Float64}),
 		op.h, Om.h, K, p, q, GSI_NORMALISER_LU_REF, Z.h, C_NULL))

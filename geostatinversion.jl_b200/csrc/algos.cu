@@ -157,7 +157,7 @@ BufPtr X_view_for_dense(gsi_op* op, int trans, const gsi_buf* X) {
 
 // ------------------------------------------------------------------ distribution helpers
 // local block (mloc x l) -> full (m x l) on every rank
-static void gather_rows(gsi_op* op, const gsi_buf* loc, gsi_buf* full) {
+void gather_rows(gsi_op* op, const gsi_buf* loc, gsi_buf* full) {
     gsi_ctx* ctx = op->ctx;
     GSI_REQUIRE(loc->ld == full->ld, GSI_ERR_INVALID_ARGUMENT, "gather_rows: pitch mismatch");
     GSI_CUDA(cudaMemcpyAsync(full->d + op->row0 * full->ld, loc->d, (size_t)op->mloc * loc->ld * 8,
@@ -228,13 +228,6 @@ void tsqr_thinQ(gsi_op* op, gsi_buf* Y, bool sharded, double* Rdev) {
     // no host synchronisation: the temporaries go back to the stream-ordered pool of this context
 }
 
-// One product step of the iteration.  `cur` holds the current iterate in distribution
-// `cur_sharded`; returns the product in `out` and its distribution.
-struct Iterate {
-    BufPtr buf;
-    bool sharded = false;     // true: this rank holds rows [row0, row0+mloc) only
-};
-
 // Multi-GPU LU normalisation: the next product needs the whole iterate on every rank anyway, so it
 // is gathered BEFORE the LU and every rank factors all rows redundantly (deterministic kernels:
 // identical factors everywhere, identical to the single-GPU result) -- no per-column pivot
@@ -257,6 +250,8 @@ static void normalise(gsi_op* op, Iterate& it, int normaliser) {
     }
 }
 
+// One product step of the iteration.  `cur` holds the current iterate in distribution
+// `cur_sharded`; returns the product in `out` and its distribution.
 static Iterate apply_step(gsi_op* op, int trans, Iterate& cur, BufPtr& full_scratch) {
     gsi_ctx* ctx = op->ctx;
     const int64_t l = cur.buf->cols;
@@ -319,7 +314,7 @@ static Iterate rangefinder_fixed_impl(gsi_op* op, const gsi_buf* Omega, int64_t 
     return cur;
 }
 
-static void deliver(gsi_op* op, Iterate& res, gsi_buf* out) {
+void deliver(gsi_op* op, Iterate& res, gsi_buf* out) {
     gsi_ctx* ctx = op->ctx;
     GSI_REQUIRE(out->layout == GSI_LAYOUT_TALL && out->cols == res.buf->cols, GSI_ERR_DIMENSION_MISMATCH,
                 "output buffer: wrong layout or column count");

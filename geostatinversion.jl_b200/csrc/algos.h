@@ -7,14 +7,34 @@ namespace gsi {
 struct BufDeleter { void operator()(gsi_buf* b) const; };
 typedef std::unique_ptr<gsi_buf, BufDeleter> BufPtr;
 
+// an iterate of the algorithm drivers and its distribution over the ranks
+struct Iterate {
+    BufPtr buf;
+    bool sharded = false;     // true: this rank holds rows [row0, row0+mloc) only
+};
+
 BufPtr make_buf(gsi_ctx* ctx, int32_t layout, int64_t rows, int64_t cols);
 void op_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* Y);
 bool op_symmetric(const gsi_op* op);
 void resolve_gemm_timing(gsi_ctx* ctx);
 BufPtr X_view_for_dense(gsi_op* op, int trans, const gsi_buf* X);
 void tsqr_thinQ(gsi_op* op, gsi_buf* Y, bool sharded, double* Rdev);
+// local block (mloc x l) -> all m rows on every rank
+void gather_rows(gsi_op* op, const gsi_buf* loc, gsi_buf* full);
+// an iterate -> the caller's TALL buffer: this rank's mloc rows or all m rows, whichever `out` has; then the deferred
+// LU / Jacobi verdicts (synchronises)
+void deliver(gsi_op* op, Iterate& res, gsi_buf* out);
 void rangefinder_fixed(gsi_op* op, const gsi_buf* Omega, int64_t q, int normaliser, gsi_buf* Q_out);
 void randsvd(gsi_op* op, const gsi_buf* Omega, int64_t K, int64_t p, int64_t q, int normaliser, gsi_buf* Z_out,
              double* S_host);
+
+// ---- extras.cu: small dense kernels of eig_nystrom (l <= 256, column-major, ld = l)
+__global__ void chol_upper_kernel(double* __restrict__ B, int l, int* __restrict__ flag);
+__global__ void triu_inverse_kernel(const double* __restrict__ C, int l, double* __restrict__ Cinv);
+__global__ void tall_head_to_cm_kernel(const double* __restrict__ T, int64_t ld, int l, double* __restrict__ M);
+
+// ---- cov_solve.cu: A X = B on a square kernel-covariance operator, preconditioned CG (one recurrence per column)
+void kernelcov_solve(gsi_op* op, const gsi_buf* B, const gsi_buf* Omega, double rtol, int64_t maxiter, gsi_buf* X_out,
+                     int64_t* iters_out, double* relres_out, double* lambda_out);
 
 }  // namespace gsi

@@ -996,3 +996,12 @@ GSI_API int32_t gsi_randsvd(gsi_op* op, const gsi_buf* Omega, int64_t K, int64_t
         randsvd(op, Omega, K, p, q, normaliser, Z_out, S_host);
     });
 }
+
+GSI_API int32_t gsi_kernelcov_solve(gsi_op* op, const gsi_buf* B, const gsi_buf* Omega, double rtol, int64_t maxiter,
+                                    gsi_buf* X, int64_t* iters_out, double* relres_out, double* lambda_out) {
+    return guarded([&] {
+        GSI_REQUIRE(op && B && X && iters_out && relres_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(op->ctx);
+        kernelcov_solve(op, B, Omega, rtol, maxiter, X, iters_out, relres_out, lambda_out);
+    });
+}

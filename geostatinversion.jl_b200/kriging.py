@@ -1,0 +1,120 @@
+"""Kriging on the matrix-free covariance operator: the solve A X = B (gsi_kernelcov_solve, preconditioned CG on the
+device) and simple / ordinary / universal kriging in dual form on top of it.  The n x n covariance matrix is never
+formed: a solve costs one operator product of width k per iteration."""
+import ctypes as C
+import numpy as np
+
+from . import _lib
+from ._lib import check, LAYOUT_TALL
+from .core import DeviceMatrix, KernelCovModelMatrix, KernelCrossCovMatrix, _f64_colmajor, _pd, as_operator
+from .randmatfact import _rng
+
+
+def cov_solve(A, B, *, rtol=1e-10, maxiter=None, rank=0, Omega=None, rng=None, full=False):
+    """X = A^-1 B for a square kernel-covariance operator A (KernelCovMatrix, GridKernelCovMatrix, KernelCovModelMatrix
+    or GridKernelCovModelMatrix; A exactly as built, nugget included).  B: n or n x k (k <= 1024).
+
+    The k columns run independent preconditioned CG recurrences that share one operator product per iteration; column
+    j stops when ||r_j|| <= rtol ||b_j||.  rank > 0 draws an n x rank Gaussian sketch from `rng` (or pass `Omega`) for
+    the randomized Nystrom preconditioner (1 <= rank <= 256, rank < n).  maxiter=None means n.  On a multi-rank context
+    each rank gets its own row block of X unless full=True.
+
+    Returns (X, info) with info["iterations"] (per column), info["relres"] (the true ||b - A x|| / ||b|| of the returned
+    X) and info["nystrom_eigenvalues"].  A column that does not converge raises GsiError (ERR_NO_CONVERGENCE) carrying
+    the same X and info as attributes; p'Ap <= 0 or a failed preconditioner raises PosDefException."""
+    op = as_operator(A)
+    ctx = op.ctx
+    n = op.shape[1]
+    Bh = np.asarray(B, dtype=np.float64)
+    vector = Bh.ndim == 1
+    Bh = Bh.reshape(n, -1) if vector else Bh
+    if Bh.shape[0] != n:
+        raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH, f"cov_solve: B has {Bh.shape[0]} rows, A is {n} x {n}")
+    k = Bh.shape[1]
+    if Omega is None and rank > 0:
+        Omega = _rng(rng).standard_normal((n, int(rank)))
+    r = 0 if Omega is None else np.shape(Omega)[1]
+    maxiter = n if maxiter is None else int(maxiter)
+    xrows = op.mloc if (ctx.world > 1 and not full) else n
+    iters = np.zeros(k, dtype=np.int64)
+    relres = np.zeros(k, dtype=np.float64)
+    lam = np.zeros(max(r, 1), dtype=np.float64)
+    Bd = DeviceMatrix.from_host(ctx, Bh)
+    Om = None
+    Xd = None
+    try:
+        if Omega is not None:
+            Om = Omega if isinstance(Omega, DeviceMatrix) else DeviceMatrix.from_host(ctx, Omega)
+        Xd = DeviceMatrix(ctx, xrows, k, LAYOUT_TALL)
+        status = ctx._lib.gsi_kernelcov_solve(op._h, Bd._h, None if Om is None else Om._h, float(rtol), maxiter, Xd._h,
+                                              iters.ctypes.data_as(C.POINTER(C.c_int64)), _pd(relres), _pd(lam))
+        X = Xd.numpy() if status in (_lib.OK, _lib.ERR_NO_CONVERGENCE) else None
+    finally:
+        Bd.free()
+        if Om is not None and Om is not Omega:
+            Om.free()
+        if Xd is not None:
+            Xd.free()
+    info = {"iterations": iters, "relres": relres, "nystrom_eigenvalues": lam[:r]}
+    if X is not None and vector:
+        X = X[:, 0]
+    try:
+        check(status)
+    except _lib.GsiError as e:
+        e.X, e.info = X, info
+        raise
+    return X, info
+
+
+def drift_matrices(drift, n, m):
+    """(F_sources n x p, F_targets m x p) of a drift specification: None (p = 0), "constant" or a pair of arrays."""
+    if drift is None:
+        return np.zeros((n, 0)), np.zeros((m, 0))
+    if isinstance(drift, str):
+        if drift != "constant":
+            raise ValueError(f"krige: unknown drift {drift!r} (None, 'constant' or (F_sources, F_targets))")
+        return np.ones((n, 1)), np.ones((m, 1))
+    Fs, Ft = (np.asarray(f, dtype=np.float64) for f in drift)
+    Fs, Ft = Fs.reshape(n, -1), Ft.reshape(m, -1)
+    if Fs.shape[1] != Ft.shape[1]:
+        raise ValueError(f"krige: drift has {Fs.shape[1]} columns at the sources and {Ft.shape[1]} at the targets")
+    return Fs, Ft
+
+
+def dual_kriging(solve, cross, y, F, FT):
+    """Dual-form kriging given solve(R) = C^-1 R and cross(w) = C(T, S) w: one solve C [alpha | B_F] = [y | F], then
+    beta = (F' B_F)^-1 F' alpha (p x p), w = alpha - B_F beta and yhat = F_T beta + C(T, S) w.  This is the solution
+    of the bordered system [C F; F' 0] [w; beta] = [y; 0]; p = 0 is simple kriging."""
+    p = F.shape[1]
+    Xs = solve(np.column_stack([y, F]))
+    alpha, BF = Xs[:, 0], Xs[:, 1:]
+    if p:
+        beta = np.linalg.solve(F.T @ BF, F.T @ alpha)
+        w = alpha - BF @ beta
+    else:
+        beta = np.zeros(0)
+        w = alpha
+    return FT @ beta + cross(w), beta, w
+
+
+def krige(structures, sources, y, targets, *, nugget=0.0, drift=None, rtol=1e-10, rank=0, rng=None,
+          return_weights=False):
+    """Kriging estimate at the targets (d x m) from observations y at the sources (d x n) under the nested covariance
+    model `structures` (CovStructure list) plus `nugget` on the observations, in dual (matrix-free) form.
+
+    drift=None: simple kriging (known zero mean); "constant": ordinary kriging; (F_sources n x p, F_targets m x p):
+    universal kriging / kriging with external drift.  The n x (1 + p) right-hand side is one cov_solve (rank > 0: with
+    a Nystrom preconditioner of that rank).  Returns yhat (m), or (yhat, beta, w) with return_weights=True."""
+    S, T = _f64_colmajor(sources), _f64_colmajor(targets)
+    n, m = S.shape[1], T.shape[1]
+    y = np.asarray(y, dtype=np.float64).reshape(n)
+    F, FT = drift_matrices(drift, n, m)
+    C_ss = KernelCovModelMatrix(structures, S, nugget)
+    C_ts = KernelCrossCovMatrix(structures, T, S, ctx=C_ss.ctx)
+    try:
+        yhat, beta, w = dual_kriging(lambda R: cov_solve(C_ss, R, rtol=rtol, rank=rank, rng=rng)[0],
+                                     lambda w: C_ts.apply(w.reshape(n, 1))[:, 0], y, F, FT)
+    finally:
+        C_ss.free()
+        C_ts.free()
+    return (yhat, beta, w) if return_weights else yhat

@@ -275,6 +275,30 @@ int32_t gsi_rangefinder_adaptive_blocked(gsi_op* op, const gsi_buf* omegas, doub
                                          gsi_buf* Q_out, int64_t* j_out);
 /* eig_nystrom(A, Q) (src/RandMatFact.jl:92-102): U_out TALL n x l, Sigma_host l.      */
 int32_t gsi_eig_nystrom(gsi_op* op, const gsi_buf* Q, gsi_buf* U_out, double* Sigma_host);
+/* Kriging solve (no reference counterpart): X = A^-1 B for a square kernel-covariance operator A (gsi_op_kernelcov,
+ * _grid, _model or _model_grid), exactly as built, nugget included -- the weights w = (C(S, S) + nugget I)^-1 (y - drift)
+ * that C(T, S) w needs, without forming the n x n matrix.  Dense, low-rank and cross-covariance operators:
+ * GSI_ERR_UNSUPPORTED.
+ *   B      TALL n x k (1 <= k <= 1024), all n rows on every rank (as Omega of gsi_randsvd).
+ *   X      TALL n x k or this rank's mloc x k (the row-count rule of gsi_rangefinder_fixed / gsi_randsvd outputs).
+ *   The k columns run independent preconditioned conjugate-gradient recurrences that share one operator product of
+ *   width k per iteration (not block CG).  Column j has converged when its recursively updated residual satisfies
+ *   ||r_j|| <= rtol ||b_j||; from then on its x_j is frozen.  A zero column of B gives x_j = 0 after 0 iterations.
+ *   iters_out[k]   iteration at which each column converged (unconverged: the iterations run)
+ *   relres_out[k]  TRUE relative residual ||b_j - A x_j|| / ||b_j|| of the returned X (one extra product; 0 if b_j = 0)
+ *   lambda_out[r]  optional (NULL allowed): the Nystrom eigenvalue estimates, descending
+ * Omega: NULL (no preconditioner) or a TALL n x r Gaussian sketch drawn by the host, 1 <= r <= 256, r < n: the
+ * randomized Nystrom preconditioner of Frangella, Tropp and Udell (SIMAX 2023, Alg. 2.1 and eq. 1.3) of A = K + mu I,
+ * mu = the operator's nugget: Omega <- thin Q of Omega, Y = A Omega - mu Omega, nu = sqrt(n) 2^-52 ||Y||_F,
+ * Y_nu = Y + nu Omega, C = chol(Omega' Y_nu), F = Y_nu C^-1 = U Sigma V', lambda = max(0, Sigma^2 - nu), applied as
+ * P^-1 R = R + U diag((lambda_r + mu) / (lambda_i + mu) - 1) U'R.
+ * Results are bit-reproducible run to run on a given GPU count (fixed reduction order, no atomics).
+ * Errors: maxiter reached with a column unconverged: GSI_ERR_NO_CONVERGENCE (X, iters_out and relres_out are still
+ * filled); p'Ap <= 0, a failed Cholesky of the sketch or lambda_r + mu <= 0: GSI_ERR_NOT_POSDEF (add a nugget or use a
+ * smaller r); bad shapes: GSI_ERR_DIMENSION_MISMATCH; rtol <= 0 or not finite, maxiter < 0, a non-finite entry of B or
+ * Omega, or r outside 1..min(256, n - 1): GSI_ERR_INVALID_ARGUMENT.                                                        */
+int32_t gsi_kernelcov_solve(gsi_op* op, const gsi_buf* B, const gsi_buf* Omega, double rtol, int64_t maxiter,
+                            gsi_buf* X, int64_t* iters_out, double* relres_out, double* lambda_out);
 
 /* FFTRF.powerlaw_structuredgrid (src/FFTRF.jl:83-100) for a batch of fields, on the device -- the
  * sampler behind getxis(samplefield, numfields, ...) (src/GeostatInversion.jl:29-38).  dim in {2, 3};

@@ -9,6 +9,7 @@
 #   eig_nystrom(A, Q), getxis(Q, numxis, p, q, seed), getxis(samplefield, numfields, numxis, p, q, seed),
 #   getxis(Val{:iwantfields}, ...), pcgalsqr / pcgadirect / pcga / rga with the reference's
 #   positional and keyword arguments,
+# plus covsolve(C, B; rtol, maxiter, rank, seed) and krige(...) on the kernel-covariance operators (new),
 # for A::Matrix{Float64}, A::KernelCovMatrix (new), A::KernelCrossCovMatrix (new, not symmetric) and
 # A::LowRankCovMatrix, whose method set is
 # the one the reference's LowRankCovMatrix provides (src/lowrank.jl:38-60,115-139):
@@ -332,6 +333,70 @@ Base.:*(a::AdjointOperator, X::Matrix{Float64}) = apply(a.parent, true, X)      
 Base.:*(a::AdjointOperator, x::Vector{Float64}) = vec(apply(a.parent, true, reshape(x, :, 1)))
 # `B' * A = (A' * B)'` (src/lowrank.jl:131-133; RandMatFact.jl:85 `Q' * A`)
 Base.:*(Bt::LinearAlgebra.Adjoint{Float64, Matrix{Float64}}, op::Operator) = Matrix(apply(op, true, Matrix(parent(Bt)))')
+
+"""
+covsolve(C, B; rtol=1e-10, maxiter=nothing, rank=0, seed=nothing, full=false) -> (X, info)
+
+X = C \\ B for a square kernel-covariance operator (KernelCovMatrix, KernelCovGrid, KernelCovModel, KernelCovModelGrid;
+nugget included) by gsi_kernelcov_solve: one preconditioned CG recurrence per column of B (k <= 1024), sharing one
+operator product per iteration; column j stops at ||r_j|| <= rtol ||b_j||.  rank > 0 draws an n x rank Gaussian sketch
+(`randn`, after `Random.seed!(seed)` when a seed is given) for the randomized Nystrom preconditioner (rank <= 256,
+rank < n).  maxiter = nothing means n.  info: iterations, relres (true ||b - C x|| / ||b||), nystrom_eigenvalues.
+Multi-GPU: this worker's rows of X unless full = true.
+"""
+function covsolve(C::KernelCovMatrix, B::VecOrMat{Float64}; rtol::Float64=1e-10, maxiter::Union{Nothing, Int}=nothing,
+		rank::Int=0, seed::Union{Nothing, Int}=nothing, full::Bool=false)
+	seed === nothing || Random.seed!(seed)
+	n = size(C, 2)
+	Bm = Matrix{Float64}(reshape(B, n, :))
+	k = size(Bm, 2)
+	Bd = upload!(DeviceMatrix(C.ctx, GSI_LAYOUT_TALL, n, k), Bm)
+	Om = rank > 0 ? upload!(DeviceMatrix(C.ctx, GSI_LAYOUT_TALL, n, rank), randn(n, rank)) : nothing
+	Xd = DeviceMatrix(C.ctx, GSI_LAYOUT_TALL, (full || C.ctx.world == 1) ? n : length(C.rows), k)
+	iters = zeros(Int64, k); relres = zeros(k); lambda = zeros(max(rank, 1))
+	status = GC.@preserve iters relres lambda ccall((:gsi_kernelcov_solve, LIB), Int32,
+		(Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Float64, Int64, Ptr{Cvoid}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}),
+		C.h, Bd.h, Om === nothing ? C_NULL : Om.h, rtol, maxiter === nothing ? n : maxiter, Xd.h, iters, relres, lambda)
+	(status == 0 || status == 10) || check(status)
+	X = download(Xd)
+	X = B isa Vector ? vec(X) : X
+	info = (iterations=iters, relres=relres, nystrom_eigenvalues=lambda[1:rank])
+	status == 10 && throw(CovSolveNoConvergence(lasterror(), X, info))     # X, iterations and relres are filled
+	return X, info
+end
+
+"a column of covsolve did not reach rtol within maxiter iterations; `X` and `info` are those of the returned solve"
+struct CovSolveNoConvergence <: Exception
+	msg::String
+	X::VecOrMat{Float64}
+	info::NamedTuple
+end
+Base.showerror(io::IO, e::CovSolveNoConvergence) = print(io, "CovSolveNoConvergence: ", e.msg)
+
+"""
+krige(kinds, sills, ranges, sources, y, targets; rotations, betas, nugget=0.0, drift=nothing, rtol=1e-10, rank=0,
+      seed=nothing) -> (yhat, beta, w)
+
+Dual-form kriging at the targets (d x m) from observations y at the sources (d x n) under the nested model of
+KernelCovModel plus `nugget`: one covsolve of C [alpha | B_F] = [y | F], beta = (F' B_F) \\ (F' alpha),
+w = alpha - B_F beta, yhat = F_T beta + C(T, S) w (multi-GPU: this worker's block of target rows, as `Cx * w`).  drift = nothing: simple kriging; :constant: ordinary kriging;
+(F_sources n x p, F_targets m x p): universal kriging / kriging with external drift.
+"""
+function krige(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, sources::Matrix{Float64},
+		y::Vector{Float64}, targets::Matrix{Float64}; rotations::Union{Nothing, Array{Float64, 3}}=nothing,
+		betas::Union{Nothing, Vector{Float64}}=nothing, nugget=0.0, drift=nothing, rtol::Float64=1e-10, rank::Int=0,
+		seed::Union{Nothing, Int}=nothing)
+	n, m = size(sources, 2), size(targets, 2)
+	F, FT = drift === nothing ? (zeros(n, 0), zeros(m, 0)) :
+		drift === :constant ? (ones(n, 1), ones(m, 1)) : (Matrix{Float64}(drift[1]), Matrix{Float64}(drift[2]))
+	C = KernelCovModel(kinds, sills, ranges, sources; rotations=rotations, betas=betas, nugget=nugget)
+	Cx = KernelCrossCov(kinds, sills, ranges, targets, sources; rotations=rotations, betas=betas)
+	X, _ = covsolve(C, hcat(y, F); rtol=rtol, rank=rank, seed=seed, full=true)
+	alpha, BF = X[:, 1], X[:, 2:end]
+	beta = size(F, 2) > 0 ? (F' * BF) \ (F' * alpha) : zeros(0)
+	w = alpha - BF * beta
+	return FT[Cx.rows, :] * beta + Cx * w, beta, w                 # this worker's target rows (all on one GPU)
+end
 
 module RandMatFact
 import ..GeostatInversionB200: LIB, check, context, Operator, DenseOperator, DeviceMatrix, upload!, download,

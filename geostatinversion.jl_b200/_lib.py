@@ -90,6 +90,14 @@ SIGNATURES = {
     "gsi_rangefinder_adaptive_blocked": (_i32, [_p, _p, _f64, _i64, _p, _pi64]),
     "gsi_eig_nystrom": (_i32, [_p, _p, _p, _pd]),
     "gsi_kernelcov_solve": (_i32, [_p, _p, _p, _f64, _i64, _p, _pi64, _pd, _pd]),
+    "gsi_op_kernelcov_block": (_i32, [_p, _i64, _i64, _p]),
+    "gsi_kernelcov_chol": (_i32, [_p, _pp, _pi64]),
+    "gsi_chol_free": (_i32, [_p]),
+    "gsi_chol_size": (_i32, [_p, _pi64]),
+    "gsi_chol_logdet": (_i32, [_p, _pd]),
+    "gsi_chol_download": (_i32, [_p, _pd, _i64]),
+    "gsi_chol_solve": (_i32, [_p, _i32, _p, _p]),
+    "gsi_chol_krige_variance": (_i32, [_p, _p, _pd, _pd, _i64, _pd]),
     "gsi_fftrf_powerlaw": (_i32, [_p, _i32, _pi64, _f64, _f64, _f64, _p, _p]),
     "gsi_pcga_lowrank_matvec": (_i32, [_p, _i64, _i64, _pd, _i64, _pd, _pd, _pd, _i64, _pd, _pd]),
     "gsi_pcga_lsqr_solve": (_i32, [_p, _i64, _i64, _pd, _i64, _pd, _pd, _pd, _i64, _pd, _f64, _f64, _f64,

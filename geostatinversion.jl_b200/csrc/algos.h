@@ -36,5 +36,17 @@ __global__ void tall_head_to_cm_kernel(const double* __restrict__ T, int64_t ld,
 // ---- cov_solve.cu: A X = B on a square kernel-covariance operator, preconditioned CG (one recurrence per column)
 void kernelcov_solve(gsi_op* op, const gsi_buf* B, const gsi_buf* Omega, double rtol, int64_t maxiter, gsi_buf* X_out,
                      int64_t* iters_out, double* relres_out, double* lambda_out);
+// out[c] = sum_i X[i, c] Y[i, c] over rows x cols of TALL blocks (pitch ld) by the solver's fixed-order column
+// reduction; part: CS_PARTS_MAX * cols doubles of scratch; nonfinite (optional) is set when an entry of X is not finite
+constexpr int CS_PARTS_MAX = 256;
+void col_dot(gsi_ctx* ctx, const double* X, const double* Y, int64_t ld, int64_t rows, int64_t cols, double* part,
+             double* out, int* nonfinite);
+
+// ---- cov_chol.cu: dense Cholesky factor of a square kernel-covariance operator, solves and kriging variance
+gsi_chol* chol_factor(gsi_op* op, int64_t* failed_column);      // *failed_column: 1-based, 0 unless NOT_POSDEF
+void chol_destroy(gsi_chol* f);
+void chol_download(const gsi_chol* f, double* host, int64_t ldh);
+void chol_solve(const gsi_chol* f, int half, const gsi_buf* B, gsi_buf* X);
+void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const double* Ft, int64_t p, double* var_out);
 
 }  // namespace gsi

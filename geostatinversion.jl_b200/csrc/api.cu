@@ -1005,3 +1005,83 @@ GSI_API int32_t gsi_kernelcov_solve(gsi_op* op, const gsi_buf* B, const gsi_buf*
         kernelcov_solve(op, B, Omega, rtol, maxiter, X, iters_out, relres_out, lambda_out);
     });
 }
+
+GSI_API int32_t gsi_op_kernelcov_block(gsi_op* op, int64_t row0, int64_t col0, gsi_buf* out) {
+    return guarded([&] {
+        GSI_REQUIRE(op && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(op->ctx);
+        GSI_REQUIRE(op->type == OP_KERNELCOV || op->type == OP_KERNELCROSS, GSI_ERR_UNSUPPORTED,
+                    "kernelcov_block needs a kernel-covariance operator");
+        GSI_REQUIRE(out->layout == GSI_LAYOUT_COLMAJOR, GSI_ERR_DIMENSION_MISMATCH, "kernelcov_block: out must be COLMAJOR");
+        const bool cross = op->type == OP_KERNELCROSS;
+        const int64_t nrows = cross ? op->mloc : op->n;
+        GSI_REQUIRE(row0 >= 0 && col0 >= 0 && row0 + out->rows <= nrows && col0 + out->cols <= op->n,
+                    GSI_ERR_DIMENSION_MISMATCH, "kernelcov_block: the block lies outside the operator");
+        KcovBlock b;
+        b.r0 = row0; b.rows = out->rows; b.c0 = col0; b.cols = out->cols;
+        b.nr_valid = nrows; b.nc_valid = op->n; b.nugget_diag = cross ? 0 : 1; b.lower = 0;
+        b.out = out->d; b.rs = 1; b.cs = out->ld;
+        kcov_block(op, cross ? KB_CROSS : KB_SQUARE, b);
+        GSI_CUDA(cudaStreamSynchronize(op->ctx->stream));
+    });
+}
+
+GSI_API int32_t gsi_kernelcov_chol(gsi_op* op, gsi_chol** out, int64_t* failed_column_out) {
+    if (failed_column_out) *failed_column_out = 0;
+    return guarded([&] {
+        GSI_REQUIRE(op && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(op->ctx);
+        *out = nullptr;
+        gsi_chol* f = chol_factor(op, failed_column_out);
+        ctx_retain(op->ctx);
+        *out = f;
+    });
+}
+
+GSI_API int32_t gsi_chol_free(gsi_chol* f) {
+    if (!f) return GSI_OK;
+    return guarded([&] {
+        gsi_ctx* c = f->ctx;
+        chol_destroy(f);
+        ctx_release(c);
+    });
+}
+
+GSI_API int32_t gsi_chol_size(const gsi_chol* f, int64_t* n_out) {
+    return guarded([&] {
+        GSI_REQUIRE(f && n_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        *n_out = f->n;
+    });
+}
+
+GSI_API int32_t gsi_chol_logdet(const gsi_chol* f, double* logdet_out) {
+    return guarded([&] {
+        GSI_REQUIRE(f && logdet_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        *logdet_out = f->logdet;
+    });
+}
+
+GSI_API int32_t gsi_chol_download(const gsi_chol* f, double* L_host, int64_t ldh) {
+    return guarded([&] {
+        GSI_REQUIRE(f, GSI_ERR_INVALID_ARGUMENT, "null factor");
+        use(f->ctx);
+        chol_download(f, L_host, ldh);
+    });
+}
+
+GSI_API int32_t gsi_chol_solve(gsi_chol* f, int32_t half, const gsi_buf* B, gsi_buf* X) {
+    return guarded([&] {
+        GSI_REQUIRE(f && B && X, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(f->ctx);
+        chol_solve(f, half, B, X);
+    });
+}
+
+GSI_API int32_t gsi_chol_krige_variance(gsi_chol* f, gsi_op* cross, const double* F_s, const double* F_t, int64_t p,
+                                        double* var_out) {
+    return guarded([&] {
+        GSI_REQUIRE(f && cross && var_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(f->ctx);
+        chol_variance(f, cross, F_s, F_t, p, var_out);
+    });
+}

@@ -165,6 +165,18 @@ struct gsi_op {
     std::vector<int64_t> part;           // row partition over ranks: part[r] .. part[r+1]
 };
 
+// dense Cholesky factor A = L L' of a square kernel-covariance operator (cov_chol.cu)
+struct gsi_chol {
+    gsi_ctx* ctx = nullptr;
+    int64_t n = 0;
+    int64_t np = 0;                      // n rounded up to the 128-column block; the padding is the identity
+    double* L = nullptr;                 // column-major np x np (pitch np), lower triangle
+    double* inv = nullptr;               // the np / 128 inverses of the diagonal blocks of L, 128 x 128 column-major each
+    double* info = nullptr;              // [0] failed column (int), [1] log det, [2..3] status flags of solve / variance
+    int* flags = nullptr;                // (int*)(info + 2)
+    double logdet = 0.0;
+};
+
 namespace gsi {
 
 // ---- tall_ops.cu
@@ -183,6 +195,18 @@ void colmajor_download(const gsi_buf* b, double* host, int64_t ldh);
 
 // ---- kcov_gemm.cu :  W[local rows] = C[rows, :] * X  (cross-covariance: trans = 1 gives W = C' X, all n rows)
 void kcov_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* W);
+// a materialised block of a kernel-covariance operator, entry (i, j) at out[(i - r0) * rs + (j - c0) * cs]
+// (kcov_gemm.cu, kcov_block_kernel: the product kernel's value code)
+enum { KB_SQUARE = 0, KB_CROSS = 1, KB_CROSS_T = 2, KB_TARGETS = 3 };
+struct KcovBlock {
+    int64_t r0, rows, c0, cols;
+    int64_t nr_valid, nc_valid;   // row / column points; entries beyond them are padding (1 on the diagonal, else 0)
+    int nugget_diag;              // add the nugget where i == j
+    int lower;                    // skip 64 x 64 tiles above the diagonal
+    double* out;
+    int64_t rs, cs;
+};
+void kcov_block(gsi_op* op, int side, const KcovBlock& b);
 // ---- dense_gemm.cu : W = A X (trans=0) or A' X (trans=1); alpha scaling
 void dense_apply(gsi_ctx*, const gsi_buf* A, int trans, const gsi_buf* X, gsi_buf* W, double alpha);
 void tall_window_update(gsi_ctx*, const double* Pd, int64_t ldp, int64_t rows, int64_t kdim, const gsi_buf* X,
@@ -213,7 +237,8 @@ void comm_unique_id(void* out128);
 
 inline void count_launch(gsi_ctx* c, int n = 1) { c->launches += n; }
 // ---- algos.cu: event-pair phase timing (active only while time_gemm is on)
-enum Phase { PH_GEMM = 0, PH_LU = 1, PH_QR = 2, PH_SVD = 3, PH_BACKMUL = 4 };
+enum Phase { PH_GEMM = 0, PH_LU = 1, PH_QR = 2, PH_SVD = 3, PH_BACKMUL = 4, PH_CHOL_FILL = 5, PH_CHOL_DIAG = 6,
+             PH_CHOL_PANEL = 7 };
 void phase_begin(gsi_ctx*);
 void phase_end(gsi_ctx*, int phase);
 // ---- api.cu: pooled device memory

@@ -1,0 +1,531 @@
+// Direct kriging on a dense Cholesky factor of a square kernel-covariance operator: A = L L' (nugget included), the
+// solves A^-1 B and L^-1 B, log det A, and the kriging variance of C(T, S) targets.  For the n of most kriging problems
+// (thousands to tens of thousands of observations) the n^3 / 3 flops of one factorisation cost less than one CG solve
+// (cov_solve.cu) and serve any number of right-hand sides; the variance needs one triangular solve per target, which
+// CG cannot offer at a useful price.
+//
+// Storage: the factor's order is rounded up to np = a multiple of CH_B = 128 and the padding is the identity,
+// A_pad = [A 0; 0 I] = [L 0; 0 I][L 0; 0 I]', so every kernel works on whole 128 x 128 tiles.  L is column-major with
+// pitch np (a multiple of 128 doubles: 16-byte aligned columns for cp.async), lower triangle only; the inverses of the
+// np / 128 diagonal blocks are kept beside it (128 x 128 each) for the triangular solves.
+//
+// Blocked right-looking factorisation, for each 128-column block k:
+//   1. chol_diag_kernel: L11 = chol(A11) and X11 = L11^-1, one CTA, the block resident in shared memory
+//   2. panel:            L21 = A21 X11'                  (chol_gemm_kernel, set)
+//   3. trailing update:  A22 -= L21 L21', lower tiles only (chol_gemm_kernel, subtract) -- the n^3 / 3 flops
+// chol_gemm_kernel is one "C = / -= A B'" kernel on FP64 tensor cores (mma.sync.m8n8k4.f64 -> DMMA.8x8x4) with the
+// 16-warp structure of the product kernels: a 128 x 128 tile per CTA, warps 4 x 4 over it, 32 x 32 each; k-tiles of 32
+// staged through a double-buffered shared tile [k][row] (pitch 136 = 8 mod 16 doubles: the four k rows of a fragment
+// load fall into the two halves of the banks -- two wavefronts for 32 doubles, the minimum).  Operand layouts are
+// template parameters, so the same kernel serves the solves: forward B_j = X_jj B_j, B_(>j) -= L_(>j, j) B_j; backward
+// B_j = X_jj' B_j, B_(<j) -= L_(j, <j)' B_j, on a row-major work block of width 128 .. 1024.
+// Every reduction has a fixed order (no atomics): factor, solve, log-determinant and variance are bit-reproducible.
+#include "common.cuh"
+#include "algos.h"
+#include "ptx.cuh"
+#include <cmath>
+
+namespace gsi {
+
+constexpr int CH_B = 128;              // block width of the factorisation and GEMM tile (rows and columns)
+constexpr int CH_K = 32;               // k values per pipeline stage of chol_gemm_kernel
+constexpr int CH_P = CH_B + 8;         // pitch of a [k][128] shared operand tile
+constexpr int CH_THREADS = 512;
+constexpr int CH_TILE = CH_K * CH_P;   // doubles of one operand tile
+constexpr size_t CH_GEMM_SMEM = (size_t)2 * 2 * CH_TILE * sizeof(double);     // 2 stages x (A, B)
+constexpr int CD_P = CH_B + 1;         // pitch of the diagonal block in shared memory
+constexpr size_t CH_DIAG_SMEM = ((size_t)CH_B * CD_P + CH_B) * sizeof(double);
+constexpr int CH_MAX_DRIFT = 32;       // drift columns of the universal-kriging variance
+constexpr int CH_MAX_CHUNK = kMaxWideCols;
+
+// C (+)= A B' on 128 x 128 tiles.  A(m, k) = A_KC ? A[m * lda + k] : A[k * lda + m];  B(n, k) likewise with B_KC;
+// C(m, n) = C_ROW ? C[m * ldc + n] : C[n * ldc + m].  K is a multiple of CH_K.  lower: only the tiles (i, j), j <= i,
+// of an mt x mt grid, blockIdx.x = i (i + 1) / 2 + j; otherwise blockIdx = (column tile, row tile).
+struct ChGemm {
+    const double* A; int64_t lda;
+    const double* B; int64_t ldb;
+    double* C; int64_t ldc;
+    int64_t K;
+    int sub;       // 1: C -= A B'   0: C = A B'
+    int lower;
+};
+
+__device__ __forceinline__ void cp_async16(void* s, const void* g) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(smem_u32(s)), "l"(g) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N) : "memory"); }
+
+// one operand tile, 128 rows (m or n) x CH_K k values, into s[k * CH_P + row]
+template <bool KC>
+__device__ __forceinline__ void ch_load_tile(double* s, const double* g, int64_t ld, int64_t row0, int64_t k0, int tid) {
+    if constexpr (!KC) {
+        // (row, k) at g[k * ld + row]: 16-byte asynchronous copies along the rows
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int c = tid + q * CH_THREADS;
+            const int k = c >> 6, r2 = (c & 63) * 2;
+            cp_async16(s + k * CH_P + r2, g + (k0 + k) * ld + row0 + r2);
+        }
+    } else {
+        // (row, k) at g[row * ld + k]: pairs along k through registers, transposed into shared memory (a lane per row:
+        // conflict-free stores)
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const int c = tid + q * CH_THREADS;
+            const int r = c & (CH_B - 1), k2 = (c >> 7) * 2;
+            const double2 v = __ldg(reinterpret_cast<const double2*>(g + (row0 + r) * ld + k0 + k2));
+            s[k2 * CH_P + r] = v.x;
+            s[(k2 + 1) * CH_P + r] = v.y;
+        }
+    }
+}
+
+template <bool A_KC, bool B_KC, bool C_ROW>
+__global__ void __launch_bounds__(CH_THREADS, 1) chol_gemm_kernel(const ChGemm a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    double* sm = reinterpret_cast<double*>(smem_raw);
+    int64_t ti, tj;
+    if (a.lower) {
+        const int64_t t = blockIdx.x;
+        int64_t i = (int64_t)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
+        while ((i + 1) * (i + 2) / 2 <= t) ++i;
+        while (i * (i + 1) / 2 > t) --i;
+        ti = i;
+        tj = t - i * (i + 1) / 2;
+    } else {
+        ti = blockIdx.y;
+        tj = blockIdx.x;
+    }
+    const int64_t m0 = ti * CH_B, n0 = tj * CH_B;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int g = lane >> 2, t = lane & 3;
+    const int wm = warp & 3, wn = warp >> 2;
+    double acc[4][4][2];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
+    const int nk = (int)(a.K / CH_K);
+    auto load = [&](int st, int kt) {
+        double* sa = sm + (size_t)st * 2 * CH_TILE;
+        ch_load_tile<A_KC>(sa, a.A, a.lda, m0, (int64_t)kt * CH_K, tid);
+        ch_load_tile<B_KC>(sa + CH_TILE, a.B, a.ldb, n0, (int64_t)kt * CH_K, tid);
+        cp_async_commit();
+    };
+    load(0, 0);
+    for (int kt = 0; kt < nk; ++kt) {
+        if (kt + 1 < nk) {
+            load((kt + 1) & 1, kt + 1);
+            cp_async_wait<1>();
+        } else {
+            cp_async_wait<0>();
+        }
+        __syncthreads();
+        const double* sa = sm + (size_t)(kt & 1) * 2 * CH_TILE;
+        const double* sb = sa + CH_TILE;
+#pragma unroll
+        for (int ks = 0; ks < CH_K / 4; ++ks) {
+            const double* ar = sa + (ks * 4 + t) * CH_P + wm * 32 + g;
+            const double* br = sb + (ks * 4 + t) * CH_P + wn * 32 + g;
+            double af[4], bf[4];
+#pragma unroll
+            for (int f = 0; f < 4; ++f) { af[f] = ar[f * 8]; bf[f] = br[f * 8]; }
+#pragma unroll
+            for (int fm = 0; fm < 4; ++fm)
+#pragma unroll
+                for (int fn = 0; fn < 4; ++fn) dmma884(acc[fm][fn][0], acc[fm][fn][1], af[fm], bf[fn]);
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int fm = 0; fm < 4; ++fm) {
+        const int64_t m = m0 + wm * 32 + fm * 8 + g;
+#pragma unroll
+        for (int fn = 0; fn < 4; ++fn) {
+            const int64_t n = n0 + wn * 32 + fn * 8 + 2 * t;
+            if constexpr (C_ROW) {
+                double2* c = reinterpret_cast<double2*>(a.C + m * a.ldc + n);
+                double2 v = make_double2(acc[fm][fn][0], acc[fm][fn][1]);
+                if (a.sub) { const double2 o = *c; v.x = o.x - v.x; v.y = o.y - v.y; }
+                *c = v;
+            } else {
+                double* c0 = a.C + n * a.ldc + m;
+                double* c1 = c0 + a.ldc;
+                if (a.sub) { *c0 -= acc[fm][fn][0]; *c1 -= acc[fm][fn][1]; }
+                else { *c0 = acc[fm][fn][0]; *c1 = acc[fm][fn][1]; }
+            }
+        }
+    }
+}
+
+// Diagonal block (k0, k0) of the column-major A (pitch lda): L11 = chol(A11) into A's lower triangle, X11 = L11^-1 into
+// inv (column-major 128 x 128, zero above the diagonal).  Shared S[r * CD_P + c]: the strict lower triangle holds L, the
+// upper triangle X transposed (S[c][r] = X(r, c), r > c), dg the diagonal of L.  A pivot that is not positive (or NaN)
+// records the 1-based global column in *info (the first failure wins; later launches return at once).
+__global__ void __launch_bounds__(CH_THREADS, 1) chol_diag_kernel(double* __restrict__ A, int64_t lda, int64_t k0,
+                                                                  double* __restrict__ inv, int* __restrict__ info) {
+    extern __shared__ __align__(16) double S[];
+    double* dg = S + CH_B * CD_P;
+    if (*info != 0) return;
+    const int tid = threadIdx.x;
+    for (int e = tid; e < CH_B * CH_B; e += CH_THREADS) {
+        const int r = e & (CH_B - 1), c = e >> 7;
+        if (r >= c) S[r * CD_P + c] = A[(k0 + c) * lda + k0 + r];
+    }
+    __syncthreads();
+    // right-looking, column by column: thread (r = tid & 127, phase tid >> 7) updates row r, columns phase, phase + 4, ..
+    const int r = tid & (CH_B - 1), ph = tid >> 7;
+    for (int j = 0; j < CH_B; ++j) {
+        const double d = S[j * CD_P + j];
+        __syncthreads();                                        // every thread has read the pivot
+        if (!(d > 0.0)) {
+            if (tid == 0) atomicCAS(info, 0, (int)(k0 + j + 1));
+            return;                                             // uniform: all threads saw the same d
+        }
+        const double s = sqrt(d);
+        if (tid == 0) dg[j] = s;
+        if (ph == 0 && r > j) S[r * CD_P + j] /= s;
+        __syncthreads();
+        if (r > j) {
+            const double lr = S[r * CD_P + j];
+            for (int c = j + 1 + ph; c <= r; c += 4) S[r * CD_P + c] -= lr * S[c * CD_P + j];
+        }
+        __syncthreads();
+    }
+    // X = L^-1 row by row: X(i, i) = 1 / L(i, i), X(i, c) = -(sum_{c <= k < i} L(i, k) X(k, c)) / L(i, i); thread
+    // (c = tid >> 2, q = tid & 3) adds k = c + q, c + q + 4, .. and the four quarters meet by shuffles (fixed order)
+    const int c = tid >> 2, q = tid & 3;
+    for (int i = 1; i < CH_B; ++i) {
+        double sum = 0.0;
+        if (c < i)
+            for (int k = c + q; k < i; k += 4) sum += S[i * CD_P + k] * (k == c ? 1.0 / dg[c] : S[c * CD_P + k]);
+        sum += __shfl_xor_sync(0xffffffffu, sum, 1);
+        sum += __shfl_xor_sync(0xffffffffu, sum, 2);
+        if (q == 0 && c < i) S[c * CD_P + i] = -sum / dg[i];
+        __syncthreads();
+    }
+    for (int e = tid; e < CH_B * CH_B; e += CH_THREADS) {
+        const int rr = e & (CH_B - 1), cc = e >> 7;
+        if (rr > cc) A[(k0 + cc) * lda + k0 + rr] = S[rr * CD_P + cc];
+        else if (rr == cc) A[(k0 + cc) * lda + k0 + rr] = dg[rr];
+        inv[cc * CH_B + rr] = rr > cc ? S[cc * CD_P + rr] : (rr == cc ? 1.0 / dg[rr] : 0.0);
+    }
+}
+
+// log det = 2 sum_i log L(i, i) over the n true rows: one CTA, thread t adds i = t, t + 1024, .. in order, then a fixed
+// tree
+__global__ void chol_logdet_kernel(const double* __restrict__ L, int64_t ld, int64_t n, double* __restrict__ out) {
+    __shared__ double red[1024];
+    double s = 0.0;
+    for (int64_t i = threadIdx.x; i < n; i += 1024) s += log(L[i * ld + i]);
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = 512; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) out[0] = 2.0 * red[0];
+}
+
+// *flag = 1 when an entry of the rows x cols TALL block (pitch ld) is not finite
+__global__ void chol_nonfinite_kernel(const double* __restrict__ X, int64_t ld, int64_t rows, int64_t cols, int* flag) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= rows * cols) return;
+    const int64_t i = idx / cols, c = idx - i * cols;
+    if (!isfinite(X[i * ld + c])) *flag = 1;
+}
+
+// var[c] = c(t, t) - ||L^-1 c_t||^2 (+ r' (G'G)^-1 r, r = f_t - G' L^-1 c_t, with R'R = G'G: r' (G'G)^-1 r = ||R^-T r||^2)
+// H: G' W (row-major, pitch ldh), Ft: the chunk's drift rows (column-major, pitch ldf), R: upper p x p (pitch p)
+__global__ void chol_variance_kernel(const double* __restrict__ colsq, const double* __restrict__ ctt, int64_t mc, int p,
+                                     const double* __restrict__ H, int64_t ldh, const double* __restrict__ Ft, int64_t ldf,
+                                     const double* __restrict__ R, double* __restrict__ var) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= mc) return;
+    double v = ctt[0] - colsq[c];
+    if (p > 0) {
+        double z[CH_MAX_DRIFT];
+        double acc = 0.0;
+#pragma unroll
+        for (int i = 0; i < CH_MAX_DRIFT; ++i) {
+            z[i] = 0.0;
+            if (i < p) {
+                double s = Ft[c + i * ldf] - H[i * ldh + c];
+#pragma unroll
+                for (int k = 0; k < i; ++k) s -= R[k + i * p] * z[k];
+                z[i] = s / R[i + i * p];
+                acc += z[i] * z[i];
+            }
+        }
+        v += acc;
+    }
+    var[c] = v;
+}
+
+namespace {
+
+template <bool AK, bool BK, bool CR>
+void gemm(gsi_ctx* ctx, const ChGemm& a, int64_t mt, int64_t nt) {
+    if (mt <= 0 || nt <= 0) return;
+    auto kfn = chol_gemm_kernel<AK, BK, CR>;
+    GSI_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CH_GEMM_SMEM));
+    const dim3 grid = a.lower ? dim3((unsigned)(mt * (mt + 1) / 2)) : dim3((unsigned)nt, (unsigned)mt);
+    kfn<<<grid, CH_THREADS, CH_GEMM_SMEM, ctx->stream>>>(a);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+}
+
+ChGemm gm(const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc, int64_t K, int sub, int lower) {
+    ChGemm a;
+    a.A = A; a.lda = lda; a.B = B; a.ldb = ldb; a.C = C; a.ldc = ldc; a.K = K; a.sub = sub; a.lower = lower;
+    return a;
+}
+
+// W (row-major np x kp, pitch ldw; kp a multiple of 128) <- L^-1 W
+void forward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp) {
+    gsi_ctx* ctx = f->ctx;
+    const int64_t nb = f->np / CH_B, nt = kp / CH_B;
+    for (int64_t kb = 0; kb < nb; ++kb) {
+        const int64_t j0 = kb * CH_B;
+        double* Wj = W + j0 * ldw;
+        gemm<false, false, true>(ctx, gm(f->inv + kb * CH_B * CH_B, CH_B, Wj, ldw, Wj, ldw, CH_B, 0, 0), 1, nt);
+        gemm<false, false, true>(ctx, gm(f->L + j0 * f->np + j0 + CH_B, f->np, Wj, ldw, Wj + CH_B * ldw, ldw, CH_B, 1, 0),
+                                 nb - kb - 1, nt);
+    }
+}
+
+// W <- L^-T W
+void backward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp) {
+    gsi_ctx* ctx = f->ctx;
+    const int64_t nb = f->np / CH_B, nt = kp / CH_B;
+    for (int64_t kb = nb - 1; kb >= 0; --kb) {
+        const int64_t j0 = kb * CH_B;
+        double* Wj = W + j0 * ldw;
+        gemm<true, false, true>(ctx, gm(f->inv + kb * CH_B * CH_B, CH_B, Wj, ldw, Wj, ldw, CH_B, 0, 0), 1, nt);
+        gemm<true, false, true>(ctx, gm(f->L + j0, f->np, Wj, ldw, W, ldw, CH_B, 1, 0), kb, nt);
+    }
+}
+
+struct DevMem {
+    void* p = nullptr;
+    explicit DevMem(size_t bytes) { GSI_CUDA(cudaMalloc(&p, bytes)); }
+    ~DevMem() { if (p) cudaFree(p); }
+    double* d() const { return static_cast<double*>(p); }
+};
+
+}  // namespace
+
+void chol_destroy(gsi_chol* f) {
+    if (!f) return;
+    cudaSetDevice(f->ctx->device);
+    if (f->L) cudaFree(f->L);
+    if (f->inv) cudaFree(f->inv);
+    if (f->info) cudaFree(f->info);
+    delete f;
+}
+
+gsi_chol* chol_factor(gsi_op* op, int64_t* failed_column) {
+    gsi_ctx* ctx = op->ctx;
+    cudaStream_t st = ctx->stream;
+    if (failed_column) *failed_column = 0;
+    GSI_REQUIRE(op->type == OP_KERNELCOV, GSI_ERR_UNSUPPORTED,
+                "kernelcov_chol needs a square kernel-covariance operator (gsi_op_kernelcov, _grid, _model or _model_grid)");
+    GSI_REQUIRE(ctx->world == 1, GSI_ERR_UNSUPPORTED, "kernelcov_chol is single-GPU: the dense factor is not distributed");
+    const int64_t n = op->n, np = round_up(n, CH_B);
+    const double need = (double)np * (double)np * 8.0 + (double)np * CH_B * 8.0 + 4096.0;
+    size_t fr = 0, tot = 0;
+    GSI_CUDA(cudaMemGetInfo(&fr, &tot));
+    if (need > (double)fr) {
+        pool_release(ctx);                                        // cached iterate blocks count as free
+        GSI_CUDA(cudaMemGetInfo(&fr, &tot));
+    }
+    if (need > (double)fr) {
+        char msg[256];
+        snprintf(msg, sizeof(msg), "kernelcov_chol: the dense factor of n = %lld needs %.0f bytes of device memory, %zu are "
+                 "free (use gsi_kernelcov_solve)", (long long)n, need, fr);
+        throw Error(GSI_ERR_UNSUPPORTED, msg);
+    }
+    std::unique_ptr<gsi_chol, void (*)(gsi_chol*)> f(new gsi_chol(), chol_destroy);
+    f->ctx = ctx; f->n = n; f->np = np;
+    GSI_CUDA(cudaMalloc(&f->L, (size_t)np * np * sizeof(double)));
+    GSI_CUDA(cudaMalloc(&f->inv, (size_t)np * CH_B * sizeof(double)));
+    GSI_CUDA(cudaMalloc(&f->info, 4 * sizeof(double)));
+    GSI_CUDA(cudaMemsetAsync(f->info, 0, 4 * sizeof(double), st));
+    int* info = reinterpret_cast<int*>(f->info);
+    f->flags = reinterpret_cast<int*>(f->info + 2);
+    double* ld_out = f->info + 1;
+    // 1. the lower triangle of A, padding included
+    phase_begin(ctx);
+    KcovBlock b;
+    b.r0 = 0; b.rows = np; b.c0 = 0; b.cols = np; b.nr_valid = n; b.nc_valid = n; b.nugget_diag = 1; b.lower = 1;
+    b.out = f->L; b.rs = 1; b.cs = np;
+    kcov_block(op, KB_SQUARE, b);
+    phase_end(ctx, PH_CHOL_FILL);
+    // 2. blocked right-looking factorisation
+    GSI_CUDA(cudaFuncSetAttribute(chol_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CH_DIAG_SMEM));
+    const int64_t nb = np / CH_B;
+    for (int64_t kb = 0; kb < nb; ++kb) {
+        const int64_t k0 = kb * CH_B, mt = nb - kb - 1;
+        double* invk = f->inv + kb * CH_B * CH_B;
+        phase_begin(ctx);
+        chol_diag_kernel<<<1, CH_THREADS, CH_DIAG_SMEM, st>>>(f->L, np, k0, invk, info);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx);
+        phase_end(ctx, PH_CHOL_DIAG);
+        if (mt == 0) break;
+        double* A21 = f->L + k0 * np + k0 + CH_B;
+        phase_begin(ctx);
+        gemm<false, false, false>(ctx, gm(A21, np, invk, CH_B, A21, np, CH_B, 0, 0), mt, 1);
+        phase_end(ctx, PH_CHOL_PANEL);
+        phase_begin(ctx);
+        gemm<false, false, false>(ctx, gm(A21, np, A21, np, f->L + (k0 + CH_B) * np + k0 + CH_B, np, CH_B, 1, 1), mt, mt);
+        phase_end(ctx, PH_GEMM);
+        if (ctx->time_gemm) {
+            ctx->gemm_launches += 1;
+            ctx->gemm_flops_accum += 2.0 * CH_B * CH_B * CH_B * (double)(mt * (mt + 1) / 2);
+        }
+    }
+    int h = 0;
+    GSI_CUDA(cudaMemcpyAsync(&h, info, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    if (h != 0) {
+        if (failed_column) *failed_column = h;
+        throw Error(GSI_ERR_NOT_POSDEF, "PosDefException(" + std::to_string(h) + "): the covariance matrix is not numerically "
+                                        "positive definite at column " + std::to_string(h) + " (add a nugget)");
+    }
+    chol_logdet_kernel<<<1, 1024, 0, st>>>(f->L, np, n, ld_out);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+    GSI_CUDA(cudaMemcpyAsync(&f->logdet, ld_out, sizeof(double), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    return f.release();
+}
+
+void chol_download(const gsi_chol* f, double* host, int64_t ldh) {
+    const int64_t n = f->n;
+    GSI_REQUIRE(host != nullptr && ldh >= n, GSI_ERR_INVALID_ARGUMENT, "chol_download: null host array or ldh < n");
+    GSI_CUDA(cudaMemcpy2DAsync(host, (size_t)ldh * 8, f->L, (size_t)f->np * 8, (size_t)n * 8, (size_t)n,
+                               cudaMemcpyDeviceToHost, f->ctx->stream));
+    GSI_CUDA(cudaStreamSynchronize(f->ctx->stream));
+    for (int64_t c = 1; c < n; ++c) std::memset(host + c * ldh, 0, (size_t)c * sizeof(double));   // strict upper triangle
+}
+
+void chol_solve(const gsi_chol* f, int half, const gsi_buf* B, gsi_buf* X) {
+    gsi_ctx* ctx = f->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = f->n;
+    GSI_REQUIRE(half == 0 || half == 1, GSI_ERR_INVALID_ARGUMENT, "chol_solve: half must be 0 (A^-1 B) or 1 (L^-1 B)");
+    GSI_REQUIRE(B->layout == GSI_LAYOUT_TALL && B->rows == n, GSI_ERR_DIMENSION_MISMATCH, "chol_solve: B must be TALL n x k");
+    GSI_REQUIRE(X->layout == GSI_LAYOUT_TALL && X->rows == n && X->cols == B->cols, GSI_ERR_DIMENSION_MISMATCH,
+                "chol_solve: X must be TALL with B's shape");
+    GSI_REQUIRE(B->ctx == ctx && X->ctx == ctx, GSI_ERR_INVALID_ARGUMENT, "chol_solve: buffers of another context");
+    const int64_t k = B->cols;
+    int* flag = f->flags;
+    GSI_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
+    chol_nonfinite_kernel<<<(unsigned)((n * k + 255) / 256), 256, 0, st>>>(B->d, B->ld, n, k, flag);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+    int h = 0;
+    GSI_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    GSI_REQUIRE(h == 0, GSI_ERR_INVALID_ARGUMENT, "chol_solve: B has a non-finite entry");
+    const int64_t kw = k < CH_MAX_CHUNK ? k : CH_MAX_CHUNK;
+    const int64_t kp = round_up(kw, CH_B);
+    DevMem W((size_t)f->np * kp * sizeof(double));
+    for (int64_t c0 = 0; c0 < k; c0 += CH_MAX_CHUNK) {
+        const int64_t w = k - c0 < CH_MAX_CHUNK ? k - c0 : CH_MAX_CHUNK;
+        const int64_t wp = round_up(w, CH_B);
+        GSI_CUDA(cudaMemsetAsync(W.d(), 0, (size_t)f->np * kp * sizeof(double), st));
+        tall_cols_copy(ctx, B->d + c0, B->ld, W.d(), kp, n, w);
+        forward(f, W.d(), kp, wp);
+        if (half == 0) backward(f, W.d(), kp, wp);
+        tall_cols_copy(ctx, W.d(), kp, X->d + c0, X->ld, n, w);
+    }
+    GSI_CUDA(cudaStreamSynchronize(st));
+}
+
+void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const double* Ft, int64_t p, double* var_out) {
+    gsi_ctx* ctx = f->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = f->n, np = f->np;
+    GSI_REQUIRE(cross->type == OP_KERNELCROSS, GSI_ERR_INVALID_ARGUMENT,
+                "chol_krige_variance needs a cross-covariance operator C(T, S) (gsi_op_kernelcov_cross or _cross_grid)");
+    GSI_REQUIRE(cross->ctx == ctx, GSI_ERR_INVALID_ARGUMENT, "chol_krige_variance: the operator belongs to another context");
+    GSI_REQUIRE(cross->n == n, GSI_ERR_DIMENSION_MISMATCH,
+                "chol_krige_variance: the operator's sources must be the factor's n points");
+    GSI_REQUIRE(p >= 0 && p <= CH_MAX_DRIFT, GSI_ERR_INVALID_ARGUMENT, "chol_krige_variance: p must be in 0..32");
+    GSI_REQUIRE(p == 0 || (Fs && Ft), GSI_ERR_INVALID_ARGUMENT, "chol_krige_variance: F_s and F_t are needed when p > 0");
+    const int64_t m = cross->mloc;
+    if (m == 0) return;
+    const int64_t kp0 = round_up(m < CH_MAX_CHUNK ? m : CH_MAX_CHUNK, CH_B);
+    DevMem W((size_t)np * kp0 * sizeof(double));
+    DevMem small((size_t)(CS_PARTS_MAX * CH_MAX_CHUNK + CH_MAX_CHUNK + m + 8) * sizeof(double));
+    double* part = small.d();
+    double* colsq = part + (size_t)CS_PARTS_MAX * CH_MAX_CHUNK;
+    double* var = colsq + CH_MAX_CHUNK;
+    double* ctt = var + m;
+    // the prior variance c(t, t): the generator's value at zero offset (a 1 x 1 block of C(T, T))
+    KcovBlock b0;
+    b0.r0 = 0; b0.rows = 1; b0.c0 = 0; b0.cols = 1; b0.nr_valid = m; b0.nc_valid = m; b0.nugget_diag = 0; b0.lower = 0;
+    b0.out = ctt; b0.rs = 1; b0.cs = 1;
+    kcov_block(cross, KB_TARGETS, b0);
+    // drift: G = L^-1 F_s (row-major np x 128), R'R = G'G (R upper p x p), F_t on the device
+    std::unique_ptr<DevMem> G, Rm, Ftd, H;
+    if (p > 0) {
+        G.reset(new DevMem((size_t)np * CH_B * sizeof(double)));
+        Rm.reset(new DevMem((size_t)(CH_B * CH_B + p * p) * sizeof(double) + 16));
+        Ftd.reset(new DevMem((size_t)m * p * sizeof(double)));
+        H.reset(new DevMem((size_t)CH_B * kp0 * sizeof(double)));
+        // F_s (host column-major n x p) as the row-major np x 128 block G, zero padded
+        std::vector<double> Gh((size_t)np * CH_B, 0.0);
+        for (int64_t q = 0; q < p; ++q)
+            for (int64_t i = 0; i < n; ++i) Gh[(size_t)i * CH_B + q] = Fs[q * n + i];
+        GSI_CUDA(cudaMemcpyAsync(G->d(), Gh.data(), Gh.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        GSI_CUDA(cudaMemcpyAsync(Ftd->d(), Ft, (size_t)m * p * sizeof(double), cudaMemcpyHostToDevice, st));
+        int* flag = f->flags;
+        GSI_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
+        chol_nonfinite_kernel<<<(unsigned)((np * CH_B + 255) / 256), 256, 0, st>>>(G->d(), CH_B, np, CH_B, flag);
+        chol_nonfinite_kernel<<<(unsigned)((m * p + 255) / 256), 256, 0, st>>>(Ftd->d(), p, m, p, flag);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx, 2);
+        forward(f, G->d(), CH_B, CH_B);
+        double* GtG = Rm->d();
+        double* R = GtG + CH_B * CH_B;
+        gemm<false, false, true>(ctx, gm(G->d(), CH_B, G->d(), CH_B, GtG, CH_B, np, 0, 0), 1, 1);
+        tall_head_to_cm_kernel<<<(unsigned)((p * p + 255) / 256), 256, 0, st>>>(GtG, CH_B, (int)p, R);
+        chol_upper_kernel<<<1, 1024, 0, st>>>(R, (int)p, flag + 1);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx, 2);
+        int hf[2] = {0, 0};
+        GSI_CUDA(cudaMemcpyAsync(hf, flag, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+        GSI_CUDA(cudaStreamSynchronize(st));
+        GSI_REQUIRE(hf[0] == 0, GSI_ERR_INVALID_ARGUMENT, "chol_krige_variance: F_s or F_t has a non-finite entry");
+        if (hf[1] != 0)
+            throw Error(GSI_ERR_NOT_POSDEF, "chol_krige_variance: F_s' C^-1 F_s is not positive definite (the drift columns "
+                                            "at the sources are linearly dependent)");
+    }
+    for (int64_t t0 = 0; t0 < m; t0 += CH_MAX_CHUNK) {
+        const int64_t w = m - t0 < CH_MAX_CHUNK ? m - t0 : CH_MAX_CHUNK;
+        const int64_t wp = round_up(w, CH_B);
+        GSI_CUDA(cudaMemsetAsync(W.d(), 0, (size_t)np * kp0 * sizeof(double), st));
+        KcovBlock b;                                               // W = C(S, T_chunk), row-major
+        b.r0 = 0; b.rows = n; b.c0 = t0; b.cols = w; b.nr_valid = n; b.nc_valid = m; b.nugget_diag = 0; b.lower = 0;
+        b.out = W.d(); b.rs = kp0; b.cs = 1;
+        kcov_block(cross, KB_CROSS_T, b);
+        forward(f, W.d(), kp0, wp);                                // W = L^-1 C(S, T_chunk)
+        col_dot(ctx, W.d(), W.d(), kp0, n, w, part, colsq, nullptr);
+        if (p > 0)                                                 // H = G' W
+            gemm<false, false, true>(ctx, gm(G->d(), CH_B, W.d(), kp0, H->d(), kp0, np, 0, 0), 1, wp / CH_B);
+        chol_variance_kernel<<<(unsigned)((w + 127) / 128), 128, 0, st>>>(colsq, ctt, w, (int)p, p > 0 ? H->d() : nullptr, kp0,
+                                                                         p > 0 ? Ftd->d() + t0 : nullptr, m,
+                                                                         p > 0 ? Rm->d() + CH_B * CH_B : nullptr, var + t0);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx);
+    }
+    GSI_CUDA(cudaMemcpyAsync(var_out, var, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+}
+
+}  // namespace gsi

@@ -210,6 +210,17 @@ __global__ void cov_solve_scale_cols_kernel(const double* __restrict__ U, double
 
 static unsigned nblk(int64_t n) { return (unsigned)((n + 255) / 256); }
 
+static_assert(CS_PARTS_MAX == CS_MAX_PARTS, "col_dot scratch size");
+void col_dot(gsi_ctx* ctx, const double* X, const double* Y, int64_t ld, int64_t rows, int64_t cols, double* part,
+             double* out, int* nonfinite) {
+    const ColLaunch L = col_launch(rows, cols);
+    cov_solve_dot_kernel<<<L.grid, L.block, 0, ctx->stream>>>(X, Y, ld, rows, cols, L.chunk, part, nonfinite);
+    GSI_CUDA(cudaGetLastError());
+    cov_solve_reduce_kernel<<<nblk(cols), 256, 0, ctx->stream>>>(part, L.nparts, cols, out);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx, 2);
+}
+
 // a TALL row block [row0, row0 + rows) of `b`, not owned
 static gsi_buf row_view(const gsi_buf* b, int64_t row0, int64_t rows) {
     gsi_buf v = *b;

@@ -911,4 +911,151 @@ void kcov_apply(gsi_op* op, int trans, const gsi_buf* X, gsi_buf* W) {
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Materialised covariance blocks (cov_chol.cu: the dense Cholesky factor and the kriging-variance chunks).
+// out[(i - r0) * rs + (j - c0) * cs] = C[i, j] for rows [r0, r0 + rows) x columns [c0, c0 + cols), from the product
+// kernel's own value code: the same r2 fma chain, kern_eval / model_value, table and signed-table look-ups, and the
+// sigma2 / nugget epilogue (sigma2 * value, then + nugget where i == j).  The product on an identity column adds exact
+// zeros to value * 1, so an entry equals (C I[:, j])[i] bit for bit.  The arithmetic kinds use the same DIM
+// instantiation as the product (d = 1 runs as DIM = 2 on a zero second coordinate).
+// Row points: p.ur / p.latr (pitch p.nr_pad); column points: p.u / p.lat (pitch p.n_pad).  Entries with i >= nr_valid
+// or j >= nc_valid are padding (the factor rounds its order up to a multiple of its block): 1 where i == j, else 0.
+// lower != 0: CTA tiles entirely above the diagonal are skipped (the factor reads the lower triangle only).
+constexpr int KB_ROWS = 64;       // rows of a CTA tile (one per threadIdx.x)
+constexpr int KB_COLS = 64;       // columns of a CTA tile
+constexpr int KB_TY = 4;          // threadIdx.y: column phases
+
+// |lattice offset| table index of row lattice point li and column point c (lattice index k at col[k * stride + c]):
+// the index the product kernel's table_index forms, |dx| + nx * (|dy| + ny * |dz|)
+template <int DIM>
+__device__ __forceinline__ int abs_table_index(const int (&li)[DIM], const int* col, int64_t stride, int64_t c, int nx, int ny) {
+    int idx = 0;
+#pragma unroll
+    for (int k = DIM - 1; k >= 0; --k) {
+        int dk = li[k] - col[k * stride + c];
+        dk = dk < 0 ? -dk : dk;
+        idx = (k == DIM - 1) ? dk : idx * (k == 0 ? nx : ny) + dk;
+    }
+    return idx;
+}
+
+template <int KIND, int DIM>
+__global__ void __launch_bounds__(KB_ROWS * KB_TY) kcov_block_kernel(const __grid_constant__ KcovParams p, int64_t r0,
+                                                                     int64_t rows, int64_t c0, int64_t cols,
+                                                                     int64_t nr_valid, int64_t nc_valid, int nugget_diag,
+                                                                     int lower, double* __restrict__ out, int64_t rs,
+                                                                     int64_t cs) {
+    __shared__ double etab[64 + (KIND == KC_KIND_MODEL ? KB_ROWS * GSI_MODEL_MAX_STRUCTURES * DIM : 0)];
+    const int tx = threadIdx.x, ty = threadIdx.y;
+    const int64_t ti = r0 + (int64_t)blockIdx.x * KB_ROWS, tj = c0 + (int64_t)blockIdx.y * KB_COLS;
+    if (lower && tj > ti + KB_ROWS - 1) return;                  // the whole CTA
+    const int tid = ty * KB_ROWS + tx;
+    if (tid < 64) etab[tid] = kExp2Table[tid];
+    const int64_t i = ti + tx;
+    const int64_t gpt = i < nr_valid ? i : nr_valid - 1;        // padding rows: any valid point (never stored)
+    double ui[DIM];
+    int li[DIM];
+    double* urow = etab + 64 + tx * (GSI_MODEL_MAX_STRUCTURES * DIM);
+    if constexpr (KIND == KC_KIND_MODEL) {
+        if (ty == 0)
+            for (int q = 0; q < p.nstruct * DIM; ++q) {
+                const int s = q / DIM, k = q - s * DIM;
+                urow[q] = p.ur[(s * 3 + k) * p.nr_pad + gpt];
+            }
+    } else {
+#pragma unroll
+        for (int k = 0; k < DIM; ++k) {
+            if (kind_is_table<KIND>()) li[k] = p.latr[k * p.nr_pad + gpt];
+            else ui[k] = p.ur[k * p.nr_pad + gpt];
+        }
+    }
+    __syncthreads();
+    if (i >= r0 + rows) return;
+    for (int q = ty; q < KB_COLS; q += KB_TY) {
+        const int64_t j = tj + q;
+        if (j >= c0 + cols) break;
+        double v;
+        if (i >= nr_valid || j >= nc_valid) {
+            v = i == j ? 1.0 : 0.0;
+        } else {
+            double kv;
+            if constexpr (KIND == KC_KIND_TABLE) {
+                kv = __ldg(p.table + abs_table_index<DIM>(li, p.lat, p.n_pad, j, p.nx, p.ny));
+            } else if constexpr (KIND == KC_KIND_TABLE_SIGNED) {
+                kv = __ldg(p.table + signed_table_index<DIM>(li, p.lat + j, p.n_pad, 0, p.nx, p.ny));
+            } else if constexpr (KIND == KC_KIND_MODEL) {
+                kv = model_value<DIM>(p, urow, p.u + j, p.n_pad, 3 * p.n_pad, etab);
+            } else {
+                double r2 = kind_takes_sqrt<KIND>() ? 1e-300 : 0.0;
+#pragma unroll
+                for (int k = 0; k < DIM; ++k) {
+                    const double dk = ui[k] - p.u[k * p.n_pad + j];
+                    r2 = fma(dk, dk, r2);
+                }
+                kv = kern_eval<KIND>(r2, p.beta, etab);
+            }
+            // the product's epilogue: sigma2 * acc, then + nugget * x (x = 1 on the diagonal) -- two roundings, no fma
+            v = __dmul_rn(p.sigma2, kv);
+            if (nugget_diag && i == j && p.nugget != 0.0) v = __dadd_rn(v, p.nugget);
+        }
+        out[(i - r0) * rs + (j - c0) * cs] = v;
+    }
+}
+
+template <int KIND, int DIM>
+static void launch_block(gsi_ctx* ctx, const KcovParams& p, const KcovBlock& b) {
+    const dim3 grid((unsigned)((b.rows + KB_ROWS - 1) / KB_ROWS), (unsigned)((b.cols + KB_COLS - 1) / KB_COLS));
+    kcov_block_kernel<KIND, DIM><<<grid, dim3(KB_ROWS, KB_TY), 0, ctx->stream>>>(
+        p, b.r0, b.rows, b.c0, b.cols, b.nr_valid, b.nc_valid, b.nugget_diag, b.lower, b.out, b.rs, b.cs);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+}
+
+template <int KIND>
+static void block_dim(gsi_ctx* ctx, const KcovParams& p, const KcovBlock& b, int dim) {
+    if (dim <= 2) launch_block<KIND, 2>(ctx, p, b);
+    else launch_block<KIND, 3>(ctx, p, b);
+}
+
+// rows index the row point set and columns the column point set of `side`:
+//   KB_SQUARE        square operator: both are its n points (the nugget on the diagonal)
+//   KB_CROSS         cross-covariance C(T, S): rows are the targets, columns the sources (the operator's orientation)
+//   KB_CROSS_T       its transpose C(S, T): rows are the sources, columns the targets
+//   KB_TARGETS       C(T, T) without nugget (the prior variance c(t, t) on the diagonal)
+void kcov_block(gsi_op* op, int side, const KcovBlock& b) {
+    gsi_ctx* ctx = op->ctx;
+    if (b.rows <= 0 || b.cols <= 0) return;
+    KcovParams p;
+    std::memset(&p, 0, sizeof(p));
+    p.u = op->ucoords; p.lat = op->lattice; p.table = op->table; p.nx = op->grid_nx; p.ny = op->grid_ny;
+    p.n = op->n; p.n_pad = op->n_pad; p.row0 = 0; p.mloc = op->mloc;
+    p.sigma2 = op->sigma2; p.nugget = op->nugget; p.beta = op->beta;
+    p.nstruct = op->nstruct;
+    for (int s = 0; s < GSI_MODEL_MAX_STRUCTURES; ++s) {
+        p.mkinds[s] = op->mkinds[s]; p.msills[s] = op->msills[s]; p.mbetas[s] = op->mbetas[s];
+    }
+    p.ur = op->ucoords; p.latr = op->lattice; p.nr_pad = op->n_pad; p.nr = op->n;
+    if (side == KB_CROSS) {
+        p.ur = op->ucoords_t; p.latr = op->lattice_t; p.nr_pad = op->nt_pad; p.nr = op->mloc;
+    } else if (side == KB_CROSS_T) {
+        p.u = op->ucoords_t; p.lat = op->lattice_t; p.n_pad = op->nt_pad; p.n = op->mloc;
+    } else if (side == KB_TARGETS) {
+        p.ur = p.u = op->ucoords_t; p.latr = p.lat = op->lattice_t; p.nr_pad = p.n_pad = op->nt_pad; p.nr = p.n = op->mloc;
+        p.nugget = 0.0;
+    }
+    const int kind = op->table ? (op->table_signed ? KC_KIND_TABLE_SIGNED : KC_KIND_TABLE) : op->kind;
+    switch (kind) {
+        case GSI_KERNEL_EXPONENTIAL: block_dim<GSI_KERNEL_EXPONENTIAL>(ctx, p, b, op->dim); break;
+        case GSI_KERNEL_GAUSSIAN: block_dim<GSI_KERNEL_GAUSSIAN>(ctx, p, b, op->dim); break;
+        case GSI_KERNEL_POWERLAW: block_dim<GSI_KERNEL_POWERLAW>(ctx, p, b, op->dim); break;
+        case GSI_KERNEL_MATERN32: block_dim<GSI_KERNEL_MATERN32>(ctx, p, b, op->dim); break;
+        case GSI_KERNEL_MATERN52: block_dim<GSI_KERNEL_MATERN52>(ctx, p, b, op->dim); break;
+        case GSI_KERNEL_SPHERICAL: block_dim<GSI_KERNEL_SPHERICAL>(ctx, p, b, op->dim); break;
+        case KC_KIND_TABLE: block_dim<KC_KIND_TABLE>(ctx, p, b, op->dim); break;
+        case KC_KIND_TABLE_SIGNED: block_dim<KC_KIND_TABLE_SIGNED>(ctx, p, b, op->dim); break;
+        case KC_KIND_MODEL: block_dim<KC_KIND_MODEL>(ctx, p, b, op->dim); break;
+        default: throw Error(GSI_ERR_INVALID_ARGUMENT, "unknown covariance kernel kind");
+    }
+}
+
 }  // namespace gsi

@@ -1,6 +1,7 @@
-"""Kriging on the matrix-free covariance operator: the solve A X = B (gsi_kernelcov_solve, preconditioned CG on the
-device) and simple / ordinary / universal kriging in dual form on top of it.  The n x n covariance matrix is never
-formed: a solve costs one operator product of width k per iteration."""
+"""Kriging on the kernel-covariance operator: the solve A X = B by preconditioned CG on the matrix-free operator
+(gsi_kernelcov_solve; the n x n covariance matrix is never formed, a solve costs one operator product of width k per
+iteration) or on a dense Cholesky factor (KernelCovCholesky, gsi_kernelcov_chol: n^3 / 3 flops once, then any number of
+solves, the kriging variance and log det A), and simple / ordinary / universal kriging in dual form on top of either."""
 import ctypes as C
 import numpy as np
 
@@ -98,23 +99,134 @@ def dual_kriging(solve, cross, y, F, FT):
 
 
 def krige(structures, sources, y, targets, *, nugget=0.0, drift=None, rtol=1e-10, rank=0, rng=None,
-          return_weights=False):
+          return_weights=False, method="cg", return_variance=False):
     """Kriging estimate at the targets (d x m) from observations y at the sources (d x n) under the nested covariance
-    model `structures` (CovStructure list) plus `nugget` on the observations, in dual (matrix-free) form.
+    model `structures` (CovStructure list) plus `nugget` on the observations, in dual form.
 
     drift=None: simple kriging (known zero mean); "constant": ordinary kriging; (F_sources n x p, F_targets m x p):
-    universal kriging / kriging with external drift.  The n x (1 + p) right-hand side is one cov_solve (rank > 0: with
-    a Nystrom preconditioner of that rank).  Returns yhat (m), or (yhat, beta, w) with return_weights=True."""
+    universal kriging / kriging with external drift.  method="cg": the n x (1 + p) right-hand side is one matrix-free
+    cov_solve (rank > 0: with a Nystrom preconditioner of that rank; rtol, rank and rng apply to it).  method="cholesky":
+    one dense factorisation (KernelCovCholesky; about 8 n^2 bytes of device memory) whose solve replaces cov_solve.
+    Returns yhat (m), or (yhat, beta, w) with return_weights=True; return_variance=True appends the kriging variance of
+    the noise-free value at every target (KernelCovCholesky.variance; method="cholesky" only)."""
+    if method not in ("cg", "cholesky"):
+        raise ValueError(f"krige: unknown method {method!r} ('cg' or 'cholesky')")
+    if return_variance and method == "cg":
+        raise ValueError("krige: return_variance needs method='cholesky' -- on the CG path the variance costs one "
+                         "iterative solve per target")
     S, T = _f64_colmajor(sources), _f64_colmajor(targets)
     n, m = S.shape[1], T.shape[1]
     y = np.asarray(y, dtype=np.float64).reshape(n)
     F, FT = drift_matrices(drift, n, m)
     C_ss = KernelCovModelMatrix(structures, S, nugget)
     C_ts = KernelCrossCovMatrix(structures, T, S, ctx=C_ss.ctx)
+    fac = None
+    var = None
     try:
-        yhat, beta, w = dual_kriging(lambda R: cov_solve(C_ss, R, rtol=rtol, rank=rank, rng=rng)[0],
-                                     lambda w: C_ts.apply(w.reshape(n, 1))[:, 0], y, F, FT)
+        cross = lambda w: C_ts.apply(w.reshape(n, 1))[:, 0]          # noqa: E731
+        if method == "cg":
+            yhat, beta, w = dual_kriging(lambda R: cov_solve(C_ss, R, rtol=rtol, rank=rank, rng=rng)[0], cross, y, F, FT)
+        else:
+            fac = KernelCovCholesky(C_ss)
+            yhat, beta, w = dual_kriging(fac.solve, cross, y, F, FT)
+            if return_variance:
+                var = fac.variance(C_ts, (F, FT) if F.shape[1] else None)
     finally:
+        if fac is not None:
+            fac.free()
         C_ss.free()
         C_ts.free()
-    return (yhat, beta, w) if return_weights else yhat
+    out = (yhat, beta, w) if return_weights else (yhat,)
+    if return_variance:
+        out = out + (var,)
+    return out if len(out) > 1 else out[0]
+
+
+class KernelCovCholesky:
+    """Dense Cholesky factor A = L L' of a square kernel-covariance operator A (KernelCovMatrix, GridKernelCovMatrix,
+    KernelCovModelMatrix or GridKernelCovModelMatrix; exactly as built, nugget included), held on the device
+    (gsi_kernelcov_chol; single GPU, about 8 n^2 bytes).  A is materialised by the product kernel's own value code and
+    factored once (n^3 / 3 flops on the FP64 tensor cores); every solve after that is two triangular sweeps.
+
+    A non-positive pivot raises PosDefException with the 1-based failing column in `.column`."""
+
+    def __init__(self, A):
+        op = as_operator(A)
+        self.ctx = op.ctx
+        self._lib = op.ctx._lib
+        self._h = C.c_void_p()
+        col = C.c_int64(0)
+        status = self._lib.gsi_kernelcov_chol(op._h, C.byref(self._h), C.byref(col))
+        try:
+            check(status)
+        except _lib.PosDefException as e:
+            e.column = int(col.value)
+            raise
+        n = C.c_int64()
+        check(self._lib.gsi_chol_size(self._h, C.byref(n)))
+        self.n = int(n.value)
+
+    @property
+    def logdet(self):
+        """log det A = 2 sum log L[i, i] (summed in a fixed order on the device)."""
+        v = C.c_double()
+        check(self._lib.gsi_chol_logdet(self._h, C.byref(v)))
+        return float(v.value)
+
+    @property
+    def L(self):
+        """The factor on the host (n x n lower triangular)."""
+        out = np.empty((self.n, self.n), dtype=np.float64, order="F")
+        check(self._lib.gsi_chol_download(self._h, _pd(out), max(1, self.n)))
+        return out
+
+    def _solve(self, B, half):
+        Bh = np.asarray(B, dtype=np.float64)
+        vector = Bh.ndim == 1
+        Bh = Bh.reshape(-1, 1) if vector else Bh
+        if Bh.ndim != 2 or Bh.shape[0] != self.n:
+            raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH,
+                                         f"KernelCovCholesky: B has shape {Bh.shape}, the factor is {self.n} x {self.n}")
+        k = Bh.shape[1]
+        X = np.empty((self.n, k), dtype=np.float64, order="F")
+        for c0 in range(0, k, 1024):                    # the widest device iterate: 1024 columns per call
+            Bd = DeviceMatrix.from_host(self.ctx, Bh[:, c0:c0 + 1024])
+            try:
+                check(self._lib.gsi_chol_solve(self._h, half, Bd._h, Bd._h))
+                X[:, c0:c0 + 1024] = Bd.numpy()
+            finally:
+                Bd.free()
+        return X[:, 0] if vector else X
+
+    def solve(self, B):
+        """A^-1 B (B: n or n x k, any k)."""
+        return self._solve(B, 0)
+
+    def solve_lower(self, B):
+        """L^-1 B (B: n or n x k, any k)."""
+        return self._solve(B, 1)
+
+    def variance(self, cross_op, drift=None):
+        """Kriging variance of the noise-free value at the m targets of cross_op = C(T, S) (KernelCrossCovMatrix or
+        GridKernelCrossCovMatrix whose sources are this factor's n points, same covariance model): c(t, t) -
+        ||L^-1 c_t||^2 for simple kriging (drift None), plus r' (G'G)^-1 r, G = L^-1 F_s, r = f_t - G' L^-1 c_t, with a
+        drift ("constant" or (F_sources n x p, F_targets m x p), p <= 32)."""
+        m = cross_op.shape[0]
+        Fs, Ft = drift_matrices(drift, self.n, m)
+        p = Fs.shape[1]
+        Fs, Ft = np.asfortranarray(Fs, dtype=np.float64), np.asfortranarray(Ft, dtype=np.float64)
+        var = np.empty(m, dtype=np.float64)
+        check(self._lib.gsi_chol_krige_variance(self._h, cross_op._h, _pd(Fs) if p else None, _pd(Ft) if p else None,
+                                                p, _pd(var)))
+        return var
+
+    def free(self):
+        if getattr(self, "_h", None) and self._h:
+            self._lib.gsi_chol_free(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass

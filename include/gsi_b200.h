@@ -104,7 +104,9 @@ int32_t gsi_ctx_gemm_timing(gsi_ctx* ctx, int32_t enable, double* ms_out, int64_
                             double* flops_out);
 
 /* CUDA-event time per phase while gemm timing is enabled: ms_out8[0] operator products,
- * [1] LU normaliser, [2] QR/TSQR, [3] small SVD, [4] back-multiplication; [5..7] reserved. */
+ * [1] LU normaliser, [2] QR/TSQR, [3] small SVD, [4] back-multiplication; of gsi_kernelcov_chol:
+ * [5] materialising A, [6] diagonal blocks, [7] panel solves, and its trailing updates in [0]
+ * (also counted by gsi_ctx_gemm_timing with their flops).                                  */
 int32_t gsi_ctx_phase_timing(gsi_ctx* ctx, double* ms_out8, int32_t reset);
 
 /* Tuning knobs (no reference counterpart; results do not depend on them beyond rounding-
@@ -299,6 +301,53 @@ int32_t gsi_eig_nystrom(gsi_op* op, const gsi_buf* Q, gsi_buf* U_out, double* Si
  * Omega, or r outside 1..min(256, n - 1): GSI_ERR_INVALID_ARGUMENT.                                                        */
 int32_t gsi_kernelcov_solve(gsi_op* op, const gsi_buf* B, const gsi_buf* Omega, double rtol, int64_t maxiter,
                             gsi_buf* X, int64_t* iters_out, double* relres_out, double* lambda_out);
+/* A materialised block of a kernel-covariance operator (no reference counterpart): out (COLMAJOR rows x cols) receives
+ * C[row0 .. row0 + rows, col0 .. col0 + cols) of a square operator (gsi_op_kernelcov, _grid, _model, _model_grid; global
+ * row indices, the nugget on the diagonal) or of a cross-covariance operator C(T, S) (rows: this rank's targets, columns:
+ * the sources).  Each entry is computed by the product kernel's own value code, so it equals gsi_op_apply on the
+ * identity column bit for bit.  A block outside the operator: GSI_ERR_DIMENSION_MISMATCH; dense or low-rank operators:
+ * GSI_ERR_UNSUPPORTED.                                                                                                     */
+int32_t gsi_op_kernelcov_block(gsi_op* op, int64_t row0, int64_t col0, gsi_buf* out);
+
+/* Direct kriging on a dense Cholesky factor (no reference counterpart).  For the n of most kriging problems (up to a few
+ * tens of thousands of observations) one factorisation, n^3 / 3 flops on the FP64 tensor cores, costs less than one CG
+ * solve of gsi_kernelcov_solve and serves any number of right-hand sides, the kriging variance and the log-determinant.
+ * The factor holds about 8 n^2 bytes of device memory.  A gsi_chol is a live object of its context (gsi_ctx_destroy waits
+ * for it, as for buffers and operators).                                                                                   */
+typedef struct gsi_chol gsi_chol;
+/* Factor the square kernel-covariance operator op exactly as built, nugget included (gsi_op_kernelcov, _grid, _model or
+ * _model_grid: every single kind, nested models, lattice and signed tables): the matrix is materialised on the device by
+ * the product kernel's value code and factored as A = L L' (blocked right-looking Cholesky, block 128).  Results are
+ * bit-reproducible run to run.
+ *   failed_column_out  optional (NULL allowed): 0, or the 1-based column of the first non-positive pivot
+ * Errors: a non-positive (or NaN) pivot: GSI_ERR_NOT_POSDEF, *failed_column_out set, nothing is kept (add a nugget);
+ * dense, low-rank and cross-covariance operators, or a context of several ranks (the factor is single-GPU):
+ * GSI_ERR_UNSUPPORTED; a factor that does not fit the free device memory (cudaMemGetInfo): GSI_ERR_UNSUPPORTED before
+ * any large allocation, the message names the bytes needed.                                                           */
+int32_t gsi_kernelcov_chol(gsi_op* op, gsi_chol** out, int64_t* failed_column_out);
+int32_t gsi_chol_free(gsi_chol* f); /* idempotent on NULL, never throws (Julia finalizer) */
+int32_t gsi_chol_size(const gsi_chol* f, int64_t* n_out);
+/* log det A = 2 sum_i log L[i, i], summed in a fixed order (Gaussian log-likelihood of covariance parameters)          */
+int32_t gsi_chol_logdet(const gsi_chol* f, double* logdet_out);
+/* L to the host: column-major n x n (leading dimension ldh >= n), zeros above the diagonal                            */
+int32_t gsi_chol_download(const gsi_chol* f, double* L_host, int64_t ldh);
+/* half = 0: X = A^-1 B;  half = 1: X = L^-1 B.  B and X: TALL n x k, 1 <= k <= 1024 (the widest TALL buffer; the Python
+ * and Julia layers split wider right-hand sides into 1024-column calls).  X may be B.  A non-finite entry of B or half
+ * outside {0, 1}: GSI_ERR_INVALID_ARGUMENT; bad shapes or layouts: GSI_ERR_DIMENSION_MISMATCH.                        */
+int32_t gsi_chol_solve(gsi_chol* f, int32_t half, const gsi_buf* B, gsi_buf* X);
+/* Kriging variance at the m targets of cross = C(T, S) (gsi_op_kernelcov_cross or _cross_grid, one rank) whose n sources
+ * are the factor's points, under the same covariance model.  It is the variance of the estimation error of the NOISE-FREE
+ * value at t (the nugget enters through A only), so it is about 0 at a source when the nugget is 0 (rounding may leave a
+ * tiny negative value) and c(t, t) far from every source.
+ *   p = 0 (simple kriging):  var(t) = c(t, t) - ||L^-1 c_t||^2,  c(t, t) = sum of the sills, c_t = C(S, t)
+ *   p >= 1 (ordinary / universal kriging, F_s host column-major n x p, F_t m x p, p <= 32): G = L^-1 F_s,
+ *          r_t = f_t - G' L^-1 c_t,  var(t) = var_SK(t) + r_t' (G'G)^-1 r_t
+ * Targets run in chunks of 1024: C(S, T_chunk) is materialised, solved forward and reduced on the device; only the m
+ * variances come to the host (var_out, m doubles).  Errors: a cross operator with another n: GSI_ERR_DIMENSION_MISMATCH;
+ * any other operator, p outside 0..32 or a non-finite drift entry: GSI_ERR_INVALID_ARGUMENT; linearly dependent drift
+ * columns at the sources: GSI_ERR_NOT_POSDEF.                                                                          */
+int32_t gsi_chol_krige_variance(gsi_chol* f, gsi_op* cross, const double* F_s, const double* F_t, int64_t p,
+                                double* var_out);
 
 /* FFTRF.powerlaw_structuredgrid (src/FFTRF.jl:83-100) for a batch of fields, on the device -- the
  * sampler behind getxis(samplefield, numfields, ...) (src/GeostatInversion.jl:29-38).  dim in {2, 3};

@@ -9,7 +9,8 @@
 #   eig_nystrom(A, Q), getxis(Q, numxis, p, q, seed), getxis(samplefield, numfields, numxis, p, q, seed),
 #   getxis(Val{:iwantfields}, ...), pcgalsqr / pcgadirect / pcga / rga with the reference's
 #   positional and keyword arguments,
-# plus covsolve(C, B; rtol, maxiter, rank, seed) and krige(...) on the kernel-covariance operators (new),
+# plus covsolve(C, B; rtol, maxiter, rank, seed), the dense factor covchol(C) with covchol_solve / covchol_logdet /
+# covchol_variance, and krige(...; method = :cg | :cholesky, variance) on the kernel-covariance operators (new),
 # for A::Matrix{Float64}, A::KernelCovMatrix (new), A::KernelCrossCovMatrix (new, not symmetric) and
 # A::LowRankCovMatrix, whose method set is
 # the one the reference's LowRankCovMatrix provides (src/lowrank.jl:38-60,115-139):
@@ -375,27 +376,91 @@ Base.showerror(io::IO, e::CovSolveNoConvergence) = print(io, "CovSolveNoConverge
 
 """
 krige(kinds, sills, ranges, sources, y, targets; rotations, betas, nugget=0.0, drift=nothing, rtol=1e-10, rank=0,
-      seed=nothing) -> (yhat, beta, w)
+      seed=nothing, method=:cg, variance=false) -> (yhat, beta, w) or (yhat, beta, w, var)
 
 Dual-form kriging at the targets (d x m) from observations y at the sources (d x n) under the nested model of
-KernelCovModel plus `nugget`: one covsolve of C [alpha | B_F] = [y | F], beta = (F' B_F) \\ (F' alpha),
+KernelCovModel plus `nugget`: one solve of C [alpha | B_F] = [y | F], beta = (F' B_F) \\ (F' alpha),
 w = alpha - B_F beta, yhat = F_T beta + C(T, S) w (multi-GPU: this worker's block of target rows, as `Cx * w`).  drift = nothing: simple kriging; :constant: ordinary kriging;
-(F_sources n x p, F_targets m x p): universal kriging / kriging with external drift.
+(F_sources n x p, F_targets m x p): universal kriging / kriging with external drift.  method = :cg solves by covsolve
+(rtol, rank, seed apply); method = :cholesky by the dense factor covchol (one GPU, about 8 n^2 bytes), and
+variance = true then appends the kriging variance of the noise-free value at every target (covchol_variance).
 """
 function krige(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, sources::Matrix{Float64},
 		y::Vector{Float64}, targets::Matrix{Float64}; rotations::Union{Nothing, Array{Float64, 3}}=nothing,
 		betas::Union{Nothing, Vector{Float64}}=nothing, nugget=0.0, drift=nothing, rtol::Float64=1e-10, rank::Int=0,
-		seed::Union{Nothing, Int}=nothing)
+		seed::Union{Nothing, Int}=nothing, method::Symbol=:cg, variance::Bool=false)
+	method in (:cg, :cholesky) || throw(ArgumentError("krige: method must be :cg or :cholesky"))
+	variance && method === :cg && throw(ArgumentError("krige: variance = true needs method = :cholesky (on the CG " *
+		"path the variance costs one iterative solve per target)"))
 	n, m = size(sources, 2), size(targets, 2)
 	F, FT = drift === nothing ? (zeros(n, 0), zeros(m, 0)) :
 		drift === :constant ? (ones(n, 1), ones(m, 1)) : (Matrix{Float64}(drift[1]), Matrix{Float64}(drift[2]))
 	C = KernelCovModel(kinds, sills, ranges, sources; rotations=rotations, betas=betas, nugget=nugget)
 	Cx = KernelCrossCov(kinds, sills, ranges, targets, sources; rotations=rotations, betas=betas)
-	X, _ = covsolve(C, hcat(y, F); rtol=rtol, rank=rank, seed=seed, full=true)
+	fct = method === :cholesky ? covchol(C) : nothing
+	X = fct === nothing ? covsolve(C, hcat(y, F); rtol=rtol, rank=rank, seed=seed, full=true)[1] : covchol_solve(fct, hcat(y, F))
 	alpha, BF = X[:, 1], X[:, 2:end]
 	beta = size(F, 2) > 0 ? (F' * BF) \ (F' * alpha) : zeros(0)
 	w = alpha - BF * beta
-	return FT[Cx.rows, :] * beta + Cx * w, beta, w                 # this worker's target rows (all on one GPU)
+	yhat = FT[Cx.rows, :] * beta + Cx * w                          # this worker's target rows (all on one GPU)
+	variance || return yhat, beta, w
+	return yhat, beta, w, covchol_variance(fct, Cx; drift=size(F, 2) > 0 ? (F, FT) : nothing)
+end
+
+"""
+covchol(C) -> CovCholesky
+
+Dense Cholesky factor C = L L' of a square kernel-covariance operator (KernelCovMatrix, KernelCovGrid, KernelCovModel,
+KernelCovModelGrid; nugget included) on the device by gsi_kernelcov_chol: one GPU, about 8 n^2 bytes.  A non-positive
+pivot throws LinearAlgebra.PosDefException(column).  Freed by its finalizer.
+"""
+mutable struct CovCholesky; h::Ptr{Cvoid}; n::Int; ctx::Context; end
+function covchol(C::KernelCovMatrix)
+	out = Ref{Ptr{Cvoid}}(C_NULL)
+	col = Ref{Int64}(0)
+	check(ccall((:gsi_kernelcov_chol, LIB), Int32, (Ptr{Cvoid}, Ptr{Ptr{Cvoid}}, Ptr{Int64}), C.h, out, col))
+	f = CovCholesky(out[], size(C, 2), C.ctx)
+	finalizer(x->ccall((:gsi_chol_free, LIB), Int32, (Ptr{Cvoid},), x.h), f)    # idempotent, never throws
+	return f
+end
+
+"log det C = 2 sum log L[i, i] (Gaussian log-likelihood of covariance parameters)"
+function covchol_logdet(f::CovCholesky)
+	v = Ref{Float64}(0.0)
+	check(ccall((:gsi_chol_logdet, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}), f.h, v))
+	return v[]
+end
+
+"C \\ B (half = false) or L \\ B (half = true), any number of columns (1024 per device call)"
+function covchol_solve(f::CovCholesky, B::VecOrMat{Float64}; half::Bool=false)
+	Bm = Matrix{Float64}(reshape(B, f.n, :))
+	X = similar(Bm)
+	for c0 in 1:1024:size(Bm, 2)
+		cols = c0:min(c0 + 1023, size(Bm, 2))
+		Bd = upload!(DeviceMatrix(f.ctx, GSI_LAYOUT_TALL, f.n, length(cols)), Bm[:, cols])
+		check(ccall((:gsi_chol_solve, LIB), Int32, (Ptr{Cvoid}, Int32, Ptr{Cvoid}, Ptr{Cvoid}), f.h, Int32(half), Bd.h, Bd.h))
+		X[:, cols] = download(Bd)
+	end
+	return B isa Vector ? vec(X) : X
+end
+
+"""
+covchol_variance(f, Cx; drift=nothing) -> var (m)
+
+Kriging variance of the noise-free value at the targets of Cx = KernelCrossCov(..., targets, sources) whose sources are
+the factor's points: c(t, t) - ||L \\ c_t||^2 (drift = nothing), plus r' (G'G) \\ r, G = L \\ F_s, r = f_t - G' (L \\ c_t)
+with drift = :constant or (F_sources n x p, F_targets m x p), p <= 32.
+"""
+function covchol_variance(f::CovCholesky, Cx::KernelCrossCovMatrix; drift=nothing)
+	m = size(Cx, 1)
+	F, FT = drift === nothing ? (zeros(f.n, 0), zeros(m, 0)) :
+		drift === :constant ? (ones(f.n, 1), ones(m, 1)) : (Matrix{Float64}(drift[1]), Matrix{Float64}(drift[2]))
+	p = size(F, 2)
+	var = zeros(m)
+	GC.@preserve F FT var check(ccall((:gsi_chol_krige_variance, LIB), Int32,
+		(Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Float64}),
+		f.h, Cx.h, p > 0 ? pointer(F) : C_NULL, p > 0 ? pointer(FT) : C_NULL, p, var))
+	return var
 end
 
 module RandMatFact

@@ -43,10 +43,14 @@ void col_dot(gsi_ctx* ctx, const double* X, const double* Y, int64_t ld, int64_t
              double* out, int* nonfinite);
 
 // ---- cov_chol.cu: dense Cholesky factor of a square kernel-covariance operator, solves and kriging variance
-gsi_chol* chol_factor(gsi_op* op, int64_t* failed_column);      // *failed_column: 1-based, 0 unless NOT_POSDEF
+// diag: NULL or n host doubles added to the diagonal after the fill; *failed_column: 1-based, 0 unless NOT_POSDEF
+gsi_chol* chol_factor(gsi_op* op, const double* diag, int64_t* failed_column);
 void chol_destroy(gsi_chol* f);
 void chol_download(const gsi_chol* f, double* host, int64_t ldh);
 void chol_solve(const gsi_chol* f, int half, const gsi_buf* B, gsi_buf* X);
 void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const double* Ft, int64_t p, double* var_out);
+// Z = F_t B + L(T, :) V: conditional (ns > 0) or unconditional (ns = 0) realisations from the factor of the joint matrix
+void chol_simulate(const gsi_chol* f, int64_t ns, const double* y, const double* Fs, const double* Ft, int64_t p,
+                   const gsi_buf* Xi, gsi_buf* Z);
 
 }  // namespace gsi

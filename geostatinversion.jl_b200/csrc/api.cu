@@ -1032,7 +1032,19 @@ GSI_API int32_t gsi_kernelcov_chol(gsi_op* op, gsi_chol** out, int64_t* failed_c
         GSI_REQUIRE(op && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
         use(op->ctx);
         *out = nullptr;
-        gsi_chol* f = chol_factor(op, failed_column_out);
+        gsi_chol* f = chol_factor(op, nullptr, failed_column_out);
+        ctx_retain(op->ctx);
+        *out = f;
+    });
+}
+
+GSI_API int32_t gsi_kernelcov_chol_diag(gsi_op* op, const double* diag, gsi_chol** out, int64_t* failed_column_out) {
+    if (failed_column_out) *failed_column_out = 0;
+    return guarded([&] {
+        GSI_REQUIRE(op && out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(op->ctx);
+        *out = nullptr;
+        gsi_chol* f = chol_factor(op, diag, failed_column_out);
         ctx_retain(op->ctx);
         *out = f;
     });
@@ -1083,5 +1095,14 @@ GSI_API int32_t gsi_chol_krige_variance(gsi_chol* f, gsi_op* cross, const double
         GSI_REQUIRE(f && cross && var_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
         use(f->ctx);
         chol_variance(f, cross, F_s, F_t, p, var_out);
+    });
+}
+
+GSI_API int32_t gsi_chol_simulate(gsi_chol* f, int64_t ns, const double* y, const double* F_s, const double* F_t,
+                                  int64_t p, const gsi_buf* Xi, gsi_buf* Z) {
+    return guarded([&] {
+        GSI_REQUIRE(f && Xi && Z, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(f->ctx);
+        chol_simulate(f, ns, y, F_s, F_t, p, Xi, Z);
     });
 }

@@ -20,6 +20,20 @@
 // template parameters, so the same kernel serves the solves: forward B_j = X_jj B_j, B_(>j) -= L_(>j, j) B_j; backward
 // B_j = X_jj' B_j, B_(<j) -= L_(j, <j)' B_j, on a row-major work block of width 128 .. 1024.
 // Every reduction has a fixed order (no atomics): factor, solve, log-determinant and variance are bit-reproducible.
+//
+// Conditional Gaussian simulation (chol_simulate; LU simulation).  The N points are ordered sources first,
+// P = [S (ns points); T (m = N - ns)], and the factor is that of the joint matrix A = C(P, P) + diag(d), d_i = the nugget
+// for i < ns (observation noise) and tau for the targets (tau = 0: the noise-free field of krige / variance; a small
+// tau > 0 is jitter for smooth kernels and close targets).  Its leading ns x ns block L_SS is the factor of
+// C(S, S) + nugget I, and A_TS = L_TS L_SS'.  For k realisations from host standard normals Xi = [Xi_S; Xi_T] (N x k) and
+// a drift F_s (ns x p), F_t (m x p), 0 <= p <= 32:
+//   g = L_SS^-1 y,  G = L_SS^-1 F_s,  B = (G'G)^-1 G' (g 1' - Xi_S)   (p x k)
+//   V = [g 1' - G B; Xi_T]   (N x k),   Z = F_t B + L(T, :) V   (m x k)
+// This is "unconditional sample plus kriging of its residual" arranged so that a batch needs one triangular product and
+// no triangular solve.  Xi = 0 gives the dual-form estimate (beta = (G'G)^-1 G'g, yhat = F_t beta + L_TS (g - G beta));
+// Cov(Z) = L_TT L_TT' + (F_t - L_TS G)(G'G)^-1(F_t - L_TS G)', whose diagonal is the kriging variance + tau; p = 0 gives
+// Z = L_TS g + L_TT Xi_T, independent of Xi_S; ns = 0 gives Z = L Xi.  The product Z = L(T, :) V is chol_trmm_kernel;
+// g and G come from a forward sweep that stops after the source blocks, G'G and G' Xi_S from chol_gemm_kernel.
 #include "common.cuh"
 #include "algos.h"
 #include "ptx.cuh"
@@ -264,6 +278,142 @@ __global__ void chol_variance_kernel(const double* __restrict__ colsq, const dou
     var[c] = v;
 }
 
+// A(i, i) += d[i] after the fill, rounded once as the fill adds the nugget (a constant d on an operator without nugget
+// gives the bits of that nugget inside the operator)
+__global__ void chol_add_diag_kernel(double* __restrict__ A, int64_t lda, const double* __restrict__ d, int64_t n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) A[i * lda + i] = __dadd_rn(A[i * lda + i], d[i]);
+}
+
+// Z = L(rows, :) V for the lower-triangular factor: L column-major (pitch np), V row-major np x kp (pitch kp), Z row-major
+// (pitch kp) holding rows r0 .. np.  One CTA per 128 x 128 tile (row tile i >= r0 / 128, column tile c) reduces over the
+// k-blocks j = 0 .. i in order; tiles are issued heaviest first (i descending), so the ragged K leaves no long tail.  The
+// strict upper triangle of L's storage is not zero (the fill skips whole tiles only, the diagonal blocks are written on
+// and below the diagonal), so the diagonal block j = i is masked to its lower triangle in shared memory.
+struct ChTrmm {
+    const double* L; int64_t np;
+    const double* V; int64_t kp;
+    double* Z; int64_t r0;
+    int64_t nct;   // column tiles: kp / 128
+};
+
+__global__ void __launch_bounds__(CH_THREADS, 1) chol_trmm_kernel(const ChTrmm a) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    double* sm = reinterpret_cast<double*>(smem_raw);
+    const int64_t t0 = blockIdx.x / a.nct;
+    const int64_t ti = a.np / CH_B - 1 - t0, tj = blockIdx.x - t0 * a.nct;
+    const int64_t m0 = ti * CH_B, n0 = tj * CH_B;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int g = lane >> 2, t = lane & 3;
+    const int wm = warp & 3, wn = warp >> 2;
+    double acc[4][4][2];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
+    const int kdiag = (int)(ti * (CH_B / CH_K));                 // first k-tile of the diagonal block
+    const int nk = kdiag + CH_B / CH_K;
+    auto load = [&](int st, int kt) {
+        double* sa = sm + (size_t)st * 2 * CH_TILE;
+        ch_load_tile<false>(sa, a.L, a.np, m0, (int64_t)kt * CH_K, tid);
+        ch_load_tile<false>(sa + CH_TILE, a.V, a.kp, n0, (int64_t)kt * CH_K, tid);
+        cp_async_commit();
+    };
+    load(0, 0);
+    for (int kt = 0; kt < nk; ++kt) {
+        if (kt + 1 < nk) {
+            load((kt + 1) & 1, kt + 1);
+            cp_async_wait<1>();
+        } else {
+            cp_async_wait<0>();
+        }
+        __syncthreads();
+        double* sa = sm + (size_t)(kt & 1) * 2 * CH_TILE;
+        if (kt >= kdiag) {                                        // L(m0 + r, m0 + kb + k) = 0 where kb + k > r
+            const int kb = (kt - kdiag) * CH_K;
+            for (int e = tid; e < CH_K * CH_B; e += CH_THREADS) {
+                const int k = e >> 7, r = e & (CH_B - 1);
+                if (kb + k > r) sa[k * CH_P + r] = 0.0;
+            }
+            __syncthreads();
+        }
+        const double* sb = sa + CH_TILE;                           // chol_gemm_kernel's k-tile step
+#pragma unroll
+        for (int ks = 0; ks < CH_K / 4; ++ks) {
+            const double* ar = sa + (ks * 4 + t) * CH_P + wm * 32 + g;
+            const double* br = sb + (ks * 4 + t) * CH_P + wn * 32 + g;
+            double af[4], bf[4];
+#pragma unroll
+            for (int f = 0; f < 4; ++f) { af[f] = ar[f * 8]; bf[f] = br[f * 8]; }
+#pragma unroll
+            for (int fm = 0; fm < 4; ++fm)
+#pragma unroll
+                for (int fn = 0; fn < 4; ++fn) dmma884(acc[fm][fn][0], acc[fm][fn][1], af[fm], bf[fn]);
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int fm = 0; fm < 4; ++fm) {
+        const int64_t m = m0 + wm * 32 + fm * 8 + g - a.r0;
+#pragma unroll
+        for (int fn = 0; fn < 4; ++fn) {
+            const int64_t n = n0 + wn * 32 + fn * 8 + 2 * t;
+            *reinterpret_cast<double2*>(a.Z + m * a.kp + n) = make_double2(acc[fm][fn][0], acc[fm][fn][1]);
+        }
+    }
+}
+
+// The drift terms of conditional simulation for a 32-column strip of the k realisations.  W: row-major (pitch 128) with
+// G = L_SS^-1 F_s in columns 0 .. p - 1 and g = L_SS^-1 y in column p; GtG = W'W (row-major, pitch 128; G'g in its
+// column p); H: G' Xi_S (row-major p x kp); R: upper p x p with R'R = G'G (column-major, pitch p).
+//   B(:, c) = R^-1 R^-T (G'g - H(:, c))   (p x kp row-major in Bm, written by the CTAs of the first row strip)
+//   V(i, c) = g_i - sum_q G(i, q) B(q, c) for the source rows i < ns  (p = 0: V(i, c) = g_i)
+constexpr int SIM_ROWS = 64;   // source rows per CTA
+__global__ void __launch_bounds__(256) chol_sim_drift_kernel(const double* __restrict__ W, const double* __restrict__ GtG,
+                                                             const double* __restrict__ H, const double* __restrict__ R,
+                                                             int p, int64_t ns, double* __restrict__ Bm,
+                                                             double* __restrict__ V, int64_t kp) {
+    __shared__ double sB[CH_MAX_DRIFT][32];
+    const int tx = threadIdx.x, ty = threadIdx.y;
+    const int64_t c = (int64_t)blockIdx.x * 32 + tx;
+    if (p > 0 && ty == 0) {
+        for (int i = 0; i < p; ++i) {                             // R' z = G'g - G' xi_c
+            double s = GtG[i * CH_B + p] - H[i * kp + c];
+            for (int k = 0; k < i; ++k) s -= R[k + i * p] * sB[k][tx];
+            sB[i][tx] = s / R[i + i * p];
+        }
+        for (int i = p - 1; i >= 0; --i) {                        // R b = z
+            double s = sB[i][tx];
+            for (int k = i + 1; k < p; ++k) s -= R[i + k * p] * sB[k][tx];
+            sB[i][tx] = s / R[i + i * p];
+        }
+        if (blockIdx.y == 0)
+            for (int i = 0; i < p; ++i) Bm[i * kp + c] = sB[i][tx];
+    }
+    __syncthreads();
+    const int64_t r1 = min(ns, (int64_t)(blockIdx.y + 1) * SIM_ROWS);
+    for (int64_t i = (int64_t)blockIdx.y * SIM_ROWS + ty; i < r1; i += 8) {
+        const double* wi = W + i * CH_B;
+        double v = wi[p];
+        for (int q = 0; q < p; ++q) v -= wi[q] * sB[q][tx];
+        V[i * kp + c] = v;
+    }
+}
+
+// Z (TALL m x k, pitch ldz) = the TRMM rows off .. off + m of Zw (pitch kp) + F_t B (F_t column-major m x p; B row-major
+// p x kp); p = 0 copies
+__global__ void chol_sim_out_kernel(const double* __restrict__ Zw, int64_t kp, int64_t off, const double* __restrict__ Ft,
+                                    int64_t m, int p, const double* __restrict__ Bm, double* __restrict__ Z, int64_t ldz,
+                                    int64_t k) {
+    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= m * k) return;
+    const int64_t r = idx / k, c = idx - r * k;
+    double fb = 0.0;
+    for (int q = 0; q < p; ++q) fb += Ft[r + q * m] * Bm[q * kp + c];
+    const double z = Zw[(off + r) * kp + c];
+    Z[r * ldz + c] = p > 0 ? fb + z : z;
+}
+
 namespace {
 
 template <bool AK, bool BK, bool CR>
@@ -283,10 +433,11 @@ ChGemm gm(const double* A, int64_t lda, const double* B, int64_t ldb, double* C,
     return a;
 }
 
-// W (row-major np x kp, pitch ldw; kp a multiple of 128) <- L^-1 W
-void forward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp) {
+// W (row-major np x kp, pitch ldw; kp a multiple of 128) <- L^-1 W on the leading nb block rows (nb = np / 128: all of
+// W; a smaller nb leaves the rows from nb * 128 on unchanged, and the rows above are those of the full solve)
+void forward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp, int64_t nb) {
     gsi_ctx* ctx = f->ctx;
-    const int64_t nb = f->np / CH_B, nt = kp / CH_B;
+    const int64_t nt = kp / CH_B;
     for (int64_t kb = 0; kb < nb; ++kb) {
         const int64_t j0 = kb * CH_B;
         double* Wj = W + j0 * ldw;
@@ -326,7 +477,7 @@ void chol_destroy(gsi_chol* f) {
     delete f;
 }
 
-gsi_chol* chol_factor(gsi_op* op, int64_t* failed_column) {
+gsi_chol* chol_factor(gsi_op* op, const double* diag, int64_t* failed_column) {
     gsi_ctx* ctx = op->ctx;
     cudaStream_t st = ctx->stream;
     if (failed_column) *failed_column = 0;
@@ -334,7 +485,10 @@ gsi_chol* chol_factor(gsi_op* op, int64_t* failed_column) {
                 "kernelcov_chol needs a square kernel-covariance operator (gsi_op_kernelcov, _grid, _model or _model_grid)");
     GSI_REQUIRE(ctx->world == 1, GSI_ERR_UNSUPPORTED, "kernelcov_chol is single-GPU: the dense factor is not distributed");
     const int64_t n = op->n, np = round_up(n, CH_B);
-    const double need = (double)np * (double)np * 8.0 + (double)np * CH_B * 8.0 + 4096.0;
+    if (diag)
+        for (int64_t i = 0; i < n; ++i)
+            GSI_REQUIRE(std::isfinite(diag[i]), GSI_ERR_INVALID_ARGUMENT, "kernelcov_chol_diag: diag has a non-finite entry");
+    const double need = (double)np * (double)np * 8.0 + (double)np * CH_B * 8.0 + 4096.0 + (diag ? (double)n * 8.0 : 0.0);
     size_t fr = 0, tot = 0;
     GSI_CUDA(cudaMemGetInfo(&fr, &tot));
     if (need > (double)fr) {
@@ -362,6 +516,14 @@ gsi_chol* chol_factor(gsi_op* op, int64_t* failed_column) {
     b.r0 = 0; b.rows = np; b.c0 = 0; b.cols = np; b.nr_valid = n; b.nc_valid = n; b.nugget_diag = 1; b.lower = 1;
     b.out = f->L; b.rs = 1; b.cs = np;
     kcov_block(op, KB_SQUARE, b);
+    if (diag) {                                                   // + diag(d), one rounding per entry as the nugget's
+        DevMem dd((size_t)n * sizeof(double));
+        GSI_CUDA(cudaMemcpyAsync(dd.d(), diag, (size_t)n * sizeof(double), cudaMemcpyHostToDevice, st));
+        chol_add_diag_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(f->L, np, dd.d(), n);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx);
+        GSI_CUDA(cudaStreamSynchronize(st));                      // dd is freed on return
+    }
     phase_end(ctx, PH_CHOL_FILL);
     // 2. blocked right-looking factorisation
     GSI_CUDA(cudaFuncSetAttribute(chol_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CH_DIAG_SMEM));
@@ -439,7 +601,7 @@ void chol_solve(const gsi_chol* f, int half, const gsi_buf* B, gsi_buf* X) {
         const int64_t wp = round_up(w, CH_B);
         GSI_CUDA(cudaMemsetAsync(W.d(), 0, (size_t)f->np * kp * sizeof(double), st));
         tall_cols_copy(ctx, B->d + c0, B->ld, W.d(), kp, n, w);
-        forward(f, W.d(), kp, wp);
+        forward(f, W.d(), kp, wp, f->np / CH_B);
         if (half == 0) backward(f, W.d(), kp, wp);
         tall_cols_copy(ctx, W.d(), kp, X->d + c0, X->ld, n, w);
     }
@@ -490,7 +652,7 @@ void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const dou
         chol_nonfinite_kernel<<<(unsigned)((m * p + 255) / 256), 256, 0, st>>>(Ftd->d(), p, m, p, flag);
         GSI_CUDA(cudaGetLastError());
         count_launch(ctx, 2);
-        forward(f, G->d(), CH_B, CH_B);
+        forward(f, G->d(), CH_B, CH_B, np / CH_B);
         double* GtG = Rm->d();
         double* R = GtG + CH_B * CH_B;
         gemm<false, false, true>(ctx, gm(G->d(), CH_B, G->d(), CH_B, GtG, CH_B, np, 0, 0), 1, 1);
@@ -514,7 +676,7 @@ void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const dou
         b.r0 = 0; b.rows = n; b.c0 = t0; b.cols = w; b.nr_valid = n; b.nc_valid = m; b.nugget_diag = 0; b.lower = 0;
         b.out = W.d(); b.rs = kp0; b.cs = 1;
         kcov_block(cross, KB_CROSS_T, b);
-        forward(f, W.d(), kp0, wp);                                // W = L^-1 C(S, T_chunk)
+        forward(f, W.d(), kp0, wp, np / CH_B);                     // W = L^-1 C(S, T_chunk)
         col_dot(ctx, W.d(), W.d(), kp0, n, w, part, colsq, nullptr);
         if (p > 0)                                                 // H = G' W
             gemm<false, false, true>(ctx, gm(G->d(), CH_B, W.d(), kp0, H->d(), kp0, np, 0, 0), 1, wp / CH_B);
@@ -525,6 +687,103 @@ void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const dou
         count_launch(ctx);
     }
     GSI_CUDA(cudaMemcpyAsync(var_out, var, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+}
+
+void chol_simulate(const gsi_chol* f, int64_t ns, const double* y, const double* Fs, const double* Ft, int64_t p,
+                   const gsi_buf* Xi, gsi_buf* Z) {
+    gsi_ctx* ctx = f->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = f->n, np = f->np, m = n - ns;
+    GSI_REQUIRE(ns >= 0 && ns < n, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: ns must be in 0 .. n - 1");
+    GSI_REQUIRE(p >= 0 && p <= CH_MAX_DRIFT, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: p must be in 0..32");
+    GSI_REQUIRE(p == 0 || ns > 0, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: a drift needs conditioning data (ns > 0)");
+    GSI_REQUIRE(ns == 0 || y, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: y is needed when ns > 0");
+    GSI_REQUIRE(p == 0 || (Fs && Ft), GSI_ERR_INVALID_ARGUMENT, "chol_simulate: F_s and F_t are needed when p > 0");
+    GSI_REQUIRE(Xi->layout == GSI_LAYOUT_TALL && Xi->rows == n && Xi->cols >= 1 && Xi->cols <= CH_MAX_CHUNK,
+                GSI_ERR_DIMENSION_MISMATCH, "chol_simulate: Xi must be TALL n x k, 1 <= k <= 1024");
+    GSI_REQUIRE(Z->layout == GSI_LAYOUT_TALL && Z->rows == m && Z->cols == Xi->cols, GSI_ERR_DIMENSION_MISMATCH,
+                "chol_simulate: Z must be TALL (n - ns) x k");
+    GSI_REQUIRE(Xi->ctx == ctx && Z->ctx == ctx, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: buffers of another context");
+    bool finite = true;
+    for (int64_t i = 0; i < ns; ++i) finite = finite && std::isfinite(y[i]);
+    for (int64_t i = 0; i < ns * p; ++i) finite = finite && std::isfinite(Fs[i]);
+    for (int64_t i = 0; i < m * p; ++i) finite = finite && std::isfinite(Ft[i]);
+    GSI_REQUIRE(finite, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: y, F_s or F_t has a non-finite entry");
+    const int64_t k = Xi->cols, kp = round_up(k, CH_B);
+    int* flag = f->flags;
+    GSI_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
+    chol_nonfinite_kernel<<<(unsigned)((n * k + 255) / 256), 256, 0, st>>>(Xi->d, Xi->ld, n, k, flag);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+    // V = [g 1' - G B; Xi_T] (row-major np x kp, zero padded), the TRMM rows from the tile that holds row ns
+    const int64_t r0 = ns / CH_B * CH_B;
+    DevMem V((size_t)np * kp * sizeof(double));
+    DevMem Zw((size_t)(np - r0) * kp * sizeof(double));
+    GSI_CUDA(cudaMemsetAsync(V.d(), 0, (size_t)np * kp * sizeof(double), st));
+    tall_cols_copy(ctx, Xi->d, Xi->ld, V.d(), kp, n, k);
+    std::unique_ptr<DevMem> W, small;
+    double *GtG = nullptr, *R = nullptr, *H = nullptr, *Bm = nullptr, *Ftd = nullptr;
+    if (ns > 0) {
+        // [G | g] = L_SS^-1 [F_s | y]: rows below ns of L^-1 [F_s y; 0] are L_SS^-1 [F_s y], so the sweep stops after
+        // the block rows that hold sources; the rows from ns on are zeroed for the reductions over the sources
+        const int64_t nbs = (ns + CH_B - 1) / CH_B;
+        W.reset(new DevMem((size_t)np * CH_B * sizeof(double)));
+        small.reset(new DevMem((size_t)(CH_B * CH_B + CH_MAX_DRIFT * CH_MAX_DRIFT + (CH_B + CH_MAX_DRIFT) * kp + m * p) *
+                               sizeof(double)));
+        GtG = small->d(); R = GtG + CH_B * CH_B; H = R + CH_MAX_DRIFT * CH_MAX_DRIFT; Bm = H + CH_B * kp;
+        Ftd = Bm + CH_MAX_DRIFT * kp;
+        std::vector<double> Wh((size_t)np * CH_B, 0.0);
+        for (int64_t i = 0; i < ns; ++i) {
+            for (int64_t q = 0; q < p; ++q) Wh[(size_t)i * CH_B + q] = Fs[q * ns + i];
+            Wh[(size_t)i * CH_B + p] = y[i];
+        }
+        GSI_CUDA(cudaMemcpyAsync(W->d(), Wh.data(), Wh.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (p > 0)
+            GSI_CUDA(cudaMemcpyAsync(Ftd, Ft, (size_t)m * p * sizeof(double), cudaMemcpyHostToDevice, st));
+        forward(f, W->d(), CH_B, CH_B, nbs);
+        GSI_CUDA(cudaMemsetAsync(W->d() + ns * CH_B, 0, (size_t)(np - ns) * CH_B * sizeof(double), st));
+        if (p > 0) {
+            gemm<false, false, true>(ctx, gm(W->d(), CH_B, W->d(), CH_B, GtG, CH_B, nbs * CH_B, 0, 0), 1, 1);   // W'W
+            gemm<false, false, true>(ctx, gm(W->d(), CH_B, V.d(), kp, H, kp, nbs * CH_B, 0, 0), 1, kp / CH_B); // W'Xi
+            tall_head_to_cm_kernel<<<(unsigned)((p * p + 255) / 256), 256, 0, st>>>(GtG, CH_B, (int)p, R);
+            chol_upper_kernel<<<1, 1024, 0, st>>>(R, (int)p, flag + 1);
+            GSI_CUDA(cudaGetLastError());
+            count_launch(ctx, 2);
+        }
+    }
+    int hf[2] = {0, 0};
+    GSI_CUDA(cudaMemcpyAsync(hf, flag, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    GSI_REQUIRE(hf[0] == 0, GSI_ERR_INVALID_ARGUMENT, "chol_simulate: Xi has a non-finite entry");
+    if (hf[1] != 0)
+        throw Error(GSI_ERR_NOT_POSDEF, "chol_simulate: F_s' C^-1 F_s is not positive definite (the drift columns at the "
+                                        "sources are linearly dependent)");
+    if (ns > 0) {
+        chol_sim_drift_kernel<<<dim3((unsigned)(kp / 32), (unsigned)((ns + SIM_ROWS - 1) / SIM_ROWS)), dim3(32, 8), 0, st>>>(
+            W->d(), GtG, H, R, (int)p, ns, Bm, V.d(), kp);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx);
+    }
+    // Zw = L(r0 .., :) V: the n^2 k flops
+    const int64_t nrt = (np - r0) / CH_B, nct = kp / CH_B;
+    ChTrmm a;
+    a.L = f->L; a.np = np; a.V = V.d(); a.kp = kp; a.Z = Zw.d(); a.r0 = r0; a.nct = nct;
+    GSI_CUDA(cudaFuncSetAttribute(chol_trmm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CH_GEMM_SMEM));
+    phase_begin(ctx);
+    chol_trmm_kernel<<<(unsigned)(nrt * nct), CH_THREADS, CH_GEMM_SMEM, st>>>(a);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+    phase_end(ctx, PH_GEMM);
+    if (ctx->time_gemm) {
+        const int64_t nb = np / CH_B, i0 = r0 / CH_B;
+        ctx->gemm_launches += 1;
+        ctx->gemm_flops_accum += 2.0 * CH_B * CH_B * CH_B * (double)nct * (double)((nb * (nb + 1) - i0 * (i0 + 1)) / 2);
+    }
+    chol_sim_out_kernel<<<(unsigned)((m * k + 255) / 256), 256, 0, st>>>(Zw.d(), kp, ns - r0, Ftd, m, (int)p, Bm, Z->d,
+                                                                         Z->ld, k);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
     GSI_CUDA(cudaStreamSynchronize(st));
 }
 

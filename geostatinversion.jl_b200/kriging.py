@@ -1,7 +1,9 @@
 """Kriging on the kernel-covariance operator: the solve A X = B by preconditioned CG on the matrix-free operator
 (gsi_kernelcov_solve; the n x n covariance matrix is never formed, a solve costs one operator product of width k per
 iteration) or on a dense Cholesky factor (KernelCovCholesky, gsi_kernelcov_chol: n^3 / 3 flops once, then any number of
-solves, the kriging variance and log det A), and simple / ordinary / universal kriging in dual form on top of either."""
+solves, the kriging variance and log det A), and simple / ordinary / universal kriging in dual form on top of either;
+conditional and unconditional Gaussian simulation on the dense factor of the joint source-target covariance
+(simulate, gsi_chol_simulate)."""
 import ctypes as C
 import numpy as np
 
@@ -142,21 +144,73 @@ def krige(structures, sources, y, targets, *, nugget=0.0, drift=None, rtol=1e-10
     return out if len(out) > 1 else out[0]
 
 
+def simulate(structures, targets, nreal, *, sources=None, y=None, nugget=0.0, target_nugget=0.0, drift=None, rng=None,
+             Xi=None):
+    """nreal Gaussian realisations (m x nreal) at the targets (d x m) under the nested covariance model `structures`,
+    conditioned on observations y at the sources (d x ns, observation noise `nugget`) or unconditional (sources=None).
+
+    LU simulation on one dense factor of the joint matrix C([S T], [S T]) + diag(nugget at the sources, target_nugget at
+    the targets) (KernelCovCholesky.simulate; about 8 (ns + m)^2 bytes of device memory).  target_nugget = 0 simulates
+    the noise-free field that krige estimates; a small target_nugget > 0 is the jitter smooth kernels need when targets
+    lie close together.  drift: None (simple kriging, known zero mean), "constant" or (F_sources ns x p, F_targets m x p)
+    as in krige; conditional simulation only.  The standard normals are drawn on the host from `rng`, 1024 columns at a
+    time; pass Xi ((ns + m) x nreal) to make a run exact."""
+    T = _f64_colmajor(targets)
+    m = T.shape[1]
+    if sources is None:
+        if drift is not None:
+            raise ValueError("simulate: a drift needs conditioning data (sources and y)")
+        S = np.zeros((T.shape[0], 0))
+    else:
+        S = _f64_colmajor(sources)
+    ns = S.shape[1]
+    nreal = int(nreal)
+    if Xi is None:
+        g = _rng(rng)
+        Xi = np.empty((ns + m, nreal), dtype=np.float64, order="F")
+        for c0 in range(0, nreal, 1024):
+            Xi[:, c0:c0 + 1024] = g.standard_normal((ns + m, min(1024, nreal - c0)))
+    elif np.shape(Xi) != (ns + m, nreal):
+        raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH,
+                                     f"simulate: Xi has shape {np.shape(Xi)}, expected {(ns + m, nreal)}")
+    P = np.concatenate([S, T], axis=1)
+    d = np.concatenate([np.full(ns, float(nugget)), np.full(m, float(target_nugget))])
+    A = KernelCovModelMatrix(structures, P, 0.0)
+    fac = None
+    try:
+        fac = KernelCovCholesky(A, diag=d)
+        return fac.simulate(Xi, n_cond=ns, y=None if ns == 0 else y, drift=drift)
+    finally:
+        if fac is not None:
+            fac.free()
+        A.free()
+
+
 class KernelCovCholesky:
     """Dense Cholesky factor A = L L' of a square kernel-covariance operator A (KernelCovMatrix, GridKernelCovMatrix,
     KernelCovModelMatrix or GridKernelCovModelMatrix; exactly as built, nugget included), held on the device
     (gsi_kernelcov_chol; single GPU, about 8 n^2 bytes).  A is materialised by the product kernel's own value code and
     factored once (n^3 / 3 flops on the FP64 tensor cores); every solve after that is two triangular sweeps.
 
+    diag (n values, optional) is added to A's diagonal before the factorisation (gsi_kernelcov_chol_diag): per-point
+    nuggets, such as heteroscedastic observation noise or the joint source / target matrix of `simulate`.
+
     A non-positive pivot raises PosDefException with the 1-based failing column in `.column`."""
 
-    def __init__(self, A):
+    def __init__(self, A, diag=None):
         op = as_operator(A)
         self.ctx = op.ctx
         self._lib = op.ctx._lib
         self._h = C.c_void_p()
         col = C.c_int64(0)
-        status = self._lib.gsi_kernelcov_chol(op._h, C.byref(self._h), C.byref(col))
+        if diag is None:
+            status = self._lib.gsi_kernelcov_chol(op._h, C.byref(self._h), C.byref(col))
+        else:
+            d = np.ascontiguousarray(diag, dtype=np.float64).reshape(-1)
+            if d.size != op.shape[1]:
+                raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH,
+                                             f"KernelCovCholesky: diag has {d.size} values, A is {op.shape[1]} x {op.shape[1]}")
+            status = self._lib.gsi_kernelcov_chol_diag(op._h, _pd(d), C.byref(self._h), C.byref(col))
         try:
             check(status)
         except _lib.PosDefException as e:
@@ -219,6 +273,44 @@ class KernelCovCholesky:
         check(self._lib.gsi_chol_krige_variance(self._h, cross_op._h, _pd(Fs) if p else None, _pd(Ft) if p else None,
                                                 p, _pd(var)))
         return var
+
+    def simulate(self, Xi, *, n_cond=0, y=None, drift=None):
+        """Realisations at the last n - n_cond points of a factor of the joint matrix [sources; targets] (gsi_chol_simulate):
+        Z = F_t B + L(T, :) V from the standard normals Xi (n x k, any k; 1024 columns per device call), conditioned on
+        y (n_cond values) at the first n_cond points with drift None (simple kriging: known zero mean), "constant" or
+        (F_sources n_cond x p, F_targets (n - n_cond) x p), p <= 32.  Xi = 0 gives the kriging estimate; n_cond = 0 gives
+        unconditional samples L Xi.  Returns (n - n_cond) x k."""
+        ns = int(n_cond)
+        m = self.n - ns
+        Xh = np.asarray(Xi, dtype=np.float64)
+        Xh = Xh.reshape(-1, 1) if Xh.ndim == 1 else Xh
+        if Xh.ndim != 2 or Xh.shape[0] != self.n:
+            raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH,
+                                         f"KernelCovCholesky.simulate: Xi has shape {Xh.shape}, the factor is {self.n} x {self.n}")
+        if drift is not None and ns == 0:
+            raise ValueError("simulate: a drift needs conditioning data (n_cond > 0)")
+        Fs, Ft = drift_matrices(drift, ns, m)
+        p = Fs.shape[1]
+        yh = np.ascontiguousarray(np.zeros(0) if y is None else y, dtype=np.float64).reshape(-1)
+        if yh.size != ns:
+            raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH,
+                                         f"KernelCovCholesky.simulate: y has {yh.size} values, n_cond is {ns}")
+        Fs, Ft = np.asfortranarray(Fs, dtype=np.float64), np.asfortranarray(Ft, dtype=np.float64)
+        k = Xh.shape[1]
+        Z = np.empty((m, k), dtype=np.float64, order="F")
+        for c0 in range(0, k, 1024):                    # the widest device iterate: 1024 columns per call
+            Xd = DeviceMatrix.from_host(self.ctx, Xh[:, c0:c0 + 1024])
+            Zd = None
+            try:
+                Zd = DeviceMatrix(self.ctx, m, Xd.shape[1], LAYOUT_TALL)
+                check(self._lib.gsi_chol_simulate(self._h, ns, _pd(yh) if ns else None, _pd(Fs) if p else None,
+                                                  _pd(Ft) if p else None, p, Xd._h, Zd._h))
+                Z[:, c0:c0 + 1024] = Zd.numpy()
+            finally:
+                Xd.free()
+                if Zd is not None:
+                    Zd.free()
+        return Z
 
     def free(self):
         if getattr(self, "_h", None) and self._h:

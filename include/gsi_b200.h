@@ -106,7 +106,8 @@ int32_t gsi_ctx_gemm_timing(gsi_ctx* ctx, int32_t enable, double* ms_out, int64_
 /* CUDA-event time per phase while gemm timing is enabled: ms_out8[0] operator products,
  * [1] LU normaliser, [2] QR/TSQR, [3] small SVD, [4] back-multiplication; of gsi_kernelcov_chol:
  * [5] materialising A, [6] diagonal blocks, [7] panel solves, and its trailing updates in [0]
- * (also counted by gsi_ctx_gemm_timing with their flops).                                  */
+ * (also counted by gsi_ctx_gemm_timing with their flops), as is the triangular product of
+ * gsi_chol_simulate.                                                                       */
 int32_t gsi_ctx_phase_timing(gsi_ctx* ctx, double* ms_out8, int32_t reset);
 
 /* Tuning knobs (no reference counterpart; results do not depend on them beyond rounding-
@@ -325,6 +326,12 @@ typedef struct gsi_chol gsi_chol;
  * GSI_ERR_UNSUPPORTED; a factor that does not fit the free device memory (cudaMemGetInfo): GSI_ERR_UNSUPPORTED before
  * any large allocation, the message names the bytes needed.                                                           */
 int32_t gsi_kernelcov_chol(gsi_op* op, gsi_chol** out, int64_t* failed_column_out);
+/* As gsi_kernelcov_chol, with a per-point diagonal: factors op + diag(d), d a host array of n doubles (NULL: exactly
+ * gsi_kernelcov_chol).  d_i is added to the materialised diagonal with one rounding, as the operator's nugget is, so a
+ * constant d on an operator without nugget gives the bits of that nugget inside the operator.  Per-point nuggets are
+ * heteroscedastic observation noise; gsi_chol_solve, gsi_chol_logdet and gsi_chol_simulate take such a factor as it is.
+ * Errors: those of gsi_kernelcov_chol, and a non-finite d_i: GSI_ERR_INVALID_ARGUMENT before any allocation.          */
+int32_t gsi_kernelcov_chol_diag(gsi_op* op, const double* diag, gsi_chol** out, int64_t* failed_column_out);
 int32_t gsi_chol_free(gsi_chol* f); /* idempotent on NULL, never throws (Julia finalizer) */
 int32_t gsi_chol_size(const gsi_chol* f, int64_t* n_out);
 /* log det A = 2 sum_i log L[i, i], summed in a fixed order (Gaussian log-likelihood of covariance parameters)          */
@@ -348,6 +355,21 @@ int32_t gsi_chol_solve(gsi_chol* f, int32_t half, const gsi_buf* B, gsi_buf* X);
  * columns at the sources: GSI_ERR_NOT_POSDEF.                                                                          */
 int32_t gsi_chol_krige_variance(gsi_chol* f, gsi_op* cross, const double* F_s, const double* F_t, int64_t p,
                                 double* var_out);
+/* Gaussian simulation (LU simulation, GSLIB LUSIM) on the factor A = L L' of the joint matrix of the points
+ * P = [S (ns sources); T (m = n - ns targets)], A = C(P, P) + diag(d): d_i = the nugget (observation noise) at the sources
+ * and tau at the targets (gsi_kernelcov_chol_diag; tau = 0 simulates the noise-free field that gsi_chol_krige_variance
+ * describes, a small tau > 0 is the jitter smooth kernels need when targets lie close together).  With L_SS the leading
+ * ns x ns block of L, host standard normals Xi = [Xi_S; Xi_T] (TALL n x k, 1 <= k <= 1024) and a drift F_s (host
+ * column-major ns x p), F_t (host column-major m x p), 0 <= p <= 32:
+ *   g = L_SS^-1 y,  G = L_SS^-1 F_s,  B = (G'G)^-1 G' (g 1' - Xi_S),  V = [g 1' - G B; Xi_T],  Z = F_t B + L(T, :) V
+ * into Z (TALL m x k): k realisations at the targets conditioned on y (host, ns values).  Xi = 0 gives the kriging estimate
+ * (simple for p = 0, else universal); Cov(Z) has the kriging variance + tau on its diagonal; p = 0 (known zero mean)
+ * gives Z = L_TS g + L_TT Xi_T and never reads Xi_S.  ns = 0 (p = 0): unconditional, Z = L Xi.  Results are
+ * bit-reproducible run to run.  Errors: ns outside 0 .. n - 1, p outside 0..32, p > 0 with ns = 0, or a non-finite
+ * entry of y, F_s, F_t or Xi: GSI_ERR_INVALID_ARGUMENT; bad shapes or layouts: GSI_ERR_DIMENSION_MISMATCH; linearly
+ * dependent drift columns at the sources: GSI_ERR_NOT_POSDEF.                                                          */
+int32_t gsi_chol_simulate(gsi_chol* f, int64_t ns, const double* y, const double* F_s, const double* F_t, int64_t p,
+                          const gsi_buf* Xi, gsi_buf* Z);
 
 /* FFTRF.powerlaw_structuredgrid (src/FFTRF.jl:83-100) for a batch of fields, on the device -- the
  * sampler behind getxis(samplefield, numfields, ...) (src/GeostatInversion.jl:29-38).  dim in {2, 3};

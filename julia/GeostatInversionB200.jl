@@ -10,7 +10,8 @@
 #   getxis(Val{:iwantfields}, ...), pcgalsqr / pcgadirect / pcga / rga with the reference's
 #   positional and keyword arguments,
 # plus covsolve(C, B; rtol, maxiter, rank, seed), the dense factor covchol(C) with covchol_solve / covchol_logdet /
-# covchol_variance, and krige(...; method = :cg | :cholesky, variance) on the kernel-covariance operators (new),
+# covchol_variance, krige(...; method = :cg | :cholesky, variance), covchol(C; diag), covchol_simulate and the
+# conditional / unconditional simulate(...) on the kernel-covariance operators (new),
 # for A::Matrix{Float64}, A::KernelCovMatrix (new), A::KernelCrossCovMatrix (new, not symmetric) and
 # A::LowRankCovMatrix, whose method set is
 # the one the reference's LowRankCovMatrix provides (src/lowrank.jl:38-60,115-139):
@@ -408,17 +409,24 @@ function krige(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{
 end
 
 """
-covchol(C) -> CovCholesky
+covchol(C; diag=nothing) -> CovCholesky
 
-Dense Cholesky factor C = L L' of a square kernel-covariance operator (KernelCovMatrix, KernelCovGrid, KernelCovModel,
-KernelCovModelGrid; nugget included) on the device by gsi_kernelcov_chol: one GPU, about 8 n^2 bytes.  A non-positive
-pivot throws LinearAlgebra.PosDefException(column).  Freed by its finalizer.
+Dense Cholesky factor C + Diagonal(diag) = L L' of a square kernel-covariance operator (KernelCovMatrix, KernelCovGrid,
+KernelCovModel, KernelCovModelGrid; nugget included) on the device by gsi_kernelcov_chol (gsi_kernelcov_chol_diag with a
+per-point diagonal of n values): one GPU, about 8 n^2 bytes.  A non-positive pivot throws
+LinearAlgebra.PosDefException(column).  Freed by its finalizer.
 """
 mutable struct CovCholesky; h::Ptr{Cvoid}; n::Int; ctx::Context; end
-function covchol(C::KernelCovMatrix)
+function covchol(C::KernelCovMatrix; diag::Union{Nothing, Vector{Float64}}=nothing)
 	out = Ref{Ptr{Cvoid}}(C_NULL)
 	col = Ref{Int64}(0)
-	check(ccall((:gsi_kernelcov_chol, LIB), Int32, (Ptr{Cvoid}, Ptr{Ptr{Cvoid}}, Ptr{Int64}), C.h, out, col))
+	if diag === nothing
+		check(ccall((:gsi_kernelcov_chol, LIB), Int32, (Ptr{Cvoid}, Ptr{Ptr{Cvoid}}, Ptr{Int64}), C.h, out, col))
+	else
+		length(diag) == size(C, 2) || throw(DimensionMismatch("covchol: diag has $(length(diag)) values, C is $(size(C, 2)) x $(size(C, 2))"))
+		check(ccall((:gsi_kernelcov_chol_diag, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Ptr{Cvoid}}, Ptr{Int64}),
+			C.h, diag, out, col))
+	end
 	f = CovCholesky(out[], size(C, 2), C.ctx)
 	finalizer(x->ccall((:gsi_chol_free, LIB), Int32, (Ptr{Cvoid},), x.h), f)    # idempotent, never throws
 	return f
@@ -461,6 +469,61 @@ function covchol_variance(f::CovCholesky, Cx::KernelCrossCovMatrix; drift=nothin
 		(Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Float64}),
 		f.h, Cx.h, p > 0 ? pointer(F) : C_NULL, p > 0 ? pointer(FT) : C_NULL, p, var))
 	return var
+end
+
+"""
+covchol_simulate(f, Xi; ncond=0, y=nothing, drift=nothing) -> Z ((n - ncond) x k)
+
+Realisations at the last n - ncond points of a factor of the joint matrix [sources; targets] (gsi_chol_simulate):
+Z = F_t B + L(T, :) V from the standard normals Xi (n x k, any k; 1024 columns per device call), conditioned on y
+(ncond values) at the first ncond points with drift = nothing (simple kriging), :constant or (F_sources, F_targets),
+p <= 32.  Xi = 0 gives the kriging estimate; ncond = 0 gives unconditional samples L Xi.
+"""
+function covchol_simulate(f::CovCholesky, Xi::VecOrMat{Float64}; ncond::Int=0, y=nothing, drift=nothing)
+	ns, m = ncond, f.n - ncond
+	drift !== nothing && ns == 0 && throw(ArgumentError("covchol_simulate: a drift needs conditioning data (ncond > 0)"))
+	F, FT = drift === nothing ? (zeros(ns, 0), zeros(m, 0)) :
+		drift === :constant ? (ones(ns, 1), ones(m, 1)) : (Matrix{Float64}(drift[1]), Matrix{Float64}(drift[2]))
+	p = size(F, 2)
+	yv = y === nothing ? zeros(0) : Vector{Float64}(y)
+	length(yv) == ns || throw(DimensionMismatch("covchol_simulate: y has $(length(yv)) values, ncond is $ns"))
+	X = Matrix{Float64}(reshape(Xi, f.n, :))
+	Z = zeros(m, size(X, 2))
+	for c0 in 1:1024:size(X, 2)
+		cols = c0:min(c0 + 1023, size(X, 2))
+		Xd = upload!(DeviceMatrix(f.ctx, GSI_LAYOUT_TALL, f.n, length(cols)), X[:, cols])
+		Zd = DeviceMatrix(f.ctx, GSI_LAYOUT_TALL, m, length(cols))
+		GC.@preserve yv F FT check(ccall((:gsi_chol_simulate, LIB), Int32,
+			(Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Cvoid}, Ptr{Cvoid}),
+			f.h, ns, ns > 0 ? pointer(yv) : C_NULL, p > 0 ? pointer(F) : C_NULL, p > 0 ? pointer(FT) : C_NULL, p,
+			Xd.h, Zd.h))
+		Z[:, cols] = download(Zd)
+	end
+	return Z
+end
+
+"""
+simulate(kinds, sills, ranges, targets, nreal; rotations, betas, sources=nothing, y=nothing, nugget=0.0,
+         target_nugget=0.0, drift=nothing, seed=nothing) -> Z (m x nreal)
+
+Gaussian realisations at the targets (d x m) under the nested model of KernelCovModel, conditioned on y at the sources
+(observation noise `nugget`) or unconditional (sources = nothing): LU simulation on one dense factor of the joint matrix
+of [sources targets] plus Diagonal(nugget at the sources, target_nugget at the targets) (covchol, covchol_simulate; one
+GPU, about 8 (ns + m)^2 bytes).  The standard normals are drawn on the host by `randn` (after `Random.seed!(seed)` when
+a seed is given).  drift as in krige, conditional simulation only.
+"""
+function simulate(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges::Matrix{Float64}, targets::Matrix{Float64},
+		nreal::Int; rotations::Union{Nothing, Array{Float64, 3}}=nothing, betas::Union{Nothing, Vector{Float64}}=nothing,
+		sources::Union{Nothing, Matrix{Float64}}=nothing, y=nothing, nugget=0.0, target_nugget=0.0, drift=nothing,
+		seed::Union{Nothing, Int}=nothing)
+	sources === nothing && drift !== nothing && throw(ArgumentError("simulate: a drift needs conditioning data"))
+	S = sources === nothing ? zeros(size(targets, 1), 0) : sources
+	ns, m = size(S, 2), size(targets, 2)
+	seed === nothing || Random.seed!(seed)
+	Xi = randn(ns + m, nreal)
+	C = KernelCovModel(kinds, sills, ranges, hcat(S, targets); rotations=rotations, betas=betas, nugget=0.0)
+	f = covchol(C; diag=vcat(fill(Float64(nugget), ns), fill(Float64(target_nugget), m)))
+	return covchol_simulate(f, Xi; ncond=ns, y=ns > 0 ? y : nothing, drift=drift)
 end
 
 module RandMatFact

@@ -375,6 +375,7 @@ class KernelCovMatrix(_Operator):
         self.row0 = int(row0)
         self.mloc = int(n - row0 if mloc is None else mloc)
         self.kind = _KINDS[kind]
+        self.dim, self.nstruct = d, 1
         check(self._lib.gsi_op_kernelcov(self.ctx._h, self.kind, d, n, _pd(coords), _pd(ell), float(sigma2),
                                          float(nugget), float(beta), self.row0, self.mloc, C.byref(self._h)))
 
@@ -398,6 +399,7 @@ class GridKernelCovMatrix(_Operator):
         self.row0 = int(row0)
         self.mloc = int(n - row0 if mloc is None else mloc)
         self.kind = _KINDS[kind]
+        self.dim, self.nstruct = d, 1
         check(self._lib.gsi_op_kernelcov_grid(self.ctx._h, self.kind, d, dims, _pd(spacing), _pd(ell), float(sigma2),
                                               float(nugget), float(beta), self.row0, self.mloc, C.byref(self._h)))
 
@@ -468,6 +470,7 @@ class KernelCovModelMatrix(_Operator):
         self.row0 = int(row0)
         self.mloc = int(n - row0 if mloc is None else mloc)
         args, self._keep = _model_args(structures, d)
+        self.dim, self.nstruct = d, args[0]
         check(self._lib.gsi_op_kernelcov_model(self.ctx._h, d, n, _pd(coords), *args, float(nugget), self.row0,
                                                self.mloc, C.byref(self._h)))
 
@@ -487,6 +490,7 @@ class GridKernelCovModelMatrix(_Operator):
         self.row0 = int(row0)
         self.mloc = int(n - row0 if mloc is None else mloc)
         args, self._keep = _model_args(structures, d)
+        self.dim, self.nstruct = d, args[0]
         check(self._lib.gsi_op_kernelcov_model_grid(self.ctx._h, d, dims, _pd(spacing), *args, float(nugget), self.row0,
                                                     self.mloc, C.byref(self._h)))
 

@@ -52,5 +52,9 @@ void chol_variance(const gsi_chol* f, gsi_op* cross, const double* Fs, const dou
 // Z = F_t B + L(T, :) V: conditional (ns > 0) or unconditional (ns = 0) realisations from the factor of the joint matrix
 void chol_simulate(const gsi_chol* f, int64_t ns, const double* y, const double* Fs, const double* Ft, int64_t p,
                    const gsi_buf* Xi, gsi_buf* Z);
+// Gaussian ML / REML log-likelihood of the operator's parameters (beta by GLS), optionally with its exact gradient
+// (grad_out: nstruct (1 + d) + 1 values); factors, evaluates and frees the factor
+void chol_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int reml, double* loglik, double* beta_out,
+                 double* grad_out, int64_t* failed_column);
 
 }  // namespace gsi

@@ -624,6 +624,8 @@ static double model_host(const CovModel& m, const double* x) {
 static void set_model(gsi_op* op, const CovModel& m, double nugget, bool generated) {
     op->type = OP_KERNELCOV; op->dim = m.d; op->nugget = nugget;
     op->kind = m.kinds[0]; op->sigma2 = m.sills[0]; op->beta = m.betas[0];
+    for (int s = 0; s < m.nstruct; ++s)
+        for (int k = 0; k < m.d; ++k) op->mranges[s][k] = m.ranges[s][k];
     if (m.nstruct == 1) return;
     op->sigma2 = 1.0; op->beta = 1.0;
     if (!generated) return;
@@ -1104,5 +1106,15 @@ GSI_API int32_t gsi_chol_simulate(gsi_chol* f, int64_t ns, const double* y, cons
         GSI_REQUIRE(f && Xi && Z, GSI_ERR_INVALID_ARGUMENT, "null argument");
         use(f->ctx);
         chol_simulate(f, ns, y, F_s, F_t, p, Xi, Z);
+    });
+}
+
+GSI_API int32_t gsi_kernelcov_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int32_t reml,
+                                     double* loglik_out, double* beta_out, double* grad_out, int64_t* failed_column_out) {
+    if (failed_column_out) *failed_column_out = 0;
+    return guarded([&] {
+        GSI_REQUIRE(op && y && loglik_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(op->ctx);
+        chol_loglik(op, y, F, p, reml, loglik_out, beta_out, grad_out, failed_column_out);
     });
 }

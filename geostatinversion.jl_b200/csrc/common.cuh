@@ -157,6 +157,9 @@ struct gsi_op {
     int32_t nstruct = 1;
     int32_t mkinds[GSI_MODEL_MAX_STRUCTURES] = {0, 0, 0, 0};
     double msills[GSI_MODEL_MAX_STRUCTURES] = {0, 0, 0, 0}, mbetas[GSI_MODEL_MAX_STRUCTURES] = {1, 1, 1, 1};
+    // the principal-axis ranges of every structure (one structure: the length scales ell), kept for the likelihood
+    // gradient in natural units (gsi_kernelcov_loglik); the kernels see them only through the scaled coordinates
+    double mranges[GSI_MODEL_MAX_STRUCTURES][3] = {};
     // cross-covariance C(T, S) (OP_KERNELCROSS): ucoords / lattice hold the n source points, these this rank's mloc
     // target points (compacted, so that bulk copies of them stay 16-byte aligned), same layouts with pitch nt_pad
     double* ucoords_t = nullptr;
@@ -207,6 +210,16 @@ struct KcovBlock {
     int64_t rs, cs;
 };
 void kcov_block(gsi_op* op, int side, const KcovBlock& b);
+// likelihood-gradient contraction over one chunk of columns [j0, j0 + w) of Z = -W (row-major, pitch ldz, rows from j0
+// on; kcov_gemm.cu, kcov_grad_kernel): per-CTA partial sums, KG_SLOTS each, into part; returns the number of CTAs.
+// Slot 4 s: sum_ij w_ij W_ij k_s, slot 4 s + 1 + a: sum_ij w_ij W_ij k_s'(r2_s) du_(s,a)^2, slot 16: sum_i W_ii
+// (w_ij = 2 off the diagonal, 1 on it; i >= j, both < n)
+constexpr int KG_SLOTS = GSI_MODEL_MAX_STRUCTURES * 4 + 1;
+constexpr int KG_ROWS = 128;      // rows of a contraction tile (one CTA)
+constexpr int KG_COLS = 64;       // columns of a contraction tile
+int64_t kcov_grad(gsi_op* op, const double* Z, int64_t ldz, int64_t j0, int64_t w, double* part);
+// out[s] = sum over the nparts rows of part (KG_SLOTS each) in a fixed order
+void kcov_grad_reduce(gsi_ctx* ctx, const double* part, int64_t nparts, double* out);
 // ---- dense_gemm.cu : W = A X (trans=0) or A' X (trans=1); alpha scaling
 void dense_apply(gsi_ctx*, const gsi_buf* A, int trans, const gsi_buf* X, gsi_buf* W, double alpha);
 void tall_window_update(gsi_ctx*, const double* Pd, int64_t ldp, int64_t rows, int64_t kdim, const gsi_buf* X,

@@ -34,6 +34,26 @@
 // Cov(Z) = L_TT L_TT' + (F_t - L_TS G)(G'G)^-1(F_t - L_TS G)', whose diagonal is the kriging variance + tau; p = 0 gives
 // Z = L_TS g + L_TT Xi_T, independent of Xi_S; ns = 0 gives Z = L Xi.  The product Z = L(T, :) V is chol_trmm_kernel;
 // g and G come from a forward sweep that stops after the source blocks, G'G and G' Xi_S from chol_gemm_kernel.
+//
+// Gaussian log-likelihood of the covariance parameters and its exact gradient (chol_loglik).  A = C(S, S) + nugget I is
+// the square operator exactly as built, y the n observations, F the n x p drift (0 <= p <= 32), A = L L'.  With
+// g = L^-1 y, G = L^-1 F, R'R = G'G (R upper triangular), beta = (G'G)^-1 G'g, e = g - G beta and q = ||e||^2:
+//   ML (beta profiled by GLS):  l = -1/2 (n log 2 pi + log det A + q)
+//   REML:                       l = -1/2 ((n - p) log 2 pi + log det A + 2 sum_k log R_kk + q)
+// The REML form leaves out log det F'F, so its value depends on the scaling of F (its gradient and maximiser do not).
+// With alpha = L^-T e (= A^-1 (y - F beta)) and H = L^-T G R^-1 (H H' = A^-1 F (F'A^-1 F)^-1 F'A^-1):
+//   W = alpha alpha' - A^-1 (ML),  W = alpha alpha' - A^-1 + H H' (REML),  dl / dtheta = 1/2 sum_ij W_ij dA_ij / dtheta
+// (for ML the envelope theorem makes this the gradient of the profile likelihood).  The parameters are, per structure s,
+// sill_s then range_(s,a), a = 0 .. d - 1, then the nugget; dA / dnugget = I, the others as in kcov_grad_kernel.
+// Device work: the factor (chol_factor); one forward sweep of [F | y] as a row-major np x 128 block, G'G and G'g on
+// chol_gemm_kernel, R on chol_upper_kernel, beta and log det R, e (and G R^-1), q in fixed-order kernels; for the gradient
+// one backward sweep of [G R^-1 | e] gives [H | alpha].  A^-1 is never held whole: for each chunk of <= 1024 columns from
+// block column j0 the identity columns are swept forward from block j0 (the rows above are zero) and backward down to
+// block j0, which gives rows >= j0 of A^-1(:, chunk) bit for bit as the full sweeps would (2 n^3 / 3 flops in all, as a
+// triangular inverse plus L^-T L^-1, in one np x 1024 block).  The rank-(p + 1) term is applied to the chunk first as one
+// chol_gemm_kernel update, Z = A^-1 - [H alpha][H alpha]' = -W on rows >= j0, with K = p + 1 rounded up to 32: on the
+// tensor cores it costs about 2 n^2 K flops in all (1 ms at n = 20 000), where folding it into the contraction would add
+// 2 (p + 1) loads and p + 1 FMAs per entry to an FP64-pipe-bound kernel.  kcov_grad_kernel then contracts each chunk.
 #include "common.cuh"
 #include "algos.h"
 #include "ptx.cuh"
@@ -414,6 +434,73 @@ __global__ void chol_sim_out_kernel(const double* __restrict__ Zw, int64_t kp, i
     Z[r * ldz + c] = p > 0 ? fb + z : z;
 }
 
+// Likelihood value, drift part.  GtG: [G | g]'[G | g] (row-major, pitch 128), R: upper p x p with R'R = G'G (column-major,
+// pitch p).  out[0 .. p - 1] = beta = R^-1 R^-T G'g, out[CH_MAX_DRIFT] = sum_k log R_kk, in order (one thread)
+__global__ void chol_lik_beta_kernel(const double* __restrict__ GtG, const double* __restrict__ R, int p,
+                                     double* __restrict__ out) {
+    double z[CH_MAX_DRIFT];
+    double ld = 0.0;
+    for (int i = 0; i < p; ++i) {                                 // R' z = G'g
+        double s = GtG[i * CH_B + p];
+        for (int k = 0; k < i; ++k) s -= R[k + i * p] * z[k];
+        z[i] = s / R[i + i * p];
+        ld += log(R[i + i * p]);
+    }
+    for (int i = p - 1; i >= 0; --i) {                            // R beta = z
+        double s = z[i];
+        for (int k = i + 1; k < p; ++k) s -= R[i + k * p] * z[k];
+        z[i] = s / R[i + i * p];
+    }
+    for (int i = 0; i < p; ++i) out[i] = z[i];
+    out[CH_MAX_DRIFT] = ld;
+}
+
+// Row i of W = [G | g] (row-major np x 128): g_i <- e_i = g_i - G_i beta.  mode 1 (ML gradient): G_i <- 0; mode 2 (REML
+// gradient): G_i <- G_i R^-1 (the row solve h R = G_i); mode 0 leaves G
+__global__ void chol_lik_resid_kernel(double* __restrict__ W, int64_t np, int p, const double* __restrict__ beta,
+                                      const double* __restrict__ R, int mode) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= np) return;
+    double* w = W + i * CH_B;
+    double e = w[p];
+    for (int q = 0; q < p; ++q) e -= w[q] * beta[q];
+    w[p] = e;
+    if (mode == 1) {
+        for (int q = 0; q < p; ++q) w[q] = 0.0;
+    } else if (mode == 2) {
+        double h[CH_MAX_DRIFT];
+        for (int k = 0; k < p; ++k) {
+            double s = w[k];
+            for (int q = 0; q < k; ++q) s -= h[q] * R[q + k * p];
+            h[k] = s / R[k + k * p];
+        }
+        for (int k = 0; k < p; ++k) w[k] = h[k];
+    }
+}
+
+// *out = sum_i W[i * 128 + col]^2 over the n true rows: one CTA, the order of chol_logdet_kernel
+__global__ void chol_lik_sumsq_kernel(const double* __restrict__ W, int64_t n, int col, double* __restrict__ out) {
+    __shared__ double red[1024];
+    double s = 0.0;
+    for (int64_t i = threadIdx.x; i < n; i += 1024) {
+        const double v = W[i * CH_B + col];
+        s = fma(v, v, s);
+    }
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = 512; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) out[0] = red[0];
+}
+
+// Z(j0 + c, c) = 1, c < w: the identity columns of a chunk (row-major, pitch ldz; the rest was zeroed)
+__global__ void chol_eye_kernel(double* __restrict__ Z, int64_t ldz, int64_t j0, int64_t w) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c < w) Z[(j0 + c) * ldz + c] = 1.0;
+}
+
 namespace {
 
 template <bool AK, bool BK, bool CR>
@@ -434,11 +521,13 @@ ChGemm gm(const double* A, int64_t lda, const double* B, int64_t ldb, double* C,
 }
 
 // W (row-major np x kp, pitch ldw; kp a multiple of 128) <- L^-1 W on the leading nb block rows (nb = np / 128: all of
-// W; a smaller nb leaves the rows from nb * 128 on unchanged, and the rows above are those of the full solve)
-void forward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp, int64_t nb) {
+// W; a smaller nb leaves the rows from nb * 128 on unchanged, and the rows above are those of the full solve).  kb0 > 0
+// starts at block row kb0 for a W whose rows above kb0 * 128 are zero: those rows are neither read nor written, and the
+// rows below are bit for bit those of the full sweep (which would only subtract exact zeros from them)
+void forward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp, int64_t nb, int64_t kb0 = 0) {
     gsi_ctx* ctx = f->ctx;
     const int64_t nt = kp / CH_B;
-    for (int64_t kb = 0; kb < nb; ++kb) {
+    for (int64_t kb = kb0; kb < nb; ++kb) {
         const int64_t j0 = kb * CH_B;
         double* Wj = W + j0 * ldw;
         gemm<false, false, true>(ctx, gm(f->inv + kb * CH_B * CH_B, CH_B, Wj, ldw, Wj, ldw, CH_B, 0, 0), 1, nt);
@@ -447,15 +536,17 @@ void forward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp, int64_t nb) 
     }
 }
 
-// W <- L^-T W
-void backward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp) {
+// W <- L^-T W.  kb1 > 0 stops after block row kb1: the rows from kb1 * 128 on are those of the full sweep (they do not
+// depend on the rows above), the rows above are neither read nor written
+void backward(const gsi_chol* f, double* W, int64_t ldw, int64_t kp, int64_t kb1 = 0) {
     gsi_ctx* ctx = f->ctx;
     const int64_t nb = f->np / CH_B, nt = kp / CH_B;
-    for (int64_t kb = nb - 1; kb >= 0; --kb) {
+    for (int64_t kb = nb - 1; kb >= kb1; --kb) {
         const int64_t j0 = kb * CH_B;
         double* Wj = W + j0 * ldw;
         gemm<true, false, true>(ctx, gm(f->inv + kb * CH_B * CH_B, CH_B, Wj, ldw, Wj, ldw, CH_B, 0, 0), 1, nt);
-        gemm<true, false, true>(ctx, gm(f->L + j0, f->np, Wj, ldw, W, ldw, CH_B, 1, 0), kb, nt);
+        gemm<true, false, true>(ctx, gm(f->L + j0 + kb1 * CH_B * f->np, f->np, Wj, ldw, W + kb1 * CH_B * ldw, ldw, CH_B, 1, 0),
+                                kb - kb1, nt);
     }
 }
 
@@ -785,6 +876,130 @@ void chol_simulate(const gsi_chol* f, int64_t ns, const double* y, const double*
     GSI_CUDA(cudaGetLastError());
     count_launch(ctx);
     GSI_CUDA(cudaStreamSynchronize(st));
+}
+
+void chol_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int reml, double* loglik, double* beta_out,
+                 double* grad_out, int64_t* failed_column) {
+    gsi_ctx* ctx = op->ctx;
+    cudaStream_t st = ctx->stream;
+    if (failed_column) *failed_column = 0;
+    GSI_REQUIRE(op->type == OP_KERNELCOV, GSI_ERR_UNSUPPORTED,
+                "kernelcov_loglik needs a square kernel-covariance operator (gsi_op_kernelcov, _grid, _model or _model_grid)");
+    GSI_REQUIRE(ctx->world == 1, GSI_ERR_UNSUPPORTED, "kernelcov_loglik is single-GPU: the dense factor is not distributed");
+    const int64_t n = op->n, np = round_up(n, CH_B), nb = np / CH_B;
+    GSI_REQUIRE(p >= 0 && p <= CH_MAX_DRIFT, GSI_ERR_INVALID_ARGUMENT, "kernelcov_loglik: p must be in 0..32");
+    GSI_REQUIRE((p == 0) == (F == nullptr), GSI_ERR_INVALID_ARGUMENT, "kernelcov_loglik: F must be given iff p > 0");
+    GSI_REQUIRE(!reml || p < n, GSI_ERR_INVALID_ARGUMENT, "kernelcov_loglik: REML needs fewer drift columns than points");
+    bool finite = true;
+    for (int64_t i = 0; i < n; ++i) finite = finite && std::isfinite(y[i]);
+    for (int64_t i = 0; i < n * p; ++i) finite = finite && std::isfinite(F[i]);
+    GSI_REQUIRE(finite, GSI_ERR_INVALID_ARGUMENT, "kernelcov_loglik: y or F has a non-finite entry");
+    const bool want_grad = grad_out != nullptr;
+    GSI_REQUIRE(!want_grad || op->table == nullptr, GSI_ERR_UNSUPPORTED,
+                "kernelcov_loglik: the gradient needs an operator on coordinates (a grid operator's lattice table has no "
+                "derivative; pass the grid nodes' coordinates to gsi_op_kernelcov / _model)");
+    // device memory of the whole call, checked before the factor is allocated: the factor (as chol_factor counts it),
+    // the [F | y] block and, for the gradient, one chunk of A^-1 and the partial sums of the contraction
+    const int64_t ldz = np < CH_MAX_CHUNK ? np : CH_MAX_CHUNK;
+    const int64_t nchunks = (n + CH_MAX_CHUNK - 1) / CH_MAX_CHUNK;
+    const int64_t max_parts = (n + KG_ROWS - 1) / KG_ROWS * (CH_MAX_CHUNK / KG_COLS);
+    const size_t small_doubles = (size_t)CH_B * CH_B + CH_MAX_DRIFT * CH_MAX_DRIFT + 2 * CH_MAX_DRIFT;
+    double need = (double)np * np * 8.0 + (double)np * CH_B * 8.0 + 4096.0 + (double)np * CH_B * 8.0 + small_doubles * 8.0;
+    if (want_grad) need += (double)np * ldz * 8.0 + (double)(max_parts + nchunks + 1) * KG_SLOTS * 8.0;
+    size_t fr = 0, tot = 0;
+    GSI_CUDA(cudaMemGetInfo(&fr, &tot));
+    if (need > (double)fr) {
+        pool_release(ctx);
+        GSI_CUDA(cudaMemGetInfo(&fr, &tot));
+    }
+    if (need > (double)fr) {
+        char msg[256];
+        snprintf(msg, sizeof(msg), "kernelcov_loglik: n = %lld needs %.0f bytes of device memory, %zu are free",
+                 (long long)n, need, fr);
+        throw Error(GSI_ERR_UNSUPPORTED, msg);
+    }
+    std::unique_ptr<gsi_chol, void (*)(gsi_chol*)> f(chol_factor(op, nullptr, failed_column), chol_destroy);
+    // value: [G | g] = L^-1 [F | y] (row-major np x 128, zero padded), beta, e, q
+    DevMem W((size_t)np * CH_B * sizeof(double));
+    DevMem small(small_doubles * sizeof(double));
+    double* GtG = small.d();
+    double* R = GtG + CH_B * CH_B;
+    double* res = R + CH_MAX_DRIFT * CH_MAX_DRIFT;             // beta (p), log det R, q
+    {
+        std::vector<double> Wh((size_t)np * CH_B, 0.0);
+        for (int64_t i = 0; i < n; ++i) {
+            for (int64_t q = 0; q < p; ++q) Wh[(size_t)i * CH_B + q] = F[q * n + i];
+            Wh[(size_t)i * CH_B + p] = y[i];
+        }
+        GSI_CUDA(cudaMemcpyAsync(W.d(), Wh.data(), Wh.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+        GSI_CUDA(cudaMemsetAsync(res, 0, 2 * CH_MAX_DRIFT * sizeof(double), st));
+        forward(f.get(), W.d(), CH_B, CH_B, nb);
+        GSI_CUDA(cudaStreamSynchronize(st));                   // Wh is freed on leaving the scope
+    }
+    int* flag = f->flags;
+    GSI_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
+    if (p > 0) {
+        gemm<false, false, true>(ctx, gm(W.d(), CH_B, W.d(), CH_B, GtG, CH_B, np, 0, 0), 1, 1);
+        tall_head_to_cm_kernel<<<(unsigned)((p * p + 255) / 256), 256, 0, st>>>(GtG, CH_B, (int)p, R);
+        chol_upper_kernel<<<1, 1024, 0, st>>>(R, (int)p, flag + 1);
+        chol_lik_beta_kernel<<<1, 1, 0, st>>>(GtG, R, (int)p, res);
+        const int mode = !want_grad ? 0 : (reml ? 2 : 1);
+        chol_lik_resid_kernel<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(W.d(), np, (int)p, res, R, mode);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx, 4);
+    }
+    chol_lik_sumsq_kernel<<<1, 1024, 0, st>>>(W.d(), n, (int)p, res + CH_MAX_DRIFT + 1);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+    double hres[2 * CH_MAX_DRIFT];
+    int hf[2] = {0, 0};
+    GSI_CUDA(cudaMemcpyAsync(hres, res, sizeof(hres), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaMemcpyAsync(hf, flag, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    if (hf[1] != 0)
+        throw Error(GSI_ERR_NOT_POSDEF, "kernelcov_loglik: F' A^-1 F is not positive definite (the drift columns are "
+                                        "linearly dependent)");
+    const double log2pi = 1.83787706640934548356;
+    const double q = hres[CH_MAX_DRIFT + 1];
+    *loglik = reml ? -0.5 * ((double)(n - p) * log2pi + f->logdet + 2.0 * hres[CH_MAX_DRIFT] + q)
+                   : -0.5 * ((double)n * log2pi + f->logdet + q);
+    if (beta_out)
+        for (int64_t k = 0; k < p; ++k) beta_out[k] = hres[k];
+    if (!want_grad) return;
+    // gradient: [H | alpha] = L^-T [G R^-1 | e] (ML: H = 0), then per chunk of A^-1 the rank update and the contraction
+    backward(f.get(), W.d(), CH_B, CH_B);
+    DevMem Z((size_t)np * ldz * sizeof(double));
+    DevMem part((size_t)max_parts * KG_SLOTS * sizeof(double));
+    DevMem csum((size_t)(nchunks + 1) * KG_SLOTS * sizeof(double));
+    const int64_t K = round_up(p + 1, CH_K);
+    int64_t c = 0;
+    for (int64_t j0 = 0; j0 < n; j0 += CH_MAX_CHUNK, ++c) {
+        const int64_t wp = np - j0 < CH_MAX_CHUNK ? np - j0 : CH_MAX_CHUNK, kb0 = j0 / CH_B;
+        double* Zc = Z.d() + j0 * ldz;
+        GSI_CUDA(cudaMemsetAsync(Zc, 0, (size_t)(np - j0) * ldz * sizeof(double), st));
+        chol_eye_kernel<<<(unsigned)((wp + 255) / 256), 256, 0, st>>>(Z.d(), ldz, j0, wp);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx);
+        forward(f.get(), Z.d(), ldz, wp, nb, kb0);
+        backward(f.get(), Z.d(), ldz, wp, kb0);
+        const double* Wj = W.d() + j0 * CH_B;
+        gemm<true, true, true>(ctx, gm(Wj, CH_B, Wj, CH_B, Zc, ldz, K, 1, 0), (np - j0) / CH_B, wp / CH_B);
+        const int64_t nparts = kcov_grad(op, Z.d(), ldz, j0, wp, part.d());
+        kcov_grad_reduce(ctx, part.d(), nparts, csum.d() + c * KG_SLOTS);
+    }
+    double* total = csum.d() + nchunks * KG_SLOTS;
+    kcov_grad_reduce(ctx, csum.d(), nchunks, total);
+    double S[KG_SLOTS];
+    GSI_CUDA(cudaMemcpyAsync(S, total, sizeof(S), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    const bool model = op->kind == KC_KIND_MODEL;
+    const int ns = model ? op->nstruct : 1, d = op->dim;
+    for (int s = 0; s < ns; ++s) {
+        const double sill = model ? op->msills[s] : op->sigma2;
+        grad_out[s * (1 + d)] = 0.5 * S[4 * s];
+        for (int a = 0; a < d; ++a) grad_out[s * (1 + d) + 1 + a] = -(sill / op->mranges[s][a]) * S[4 * s + 1 + a];
+    }
+    grad_out[ns * (1 + d)] = 0.5 * S[KG_SLOTS - 1];
 }
 
 }  // namespace gsi

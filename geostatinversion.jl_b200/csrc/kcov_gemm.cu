@@ -1058,4 +1058,191 @@ void kcov_block(gsi_op* op, int side, const KcovBlock& b) {
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Likelihood gradient (cov_chol.cu, chol_loglik): the contraction sum_ij w_ij W_ij dA_ij / dtheta over one chunk of
+// columns of W = alpha alpha' - A^-1 (+ H H'), the chunk held as Z = -W (row-major, pitch ldz, row i at Z + i * ldz).
+// Every parameter's dA / dtheta comes from the operator's own scaled coordinates u (layout [nstruct][3][n_pad]; a single
+// kind is the one-structure case of that layout):
+//   dA_ij / dsill_s        = k_s(r2_s)                        (the value kern_eval gives the factor's fill, bit for bit)
+//   dA_ij / drange_(s,a)   = sill_s k_s'(r2_s) (-2 du_(s,a)^2) / range_(s,a),   k' = dk / dr2 in the kernel's own units
+// The kernel sums w W k_s and w W k_s' du_(s,a)^2 (w = 2 below the diagonal, 1 on it) per structure and axis; the host
+// applies sill_s, -2 / range_(s,a) and the factor 1/2.  A single kind with d = 1 runs as DIM = 2 on a zero second
+// coordinate: its axis-1 sums are exact zeros.
+//
+// dk / dr2 per kind (s = sqrt(r2) by fast_sqrt_pos; the 1e-300 offset of r2 makes du = 0 give 0 * finite = 0 for the
+// kinds that divide by s, and du_a^2 / s <= s keeps them finite near the diagonal).  Relative error of the derivative
+// value in units of 2^-52, in the style of the bounds beside kern_eval (2.5 for fast_exp_neg, 2 ulp of s entering with
+// the conditioning of the expression in s, 0.5 per rounding):
+//   exponential  RN(RN(-0.5 e) / s), e = e^-s:        2.5 + 2 s (s in e) + 2 (s in the divisor) + 0.5          = 5 + 2 s
+//   gaussian     -e^-r2:                              2.5                                                      = 2.5
+//   powerlaw     RN(RN(-beta v) / RN(1 + r2)), v the library value (2 + 4 |z|, z = beta log1p r2): + 1.5  = 3.5 + 4 |z|
+//   matern32     RN(-0.5 e):                          2.5 + 2 s                                                = 2.5 + 2 s
+//   matern52     RN(RN(RN(s + 1) e) RN(-1/6)):        2.5 + 2 s + 2 s / (1 + s) + 0.5 + 0.5 + 0.25 + 0.5      = 6.25 + 4 s
+//   spherical    RN(RN(RN(-0.75 t) RN(1 + s)) / s), t = 1 - s (exact for s >= 0.5, 2^-53 below):
+//                0.5 + 0.5 + 0.5 + 0.5 + 0.5 + 2 c, c = 1 + s / (1 - s) + s / (1 + s)                        = 2.5 + 2 c
+// (c grows as s -> 1, where the derivative itself goes to 0 and its absolute error with it.)  Each summed term adds
+// the roundings of w W k' du^2 (3 products and one fma: < 2 units) to these.  The sums are not asserted entry by entry:
+// they cancel near the optimum (W = alpha alpha' - A^-1), so tests/test_gpu_kcov_lik.py bounds each gradient component
+// by 1e-9 S_theta, S_theta = 1/2 sum_ij |W_ij| |dA_ij / dtheta|, the conditioning of the sum.
+// Cost: one kern_eval-sized evaluation plus the derivative (one more FP64 multiply, a division for the exponential and
+// spherical kinds) and 2 + d FMAs per structure per entry: FP64-pipe bound, about 30 FP64 instructions per entry and
+// structure.  Every partial sum has a fixed order (thread: rows in order; warp: a fixed xor tree; CTA: warps in order;
+// then kcov_grad_reduce over the CTAs and the chunks), so the gradient is bit-reproducible.
+constexpr int KG_TY = 4;          // threadIdx.y: row phases (a thread takes rows ty, ty + 4, .. of the tile)
+
+struct KcovGrad {
+    const double* u; int64_t n_pad, n;
+    int nstruct;
+    int kinds[GSI_MODEL_MAX_STRUCTURES];
+    double betas[GSI_MODEL_MAX_STRUCTURES];
+    const double* Z; int64_t ldz, j0, w;
+    double* part;
+};
+
+// k(r2) exactly as kern_eval<kind> computes it, and dk / dr2 in the same scaled units
+__device__ __forceinline__ double kern_value_deriv(int kind, double r2, double beta, const double* __restrict__ tab,
+                                                   double& dk) {
+    if (kind == GSI_KERNEL_GAUSSIAN) {
+        const double e = fast_exp_neg(r2, tab);
+        dk = -e;
+        return e;
+    }
+    if (kind == GSI_KERNEL_POWERLAW) {
+        const double v = exp(-beta * log1p(r2));
+        dk = (-beta * v) / (1.0 + r2);
+        return v;
+    }
+    const double s = fast_sqrt_pos(r2);
+    if (kind == GSI_KERNEL_SPHERICAL) {
+        const double t = 1.0 - s;
+        dk = s < 1.0 ? (-0.75 * t) * (1.0 + s) / s : 0.0;      // -3/4 (1 - s)(1 + s) / s
+        return s < 1.0 ? (0.5 * t) * t * (2.0 + s) : 0.0;
+    }
+    const double e = fast_exp_neg(s, tab);
+    if (kind == GSI_KERNEL_EXPONENTIAL) {
+        dk = (-0.5 * e) / s;                                    // -e^-s / (2 s)
+        return e;
+    }
+    if (kind == GSI_KERNEL_MATERN32) {
+        dk = -0.5 * e;                                          // -e^-s / 2
+        return fma(s, e, e);
+    }
+    dk = ((s + 1.0) * e) * (-1.0 / 6.0);                        // -(1 + s) e^-s / 6
+    return fmin(fma(r2, 1.0 / 3.0, s + 1.0) * e, 1.0);
+}
+
+// One CTA per KG_ROWS x KG_COLS tile of the chunk (rows from j0, chunk columns c = blockIdx.y * KG_COLS + threadIdx.x);
+// tiles wholly above the diagonal write zero partials.  part[(blockIdx.y * gridDim.x + blockIdx.x) * KG_SLOTS + slot].
+template <int DIM>
+__global__ void __launch_bounds__(KG_COLS * KG_TY) kcov_grad_kernel(const __grid_constant__ KcovGrad a) {
+    constexpr int UP = GSI_MODEL_MAX_STRUCTURES * DIM;            // row coordinates per point in shared memory
+    __shared__ double etab[64];
+    __shared__ double urow[KG_ROWS * UP];
+    __shared__ double red[KG_COLS * KG_TY / 32][KG_SLOTS];
+    const int tx = threadIdx.x, ty = threadIdx.y, tid = ty * KG_COLS + tx;
+    const int ns = a.nstruct;
+    const int64_t i0 = a.j0 + (int64_t)blockIdx.x * KG_ROWS;
+    const int64_t c = (int64_t)blockIdx.y * KG_COLS + tx;
+    const int64_t j = a.j0 + c;
+    if (tid < 64) etab[tid] = kExp2Table[tid];
+    for (int e = tid; e < KG_ROWS * ns * DIM; e += KG_COLS * KG_TY) {
+        const int r = e / (ns * DIM), q = e - r * (ns * DIM), s = q / DIM, k = q - s * DIM;
+        const int64_t gi = i0 + r < a.n ? i0 + r : a.n - 1;
+        urow[r * UP + q] = a.u[(s * 3 + k) * a.n_pad + gi];
+    }
+    const int64_t jc = j < a.n ? j : a.n - 1;
+    double uj[GSI_MODEL_MAX_STRUCTURES][DIM];
+#pragma unroll
+    for (int s = 0; s < GSI_MODEL_MAX_STRUCTURES; ++s)
+#pragma unroll
+        for (int k = 0; k < DIM; ++k) uj[s][k] = s < ns ? a.u[(s * 3 + k) * a.n_pad + jc] : 0.0;
+    double acc[KG_SLOTS];
+#pragma unroll
+    for (int q = 0; q < KG_SLOTS; ++q) acc[q] = 0.0;
+    __syncthreads();
+    const bool col_ok = c < a.w && j < a.n;
+    if (a.j0 + (int64_t)blockIdx.y * KG_COLS <= i0 + KG_ROWS - 1) {      // the tile reaches the lower triangle
+        for (int r = ty; r < KG_ROWS; r += KG_TY) {
+            const int64_t i = i0 + r;
+            if (!col_ok || i < j || i >= a.n) continue;
+            const double wv = -a.Z[i * a.ldz + c];
+            const double wt = i == j ? wv : 2.0 * wv;
+            const double* ur = urow + r * UP;
+#pragma unroll
+            for (int s = 0; s < GSI_MODEL_MAX_STRUCTURES; ++s) {
+                if (s < ns) {
+                    const int kind = a.kinds[s];
+                    double du[DIM];
+                    double r2 = kind_takes_sqrt_runtime(kind) ? 1e-300 : 0.0;
+#pragma unroll
+                    for (int k = 0; k < DIM; ++k) {                       // model_value's r2 chain, row minus column
+                        du[k] = ur[s * DIM + k] - uj[s][k];
+                        r2 = fma(du[k], du[k], r2);
+                    }
+                    double dk;
+                    const double kv = kern_value_deriv(kind, r2, a.betas[s], etab, dk);
+                    acc[4 * s] = fma(wt, kv, acc[4 * s]);
+                    const double g = wt * dk;
+#pragma unroll
+                    for (int k = 0; k < DIM; ++k) acc[4 * s + 1 + k] = fma(g, du[k] * du[k], acc[4 * s + 1 + k]);
+                }
+            }
+            if (i == j) acc[KG_SLOTS - 1] += wv;
+        }
+    }
+    const int warp = tid >> 5, lane = tid & 31;
+#pragma unroll
+    for (int q = 0; q < KG_SLOTS; ++q) {
+        double v = acc[q];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (lane == 0) red[warp][q] = v;
+    }
+    __syncthreads();
+    if (tid < KG_SLOTS) {
+        double v = 0.0;
+#pragma unroll
+        for (int w = 0; w < KG_COLS * KG_TY / 32; ++w) v += red[w][tid];
+        a.part[((int64_t)blockIdx.y * gridDim.x + blockIdx.x) * KG_SLOTS + tid] = v;
+    }
+}
+
+// out[slot] = sum over the nparts rows of part: lane l adds rows l, l + 32, .. in order, then a fixed xor tree
+__global__ void __launch_bounds__(32 * KG_SLOTS) kcov_grad_reduce_kernel(const double* __restrict__ part, int64_t nparts,
+                                                                         double* __restrict__ out) {
+    const int lane = threadIdx.x, slot = threadIdx.y;
+    double v = 0.0;
+    for (int64_t k = lane; k < nparts; k += 32) v += part[k * KG_SLOTS + slot];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) out[slot] = v;
+}
+
+int64_t kcov_grad(gsi_op* op, const double* Z, int64_t ldz, int64_t j0, int64_t w, double* part) {
+    gsi_ctx* ctx = op->ctx;
+    KcovGrad a;
+    std::memset(&a, 0, sizeof(a));
+    a.u = op->ucoords; a.n_pad = op->n_pad; a.n = op->n;
+    const bool model = op->kind == KC_KIND_MODEL;
+    a.nstruct = model ? op->nstruct : 1;
+    for (int s = 0; s < GSI_MODEL_MAX_STRUCTURES; ++s) {
+        a.kinds[s] = model ? op->mkinds[s] : op->kind;
+        a.betas[s] = model ? op->mbetas[s] : op->beta;
+    }
+    a.Z = Z; a.ldz = ldz; a.j0 = j0; a.w = w; a.part = part;
+    const int64_t rows = op->n - j0, cols = w < rows ? w : rows;
+    const dim3 grid((unsigned)((rows + KG_ROWS - 1) / KG_ROWS), (unsigned)((cols + KG_COLS - 1) / KG_COLS));
+    if (op->dim <= 2) kcov_grad_kernel<2><<<grid, dim3(KG_COLS, KG_TY), 0, ctx->stream>>>(a);
+    else kcov_grad_kernel<3><<<grid, dim3(KG_COLS, KG_TY), 0, ctx->stream>>>(a);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+    return (int64_t)grid.x * grid.y;
+}
+
+void kcov_grad_reduce(gsi_ctx* ctx, const double* part, int64_t nparts, double* out) {
+    kcov_grad_reduce_kernel<<<1, dim3(32, KG_SLOTS), 0, ctx->stream>>>(part, nparts, out);
+    GSI_CUDA(cudaGetLastError());
+    count_launch(ctx);
+}
+
 }  // namespace gsi

@@ -370,6 +370,30 @@ int32_t gsi_chol_krige_variance(gsi_chol* f, gsi_op* cross, const double* F_s, c
  * dependent drift columns at the sources: GSI_ERR_NOT_POSDEF.                                                          */
 int32_t gsi_chol_simulate(gsi_chol* f, int64_t ns, const double* y, const double* F_s, const double* F_t, int64_t p,
                           const gsi_buf* Xi, gsi_buf* Z);
+/* Gaussian log-likelihood of the covariance parameters of the square kernel-covariance operator op (any square operator
+ * of gsi_kernelcov_chol, one rank), with the drift coefficients profiled out by GLS, and optionally its exact gradient.
+ * A = C(S, S) + nugget I exactly as built, y the n observations, F the drift (host column-major n x p, 0 <= p <= 32; NULL
+ * iff p = 0), A = L L'.  With g = L^-1 y, G = L^-1 F, R'R = G'G (R upper triangular), beta = (G'G)^-1 G'g, e = g - G beta
+ * and q = ||e||^2:
+ *   reml = 0 (ML):    loglik = -1/2 (n log 2 pi + log det A + q)
+ *   reml = 1 (REML):  loglik = -1/2 ((n - p) log 2 pi + log det A + 2 sum_k log R_kk + q)
+ * The REML form leaves out log det F'F: its value depends on the scaling of F, its gradient and maximiser do not.
+ * beta_out (optional, p doubles) receives beta.  grad_out (optional) receives d loglik / d theta for the natural
+ * parameters, nstruct (1 + d) + 1 values: per structure s, sill_s then its principal-axis ranges range_(s,0 .. d-1), then
+ * the nugget (a single kind: nstruct = 1, sill = sigma2, ranges = ell).  Rotations and power-law exponents are held fixed.
+ * With alpha = A^-1 (y - F beta), H H' = A^-1 F (F'A^-1 F)^-1 F'A^-1 and W = alpha alpha' - A^-1 (+ H H' for REML),
+ * d loglik / d theta = 1/2 sum_ij W_ij dA_ij / dtheta (for ML the gradient of the profile likelihood).
+ * The call factors A, evaluates and frees the factor: the value costs the factor plus a few sweeps of width 128, the
+ * gradient about 2 n^3 / 3 more flops (A^-1 in chunks of 1024 columns, never held whole) and one contraction over the
+ * lower triangle.  Value and gradient are bit-reproducible run to run; the value does not depend on grad_out.
+ *   failed_column_out  optional: 0, or the 1-based column of the first non-positive pivot of A
+ * Errors: a non-positive pivot: GSI_ERR_NOT_POSDEF with *failed_column_out set; linearly dependent drift columns:
+ * GSI_ERR_NOT_POSDEF; a non-finite entry of y or F, p outside 0..32, F given with p = 0 or missing with p > 0, or REML with
+ * p >= n: GSI_ERR_INVALID_ARGUMENT; grad_out on a grid operator (lattice table), any operator gsi_kernelcov_chol refuses,
+ * or a call whose factor and work blocks do not fit the free device memory (checked before any allocation):
+ * GSI_ERR_UNSUPPORTED.                                                                                                 */
+int32_t gsi_kernelcov_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int32_t reml, double* loglik_out,
+                             double* beta_out, double* grad_out, int64_t* failed_column_out);
 
 /* FFTRF.powerlaw_structuredgrid (src/FFTRF.jl:83-100) for a batch of fields, on the device -- the
  * sampler behind getxis(samplefield, numfields, ...) (src/GeostatInversion.jl:29-38).  dim in {2, 3};

@@ -10,8 +10,9 @@
 #   getxis(Val{:iwantfields}, ...), pcgalsqr / pcgadirect / pcga / rga with the reference's
 #   positional and keyword arguments,
 # plus covsolve(C, B; rtol, maxiter, rank, seed), the dense factor covchol(C) with covchol_solve / covchol_logdet /
-# covchol_variance, krige(...; method = :cg | :cholesky, variance), covchol(C; diag), covchol_simulate and the
-# conditional / unconditional simulate(...) on the kernel-covariance operators (new),
+# covchol_variance, krige(...; method = :cg | :cholesky, variance), covchol(C; diag), covchol_simulate, the
+# conditional / unconditional simulate(...) and the likelihood covloglik(C, y; drift, reml, grad) on the kernel-covariance
+# operators (new),
 # for A::Matrix{Float64}, A::KernelCovMatrix (new), A::KernelCrossCovMatrix (new, not symmetric) and
 # A::LowRankCovMatrix, whose method set is
 # the one the reference's LowRankCovMatrix provides (src/lowrank.jl:38-60,115-139):
@@ -141,7 +142,8 @@ const MAXWIDECOLS = 1024
 abstract type Operator end
 # `rows` = this worker's block of global rows (all rows on a single-GPU context)
 mutable struct DenseOperator <: Operator; h::Ptr{Cvoid}; buf::DeviceMatrix; ctx::Context; rows::UnitRange{Int}; end
-mutable struct KernelCovMatrix <: Operator; h::Ptr{Cvoid}; n::Int; ctx::Context; rows::UnitRange{Int}; end
+# nparams: the length of the likelihood gradient (covloglik), nstruct (1 + d) + 1
+mutable struct KernelCovMatrix <: Operator; h::Ptr{Cvoid}; n::Int; ctx::Context; rows::UnitRange{Int}; nparams::Int; end
 mutable struct LowRankCovMatrix <: Operator; h::Ptr{Cvoid}; buf::DeviceMatrix; ctx::Context; rows::UnitRange{Int}; end
 # cross-covariance C(T, S): `rows` = this worker's block of target rows
 mutable struct KernelCrossCovMatrix <: Operator; h::Ptr{Cvoid}; n::Int; ctx::Context; rows::UnitRange{Int}; end
@@ -174,7 +176,7 @@ function KernelCovMatrix(kind::Integer, coords::Matrix{Float64}, ell::Vector{Flo
 	GC.@preserve coords ell check(ccall((:gsi_op_kernelcov, LIB), Int32,
 		(Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Float64}, Ptr{Float64}, Float64, Float64, Float64, Int64, Int64, Ref{Ptr{Cvoid}}),
 		ctx.h, kind, d, n, coords, ell, sigma2, nugget, beta, first(rows) - 1, length(rows), out))
-	op = KernelCovMatrix(out[], n, ctx, rows)
+	op = KernelCovMatrix(out[], n, ctx, rows, d + 2)
 	finalizer(freeop, op)
 	return op
 end
@@ -189,7 +191,7 @@ function KernelCovGrid(kind::Integer, dims::Vector{Int}, spacing::Vector{Float64
 	GC.@preserve dims64 spacing ell check(ccall((:gsi_op_kernelcov_grid, LIB), Int32,
 		(Ptr{Cvoid}, Int32, Int32, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Float64, Float64, Float64, Int64, Int64, Ref{Ptr{Cvoid}}),
 		ctx.h, kind, d, dims64, spacing, ell, sigma2, nugget, beta, first(rows) - 1, length(rows), out))
-	op = KernelCovMatrix(out[], n, ctx, rows)
+	op = KernelCovMatrix(out[], n, ctx, rows, d + 2)
 	finalizer(freeop, op)
 	return op
 end
@@ -209,7 +211,7 @@ function KernelCovModel(kinds::Vector{<:Integer}, sills::Vector{Float64}, ranges
 		(Ptr{Cvoid}, Int32, Int64, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
 		 Float64, Int64, Int64, Ref{Ptr{Cvoid}}),
 		ctx.h, d, n, coords, length(kinds32), kinds32, sills, ranges, rot, bet, nugget, first(rows) - 1, length(rows), out))
-	op = KernelCovMatrix(out[], n, ctx, rows)
+	op = KernelCovMatrix(out[], n, ctx, rows, length(kinds) * (1 + d) + 1)
 	finalizer(freeop, op)
 	return op
 end
@@ -230,7 +232,7 @@ function KernelCovModelGrid(kinds::Vector{<:Integer}, sills::Vector{Float64}, ra
 		(Ptr{Cvoid}, Int32, Ptr{Int64}, Ptr{Float64}, Int32, Ptr{Int32}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
 		 Float64, Int64, Int64, Ref{Ptr{Cvoid}}),
 		ctx.h, d, dims64, spacing, length(kinds32), kinds32, sills, ranges, rot, bet, nugget, first(rows) - 1, length(rows), out))
-	op = KernelCovMatrix(out[], n, ctx, rows)
+	op = KernelCovMatrix(out[], n, ctx, rows, length(kinds) * (1 + d) + 1)
 	finalizer(freeop, op)
 	return op
 end
@@ -500,6 +502,30 @@ function covchol_simulate(f::CovCholesky, Xi::VecOrMat{Float64}; ncond::Int=0, y
 		Z[:, cols] = download(Zd)
 	end
 	return Z
+end
+
+"""
+covloglik(C, y; drift=nothing, reml=false, grad=false) -> (value, beta) or (value, beta, gradient)
+
+Gaussian log-likelihood of the observations y under the square kernel-covariance operator C (nugget included), the
+drift coefficients profiled out by GLS (gsi_kernelcov_loglik; one dense factorisation on one GPU, about 8 n^2 bytes).
+drift = nothing, :constant or an n x p matrix F (p <= 32).  reml = false: -1/2 (n log 2 pi + log det C + q); reml = true:
+-1/2 ((n - p) log 2 pi + log det C + log det F'C^-1 F + q), without log det F'F; q the GLS residual quadratic form.  With
+grad = true the exact gradient for, per structure, the sill then the d ranges, and last the nugget (not on grid
+operators).  A non-positive pivot throws LinearAlgebra.PosDefException(column).
+"""
+function covloglik(C::KernelCovMatrix, y::Vector{Float64}; drift=nothing, reml::Bool=false, grad::Bool=false)
+	n = size(C, 2)
+	F = drift === nothing ? zeros(n, 0) : drift === :constant ? ones(n, 1) : Matrix{Float64}(drift)
+	p = size(F, 2)
+	val = Ref{Float64}(0.0)
+	col = Ref{Int64}(0)
+	beta = zeros(max(p, 1))
+	g = zeros(C.nparams)
+	GC.@preserve y F beta g check(ccall((:gsi_kernelcov_loglik, LIB), Int32,
+		(Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
+		C.h, y, p > 0 ? pointer(F) : C_NULL, p, Int32(reml), val, beta, grad ? pointer(g) : C_NULL, col))
+	return grad ? (val[], beta[1:p], g) : (val[], beta[1:p])
 end
 
 """

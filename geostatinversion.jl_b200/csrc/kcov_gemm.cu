@@ -1081,9 +1081,11 @@ void kcov_block(gsi_op* op, int side, const KcovBlock& b) {
 //   spherical    RN(RN(RN(-0.75 t) RN(1 + s)) / s), t = 1 - s (exact for s >= 0.5, 2^-53 below):
 //                0.5 + 0.5 + 0.5 + 0.5 + 0.5 + 2 c, c = 1 + s / (1 - s) + s / (1 + s)                        = 2.5 + 2 c
 // (c grows as s -> 1, where the derivative itself goes to 0 and its absolute error with it.)  Each summed term adds
-// the roundings of w W k' du^2 (3 products and one fma: < 2 units) to these.  The sums are not asserted entry by entry:
-// they cancel near the optimum (W = alpha alpha' - A^-1), so tests/test_gpu_kcov_lik.py bounds each gradient component
-// by 1e-9 S_theta, S_theta = 1/2 sum_ij |W_ij| |dA_ij / dtheta|, the conditioning of the sum.
+// the roundings of w W k' du^2 (3 products and one fma: < 2 units) to these.  The derivative bounds are asserted
+// argument by argument by tests/test_gpu_kcov_lik_exact.py::test_derivative_per_argument (one pair of points per call,
+// so each range component is a single term).  The full sums cancel near the optimum (W = alpha alpha' - A^-1), so
+// tests/test_gpu_kcov_lik.py bounds each gradient component by 1e-11 S_theta, S_theta = 1/2 sum_ij |W_ij| |dA_ij / dtheta|,
+// the conditioning of the sum.
 // Cost: one kern_eval-sized evaluation plus the derivative (one more FP64 multiply, a division for the exponential and
 // spherical kinds) and 2 + d FMAs per structure per entry: FP64-pipe bound, about 30 FP64 instructions per entry and
 // structure.  Every partial sum has a fixed order (thread: rows in order; warp: a fixed xor tree; CTA: warps in order;

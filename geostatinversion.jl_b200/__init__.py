@@ -15,7 +15,8 @@ from .core import (Context, DeviceMatrix, DenseMatrix, LowRankCovMatrix, KernelC
                    GridKernelCovModelMatrix, KernelCrossCovMatrix, GridKernelCrossCovMatrix)
 from . import randmatfact as RandMatFact
 from .randmatfact import randsvd, rangefinder, eig_nystrom
-from .kriging import cov_solve, krige, simulate, KernelCovCholesky, loglik, fit_covariance
+from .kriging import (cov_solve, krige, simulate, KernelCovCholesky, loglik, fit_covariance, cross_validate,
+                      CrossValidation)
 from . import dist
 from . import fftrf as FFTRF
 from .fftrf import PowerLawFieldSampler

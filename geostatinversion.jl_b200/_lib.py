@@ -101,6 +101,7 @@ SIGNATURES = {
     "gsi_kernelcov_chol_diag": (_i32, [_p, _pd, _pp, _pi64]),
     "gsi_chol_simulate": (_i32, [_p, _i64, _pd, _pd, _pd, _i64, _p, _p]),
     "gsi_kernelcov_loglik": (_i32, [_p, _pd, _pd, _i64, _i32, _pd, _pd, _pd, _pi64]),
+    "gsi_chol_crossval": (_i32, [_p, _pd, _pd, _i64, _i64, _pi64, _pi64, _pd, _pd, _pd, _pi64]),
     "gsi_fftrf_powerlaw": (_i32, [_p, _i32, _pi64, _f64, _f64, _f64, _p, _p]),
     "gsi_pcga_lowrank_matvec": (_i32, [_p, _i64, _i64, _pd, _i64, _pd, _pd, _pd, _i64, _pd, _pd]),
     "gsi_pcga_lsqr_solve": (_i32, [_p, _i64, _i64, _pd, _i64, _pd, _pd, _pd, _i64, _pd, _f64, _f64, _f64,

@@ -56,5 +56,11 @@ void chol_simulate(const gsi_chol* f, int64_t ns, const double* y, const double*
 // (grad_out: nstruct (1 + d) + 1 values); factors, evaluates and frees the factor
 void chol_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int reml, double* loglik, double* beta_out,
                  double* grad_out, int64_t* failed_column);
+// cross-validation of universal kriging on the factor: for each held-out group B (CSR group_ptr / group_idx; group_ptr
+// NULL: leave-one-out), err_B = P_BB^-1 (P y)_B, var_B = diag(P_BB^-1) and the log-density of y_B given the other points;
+// *failed_group: 1-based, 0 unless a P_BB is not positive definite
+void chol_crossval(const gsi_chol* f, const double* y, const double* F, int64_t p, int64_t ngroups,
+                   const int64_t* group_ptr, const int64_t* group_idx, double* err_out, double* var_out,
+                   double* logpdf_out, int64_t* failed_group);
 
 }  // namespace gsi

@@ -1118,3 +1118,14 @@ GSI_API int32_t gsi_kernelcov_loglik(gsi_op* op, const double* y, const double* 
         chol_loglik(op, y, F, p, reml, loglik_out, beta_out, grad_out, failed_column_out);
     });
 }
+
+GSI_API int32_t gsi_chol_crossval(gsi_chol* f, const double* y, const double* F, int64_t p, int64_t ngroups,
+                                  const int64_t* group_ptr, const int64_t* group_idx, double* err_out, double* var_out,
+                                  double* logpdf_out, int64_t* failed_group_out) {
+    if (failed_group_out) *failed_group_out = 0;
+    return guarded([&] {
+        GSI_REQUIRE(f && y && err_out && var_out, GSI_ERR_INVALID_ARGUMENT, "null argument");
+        use(f->ctx);
+        chol_crossval(f, y, F, p, ngroups, group_ptr, group_idx, err_out, var_out, logpdf_out, failed_group_out);
+    });
+}

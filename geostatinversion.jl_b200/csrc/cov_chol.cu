@@ -54,9 +54,17 @@
 // chol_gemm_kernel update, Z = A^-1 - [H alpha][H alpha]' = -W on rows >= j0, with K = p + 1 rounded up to 32: on the
 // tensor cores it costs about 2 n^2 K flops in all (1 ms at n = 20 000), where folding it into the contraction would add
 // 2 (p + 1) loads and p + 1 FMAs per entry to an FP64-pipe-bound kernel.  kcov_grad_kernel then contracts each chunk.
+//
+// Cross-validation (chol_crossval; Dubrule 1983).  With P = A^-1 - A^-1 F (F'A^-1 F)^-1 F'A^-1 = L^-T (I - G^ G^') L^-1,
+// G^ = G R^-1 (orthonormal columns), and alpha = P y = L^-T e, a held-out set B has err_B = P_BB^-1 alpha_B,
+// var_B = diag(P_BB^-1) and log p(y_B | y_-B) = -1/2 (alpha_B' err_B + |B| log 2 pi - log det P_BB).  The groups are packed
+// into chunks of <= 1024 columns; per chunk W = (I - G^ G^') L^-1 E_chunk (forward from the chunk's first block row, two
+// chol_gemm_kernel launches for the projection) and Q = W'W on chol_gemm_kernel, so P_BB = Q_BB is a Gram;
+// chol_cv_group_kernel factors each P_BB.
 #include "common.cuh"
 #include "algos.h"
 #include "ptx.cuh"
+#include <algorithm>
 #include <cmath>
 
 namespace gsi {
@@ -501,6 +509,120 @@ __global__ void chol_eye_kernel(double* __restrict__ Z, int64_t ldz, int64_t j0,
     if (c < w) Z[(j0 + c) * ldz + c] = 1.0;
 }
 
+// Z(cidx[c], c) = 1, c < w: the held-out points of a cross-validation chunk (row-major, pitch ldz; the rest was zeroed)
+__global__ void chol_cv_scatter_kernel(double* __restrict__ Z, int64_t ldz, const int64_t* __restrict__ cidx, int64_t w) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c < w) Z[cidx[c] * ldz + c] = 1.0;
+}
+
+// One held-out group of a cross-validation chunk: its points are the chunk columns col .. col + size - 1, in the caller's
+// order, and its results go to entries pos .. pos + size - 1 of the outputs and to entry g of the log-densities
+struct CvGroup {
+    int64_t pos;
+    int32_t size, col, g, pad;
+};
+constexpr int CV_THREADS = 128;
+// A pivot of P_BB at or below CV_PIVOT_TOL (A^-1)_jj counts as zero: the projection and the Gram leave an error of a few
+// units of roundoff times (A^-1)_jj on a pivot that is zero in exact arithmetic, and a group whose drift the remaining
+// points cannot identify has such a pivot
+constexpr double CV_PIVOT_TOL = 0x1p-36;
+
+// The groups of a chunk, SMAX = 32 (a warp per group of <= 32 points, four per CTA) or 128 (a CTA per group).  From the
+// chunk Gram Q = P(chunk, chunk) (lower triangle, row-major, pitch ldq), ref (the unprojected (A^-1)_jj of the chunk's
+// columns) and alpha (alpha_i at alpha[i * CH_B]): P_BB = L_B L_B' and X = L_B^-1 in shared memory (S[r * SP + c]: L
+// strictly below the diagonal, X transposed above it, dg the diagonal of L, rf its reciprocals), then with z = X alpha_B
+//   err = X' z = P_BB^-1 alpha_B,  var = the squared column norms of X = diag(P_BB^-1),
+//   logpdf = -1/2 (||z||^2 + size log 2 pi - 2 sum log dg)
+// Thread t of a team owns row t in the factorisation and column t of X; every sum runs in a fixed order, so a group's
+// results depend only on its own P_BB, alpha_B and ref.  A pivot at or below the tolerance records the 1-based group in
+// *failed (atomicMin: the lowest failing group wins whatever the launch order).
+template <int SMAX>
+__global__ void __launch_bounds__(CV_THREADS) chol_cv_group_kernel(const CvGroup* __restrict__ grp, int ng,
+                                                                   const double* __restrict__ Q, int64_t ldq,
+                                                                   const double* __restrict__ ref,
+                                                                   const int64_t* __restrict__ cidx,
+                                                                   const double* __restrict__ alpha,
+                                                                   double* __restrict__ err, double* __restrict__ var,
+                                                                   double* __restrict__ logpdf, int* __restrict__ failed) {
+    constexpr int TEAMS = CV_THREADS / SMAX, SP = SMAX + 1;
+    extern __shared__ __align__(16) double cv_smem[];
+    const int team = threadIdx.x / SMAX, t = threadIdx.x % SMAX;
+    const int gi = blockIdx.x * TEAMS + team;
+    if (gi >= ng) return;                                        // uniform over the team
+    auto bar = [] { if constexpr (SMAX == CV_THREADS) __syncthreads(); else __syncwarp(); };
+    double* S = cv_smem + (size_t)team * (SMAX * SP + 4 * SMAX);
+    double* dg = S + SMAX * SP;
+    double* a = dg + SMAX;
+    double* z = a + SMAX;
+    double* rf = z + SMAX;
+    const CvGroup G = grp[gi];
+    const int s = G.size;
+    for (int e = t; e < s * s; e += SMAX) {
+        const int r = e / s, c = e - r * s;
+        if (r >= c) S[r * SP + c] = Q[(int64_t)(G.col + r) * ldq + G.col + c];
+    }
+    if (t < s) {
+        a[t] = alpha[cidx[G.col + t] * CH_B];
+        rf[t] = ref[G.col + t];
+    }
+    bar();
+    for (int j = 0; j < s; ++j) {
+        const double d = S[j * SP + j];
+        if (!(d > CV_PIVOT_TOL * rf[j])) {                       // uniform: the team saw the same d and rf[j]
+            if (t == 0) atomicMin(failed, G.g + 1);
+            return;
+        }
+        const double sq = sqrt(d), rq = 1.0 / sq;
+        if (t > j && t < s) S[t * SP + j] *= rq;
+        bar();                                                   // every thread has also read rf[j]
+        if (t == j) {
+            dg[j] = sq;
+            rf[j] = rq;                                          // 1 / L(j, j) from here on
+        }
+        if (t > j && t < s) {
+            const double l = S[t * SP + j];
+            for (int c = j + 1; c <= t; ++c) S[t * SP + c] -= l * S[c * SP + j];
+        }
+        bar();
+    }
+    // column t of X: X(t, t) = 1 / L(t, t), X(i, t) = -(sum_{t <= k < i} L(i, k) X(k, t)) / L(i, i)
+    if (t < s) {
+        const double xt = rf[t];
+        double v = xt * xt;
+        for (int i = t + 1; i < s; ++i) {
+            double sum = S[i * SP + t] * xt;
+            for (int k = t + 1; k < i; ++k) sum = fma(S[i * SP + k], S[t * SP + k], sum);
+            const double x = -sum * rf[i];
+            S[t * SP + i] = x;
+            v = fma(x, x, v);
+        }
+        var[G.pos + t] = v;
+    }
+    bar();
+    if (t < s) {                                                  // z_t = sum_{j <= t} X(t, j) alpha_j
+        double zt = 0.0;
+        for (int j = 0; j < t; ++j) zt = fma(S[j * SP + t], a[j], zt);
+        z[t] = fma(a[t], rf[t], zt);
+    }
+    bar();
+    if (t < s) {                                                  // err_t = sum_{i >= t} X(i, t) z_i
+        double et = z[t] * rf[t];
+        for (int i = t + 1; i < s; ++i) et = fma(S[t * SP + i], z[i], et);
+        err[G.pos + t] = et;
+    }
+    if (logpdf && t == 0) {
+        double q = 0.0, ld = 0.0;
+        for (int i = 0; i < s; ++i) {
+            q = fma(z[i], z[i], q);
+            ld += log(dg[i]);
+        }
+        logpdf[G.g] = -0.5 * (q + s * 1.83787706640934548356 - 2.0 * ld);
+    }
+}
+
+template <int SMAX>
+constexpr size_t cv_group_smem() { return (size_t)(CV_THREADS / SMAX) * (SMAX * (SMAX + 1) + 4 * SMAX) * sizeof(double); }
+
 namespace {
 
 template <bool AK, bool BK, bool CR>
@@ -556,6 +678,50 @@ struct DevMem {
     ~DevMem() { if (p) cudaFree(p); }
     double* d() const { return static_cast<double*>(p); }
 };
+
+// The drift part of the likelihood and of cross-validation, enqueued without a synchronisation: [G | g] = L^-1 [F | y]
+// into W (row-major np x 128, zero padded; Wh is its host staging block and must live until the stream has passed the
+// copy), then with p > 0 GtG = [G | g]'[G | g], R'R = G'G (a failed factor sets flag[1]), beta and sum log R_kk into res
+// and chol_lik_resid_kernel in `mode`.  res must be zeroed by the caller
+void drift_residual(const gsi_chol* f, const double* y, const double* F, int64_t p, int mode, double* W, double* GtG,
+                    double* R, double* res, int* flag, std::vector<double>& Wh) {
+    gsi_ctx* ctx = f->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = f->n, np = f->np;
+    Wh.assign((size_t)np * CH_B, 0.0);
+    for (int64_t i = 0; i < n; ++i) {
+        for (int64_t q = 0; q < p; ++q) Wh[(size_t)i * CH_B + q] = F[q * n + i];
+        Wh[(size_t)i * CH_B + p] = y[i];
+    }
+    GSI_CUDA(cudaMemcpyAsync(W, Wh.data(), Wh.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    forward(f, W, CH_B, CH_B, np / CH_B);
+    GSI_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
+    if (p > 0) {
+        gemm<false, false, true>(ctx, gm(W, CH_B, W, CH_B, GtG, CH_B, np, 0, 0), 1, 1);
+        tall_head_to_cm_kernel<<<(unsigned)((p * p + 255) / 256), 256, 0, st>>>(GtG, CH_B, (int)p, R);
+        chol_upper_kernel<<<1, 1024, 0, st>>>(R, (int)p, flag + 1);
+        chol_lik_beta_kernel<<<1, 1, 0, st>>>(GtG, R, (int)p, res);
+        chol_lik_resid_kernel<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(W, np, (int)p, res, R, mode);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx, 4);
+    }
+}
+
+// device memory of a call that needs `need` bytes besides what it holds, checked before any allocation
+void require_free(gsi_ctx* ctx, double need, const char* what, int64_t n) {
+    size_t fr = 0, tot = 0;
+    GSI_CUDA(cudaMemGetInfo(&fr, &tot));
+    if (need > (double)fr) {
+        pool_release(ctx);
+        GSI_CUDA(cudaMemGetInfo(&fr, &tot));
+    }
+    if (need > (double)fr) {
+        char msg[256];
+        snprintf(msg, sizeof(msg), "%s: n = %lld needs %.0f bytes of device memory, %zu are free", what, (long long)n,
+                 need, fr);
+        throw Error(GSI_ERR_UNSUPPORTED, msg);
+    }
+}
 
 }  // namespace
 
@@ -906,18 +1072,7 @@ void chol_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int re
     const size_t small_doubles = (size_t)CH_B * CH_B + CH_MAX_DRIFT * CH_MAX_DRIFT + 2 * CH_MAX_DRIFT;
     double need = (double)np * np * 8.0 + (double)np * CH_B * 8.0 + 4096.0 + (double)np * CH_B * 8.0 + small_doubles * 8.0;
     if (want_grad) need += (double)np * ldz * 8.0 + (double)(max_parts + nchunks + 1) * KG_SLOTS * 8.0;
-    size_t fr = 0, tot = 0;
-    GSI_CUDA(cudaMemGetInfo(&fr, &tot));
-    if (need > (double)fr) {
-        pool_release(ctx);
-        GSI_CUDA(cudaMemGetInfo(&fr, &tot));
-    }
-    if (need > (double)fr) {
-        char msg[256];
-        snprintf(msg, sizeof(msg), "kernelcov_loglik: n = %lld needs %.0f bytes of device memory, %zu are free",
-                 (long long)n, need, fr);
-        throw Error(GSI_ERR_UNSUPPORTED, msg);
-    }
+    require_free(ctx, need, "kernelcov_loglik", n);
     std::unique_ptr<gsi_chol, void (*)(gsi_chol*)> f(chol_factor(op, nullptr, failed_column), chol_destroy);
     // value: [G | g] = L^-1 [F | y] (row-major np x 128, zero padded), beta, e, q
     DevMem W((size_t)np * CH_B * sizeof(double));
@@ -925,29 +1080,10 @@ void chol_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int re
     double* GtG = small.d();
     double* R = GtG + CH_B * CH_B;
     double* res = R + CH_MAX_DRIFT * CH_MAX_DRIFT;             // beta (p), log det R, q
-    {
-        std::vector<double> Wh((size_t)np * CH_B, 0.0);
-        for (int64_t i = 0; i < n; ++i) {
-            for (int64_t q = 0; q < p; ++q) Wh[(size_t)i * CH_B + q] = F[q * n + i];
-            Wh[(size_t)i * CH_B + p] = y[i];
-        }
-        GSI_CUDA(cudaMemcpyAsync(W.d(), Wh.data(), Wh.size() * sizeof(double), cudaMemcpyHostToDevice, st));
-        GSI_CUDA(cudaMemsetAsync(res, 0, 2 * CH_MAX_DRIFT * sizeof(double), st));
-        forward(f.get(), W.d(), CH_B, CH_B, nb);
-        GSI_CUDA(cudaStreamSynchronize(st));                   // Wh is freed on leaving the scope
-    }
     int* flag = f->flags;
-    GSI_CUDA(cudaMemsetAsync(flag, 0, 2 * sizeof(int), st));
-    if (p > 0) {
-        gemm<false, false, true>(ctx, gm(W.d(), CH_B, W.d(), CH_B, GtG, CH_B, np, 0, 0), 1, 1);
-        tall_head_to_cm_kernel<<<(unsigned)((p * p + 255) / 256), 256, 0, st>>>(GtG, CH_B, (int)p, R);
-        chol_upper_kernel<<<1, 1024, 0, st>>>(R, (int)p, flag + 1);
-        chol_lik_beta_kernel<<<1, 1, 0, st>>>(GtG, R, (int)p, res);
-        const int mode = !want_grad ? 0 : (reml ? 2 : 1);
-        chol_lik_resid_kernel<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(W.d(), np, (int)p, res, R, mode);
-        GSI_CUDA(cudaGetLastError());
-        count_launch(ctx, 4);
-    }
+    std::vector<double> Wh;
+    GSI_CUDA(cudaMemsetAsync(res, 0, 2 * CH_MAX_DRIFT * sizeof(double), st));
+    drift_residual(f.get(), y, F, p, !want_grad ? 0 : (reml ? 2 : 1), W.d(), GtG, R, res, flag, Wh);
     chol_lik_sumsq_kernel<<<1, 1024, 0, st>>>(W.d(), n, (int)p, res + CH_MAX_DRIFT + 1);
     GSI_CUDA(cudaGetLastError());
     count_launch(ctx);
@@ -1000,6 +1136,184 @@ void chol_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int re
         for (int a = 0; a < d; ++a) grad_out[s * (1 + d) + 1 + a] = -(sill / op->mranges[s][a]) * S[4 * s + 1 + a];
     }
     grad_out[ns * (1 + d)] = 0.5 * S[KG_SLOTS - 1];
+}
+
+void chol_crossval(const gsi_chol* f, const double* y, const double* F, int64_t p, int64_t ngroups,
+                   const int64_t* group_ptr, const int64_t* group_idx, double* err_out, double* var_out,
+                   double* logpdf_out, int64_t* failed_group) {
+    gsi_ctx* ctx = f->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = f->n, np = f->np, nb = np / CH_B;
+    if (failed_group) *failed_group = 0;
+    // ---- arguments, all on the host before any device work
+    GSI_REQUIRE(p >= 0 && p <= CH_MAX_DRIFT, GSI_ERR_INVALID_ARGUMENT, "chol_crossval: p must be in 0..32");
+    GSI_REQUIRE((p == 0) == (F == nullptr), GSI_ERR_INVALID_ARGUMENT, "chol_crossval: F must be given iff p > 0");
+    bool finite = true;
+    for (int64_t i = 0; i < n; ++i) finite = finite && std::isfinite(y[i]);
+    for (int64_t i = 0; i < n * p; ++i) finite = finite && std::isfinite(F[i]);
+    GSI_REQUIRE(finite, GSI_ERR_INVALID_ARGUMENT, "chol_crossval: y or F has a non-finite entry");
+    std::vector<int64_t> loo_ptr, loo_idx;
+    if (!group_ptr) {                                            // leave-one-out: n singletons in index order
+        GSI_REQUIRE(group_idx == nullptr && ngroups == n, GSI_ERR_INVALID_ARGUMENT,
+                    "chol_crossval: leave-one-out (group_ptr NULL) takes group_idx NULL and ngroups = n");
+        loo_ptr.resize(n + 1);
+        loo_idx.resize(n);
+        for (int64_t i = 0; i <= n; ++i) loo_ptr[i] = i;
+        for (int64_t i = 0; i < n; ++i) loo_idx[i] = i;
+        group_ptr = loo_ptr.data();
+        group_idx = loo_idx.data();
+    }
+    GSI_REQUIRE(ngroups >= 1 && ngroups <= n && group_idx != nullptr && group_ptr[0] == 0, GSI_ERR_INVALID_ARGUMENT,
+                "chol_crossval: the groups need 1 <= ngroups <= n, group_idx and group_ptr[0] = 0");
+    std::vector<char> seen(n, 0);
+    for (int64_t g = 0; g < ngroups; ++g) {
+        const int64_t s = group_ptr[g + 1] - group_ptr[g];
+        GSI_REQUIRE(s >= 1 && s <= CH_B, GSI_ERR_INVALID_ARGUMENT,
+                    "chol_crossval: group " + std::to_string(g) + " has " + std::to_string(s) +
+                        " points (group_ptr must increase by 1..128)");
+        for (int64_t k = group_ptr[g]; k < group_ptr[g + 1]; ++k) {
+            const int64_t i = group_idx[k];
+            GSI_REQUIRE(i >= 0 && i < n, GSI_ERR_INVALID_ARGUMENT,
+                        "chol_crossval: group " + std::to_string(g) + " has the point index " + std::to_string(i) +
+                            " outside 0 .. n - 1");
+            GSI_REQUIRE(!seen[i], GSI_ERR_INVALID_ARGUMENT,
+                        "chol_crossval: the point index " + std::to_string(i) + " is held out twice");
+            seen[i] = 1;
+        }
+    }
+    const int64_t m = group_ptr[ngroups];
+    // ---- chunks: the groups by their smallest index, packed whole into <= 1024 columns.  cidx: the point of every
+    // chunk column; desc: per chunk its groups of <= 32 points, then the larger ones
+    std::vector<int64_t> order(ngroups), gmin(ngroups);
+    for (int64_t g = 0; g < ngroups; ++g) {
+        order[g] = g;
+        gmin[g] = *std::min_element(group_idx + group_ptr[g], group_idx + group_ptr[g + 1]);
+    }
+    std::sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return gmin[a] < gmin[b]; });
+    struct Chunk { int64_t c0, w, kb0, d0, nsmall, nlarge; };
+    std::vector<Chunk> chunks;
+    std::vector<int64_t> cidx(m);
+    std::vector<CvGroup> desc(ngroups);
+    {
+        int64_t c0 = 0, gpos = 0;
+        for (int64_t k = 0; k < ngroups;) {
+            Chunk ch{c0, 0, gmin[order[k]] / CH_B, gpos, 0, 0};
+            int64_t k1 = k;
+            while (k1 < ngroups && ch.w + (group_ptr[order[k1] + 1] - group_ptr[order[k1]]) <= CH_MAX_CHUNK)
+                ch.w += group_ptr[order[k1] + 1] - group_ptr[order[k1]], ++k1;
+            for (int pass = 0; pass < 2; ++pass) {                 // small groups first, then the large ones
+                int64_t col = 0;
+                for (int64_t q = k; q < k1; ++q) {
+                    const int64_t g = order[q], s = group_ptr[g + 1] - group_ptr[g];
+                    if ((s > 32) == (pass == 1)) {
+                        desc[gpos++] = CvGroup{group_ptr[g], (int32_t)s, (int32_t)col, (int32_t)g, 0};
+                        (pass ? ch.nlarge : ch.nsmall) += 1;
+                    }
+                    if (pass == 0)
+                        for (int64_t r = 0; r < s; ++r) cidx[c0 + col + r] = group_idx[group_ptr[g] + r];
+                    col += s;
+                }
+            }
+            chunks.push_back(ch);
+            c0 += ch.w;
+            k = k1;
+        }
+    }
+    int64_t wmax = 0;
+    for (const Chunk& ch : chunks) wmax = std::max(wmax, ch.w);
+    const int64_t ld = round_up(wmax, CH_B);
+    // ---- device memory: [G^ | e] and its backward copy, the chunk block, its Gram and G^'W, the column norms, the
+    // drift scalars, the index and group tables, the outputs
+    const size_t small_doubles = (size_t)CH_B * CH_B + CH_MAX_DRIFT * CH_MAX_DRIFT + 2 * CH_MAX_DRIFT;
+    const size_t tail_doubles = (size_t)CS_PARTS_MAX * ld + ld + 2 * (size_t)m + (size_t)ngroups + 1;
+    const double need = 2.0 * np * CH_B * 8.0 + (double)np * ld * 8.0 + (double)ld * ld * 8.0 + (double)CH_B * ld * 8.0 +
+                        (double)(small_doubles + tail_doubles) * 8.0 + (double)m * 8.0 + (double)ngroups * sizeof(CvGroup);
+    require_free(ctx, need, "chol_crossval", n);
+    DevMem W((size_t)np * CH_B * sizeof(double)), Wa((size_t)np * CH_B * sizeof(double));
+    DevMem Z((size_t)np * ld * sizeof(double)), Q((size_t)ld * ld * sizeof(double)), H((size_t)CH_B * ld * sizeof(double));
+    DevMem small(small_doubles * sizeof(double)), tail(tail_doubles * sizeof(double));
+    DevMem cidx_d((size_t)m * sizeof(int64_t)), desc_d((size_t)ngroups * sizeof(CvGroup));
+    double* GtG = small.d();
+    double* R = GtG + CH_B * CH_B;
+    double* res = R + CH_MAX_DRIFT * CH_MAX_DRIFT;
+    double* part = tail.d();
+    double* colsq = part + (size_t)CS_PARTS_MAX * ld;
+    double* err = colsq + ld;
+    double* var = err + m;
+    double* lpd = var + m;
+    int* failed = reinterpret_cast<int*>(lpd + ngroups);
+    const int64_t* cidx_dev = static_cast<const int64_t*>(cidx_d.p);
+    const CvGroup* desc_dev = static_cast<const CvGroup*>(desc_d.p);
+    GSI_CUDA(cudaMemcpyAsync(cidx_d.p, cidx.data(), (size_t)m * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    GSI_CUDA(cudaMemcpyAsync(desc_d.p, desc.data(), (size_t)ngroups * sizeof(CvGroup), cudaMemcpyHostToDevice, st));
+    GSI_CUDA(cudaMemsetAsync(failed, 0x7f, sizeof(int), st));  // 0x7f7f7f7f: no group failed
+    // ---- 1. [G^ | e] = [G R^-1 | g - G beta] in W (kept for the projection), alpha = L^-T e from a copy
+    int* flag = f->flags;
+    std::vector<double> Wh;
+    GSI_CUDA(cudaMemsetAsync(res, 0, 2 * CH_MAX_DRIFT * sizeof(double), st));
+    drift_residual(f, y, F, p, 2, W.d(), GtG, R, res, flag, Wh);
+    int hf[2] = {0, 0};
+    GSI_CUDA(cudaMemcpyAsync(hf, flag, 2 * sizeof(int), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    if (hf[1] != 0)
+        throw Error(GSI_ERR_NOT_POSDEF, "chol_crossval: F' A^-1 F is not positive definite (the drift columns are "
+                                        "linearly dependent)");
+    GSI_CUDA(cudaMemcpyAsync(Wa.d(), W.d(), (size_t)np * CH_B * sizeof(double), cudaMemcpyDeviceToDevice, st));
+    backward(f, Wa.d(), CH_B, CH_B);
+    const double* alpha = Wa.d() + p;
+    // ---- 2. per chunk: W = (I - G^ G^') L^-1 E_chunk, Q = W'W, then the groups
+    const int64_t K = round_up(p, CH_K);
+    GSI_CUDA(cudaFuncSetAttribute(chol_cv_group_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)cv_group_smem<32>()));
+    GSI_CUDA(cudaFuncSetAttribute(chol_cv_group_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)cv_group_smem<128>()));
+    for (const Chunk& ch : chunks) {
+        const int64_t wp = round_up(ch.w, CH_B), mt = wp / CH_B;
+        // the whole block is zeroed: rows above kb0 stay exact zeros through the sweep, and the column norms and the
+        // projection read every row (a column's norm then has the same bits in every chunk: col_dot's row partition
+        // depends on the row count only).  The Gram of p = 0 skips those zero rows
+        const int64_t r0 = p > 0 ? 0 : ch.kb0 * CH_B;
+        GSI_CUDA(cudaMemsetAsync(Z.d(), 0, (size_t)np * ld * sizeof(double), st));
+        chol_cv_scatter_kernel<<<(unsigned)((ch.w + 255) / 256), 256, 0, st>>>(Z.d(), ld, cidx_dev + ch.c0, ch.w);
+        GSI_CUDA(cudaGetLastError());
+        count_launch(ctx);
+        forward(f, Z.d(), ld, wp, nb, ch.kb0);
+        col_dot(ctx, Z.d(), Z.d(), ld, n, ch.w, part, colsq, nullptr);   // (A^-1)_jj, the pivot scale
+        if (p > 0) {
+            gemm<false, false, true>(ctx, gm(W.d(), CH_B, Z.d(), ld, H.d(), ld, np, 0, 0), 1, mt);   // H = [G^ | e]' W
+            if (K > p) GSI_CUDA(cudaMemsetAsync(H.d() + p * ld, 0, (size_t)(K - p) * ld * sizeof(double), st));
+            gemm<true, false, true>(ctx, gm(W.d(), CH_B, H.d(), ld, Z.d(), ld, K, 1, 0), nb, mt);   // W -= G^ H
+        }
+        gemm<false, false, true>(ctx, gm(Z.d() + r0 * ld, ld, Z.d() + r0 * ld, ld, Q.d(), ld, np - r0, 0, 1), mt, mt);
+        const double* Qc = Q.d();
+        if (ch.nsmall > 0) {
+            chol_cv_group_kernel<32><<<(unsigned)((ch.nsmall + 3) / 4), CV_THREADS, cv_group_smem<32>(), st>>>(
+                desc_dev + ch.d0, (int)ch.nsmall, Qc, ld, colsq, cidx_dev + ch.c0, alpha, err, var,
+                logpdf_out ? lpd : nullptr, failed);
+            GSI_CUDA(cudaGetLastError());
+            count_launch(ctx);
+        }
+        if (ch.nlarge > 0) {
+            chol_cv_group_kernel<128><<<(unsigned)ch.nlarge, CV_THREADS, cv_group_smem<128>(), st>>>(
+                desc_dev + ch.d0 + ch.nsmall, (int)ch.nlarge, Qc, ld, colsq, cidx_dev + ch.c0, alpha, err, var,
+                logpdf_out ? lpd : nullptr, failed);
+            GSI_CUDA(cudaGetLastError());
+            count_launch(ctx);
+        }
+    }
+    int hfail = 0;
+    GSI_CUDA(cudaMemcpyAsync(&hfail, failed, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaMemcpyAsync(err_out, err, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaMemcpyAsync(var_out, var, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (logpdf_out)
+        GSI_CUDA(cudaMemcpyAsync(logpdf_out, lpd, (size_t)ngroups * sizeof(double), cudaMemcpyDeviceToHost, st));
+    GSI_CUDA(cudaStreamSynchronize(st));
+    if (hfail != 0x7f7f7f7f) {
+        if (failed_group) *failed_group = hfail;
+        throw Error(GSI_ERR_NOT_POSDEF, "chol_crossval: P_BB of group " + std::to_string(hfail) + " (1-based) is not "
+                                        "positive definite (the remaining points do not identify the drift, or the "
+                                        "block is numerically singular)");
+    }
 }
 
 }  // namespace gsi

@@ -4,8 +4,11 @@ iteration) or on a dense Cholesky factor (KernelCovCholesky, gsi_kernelcov_chol:
 solves, the kriging variance and log det A), and simple / ordinary / universal kriging in dual form on top of either;
 conditional and unconditional Gaussian simulation on the dense factor of the joint source-target covariance
 (simulate, gsi_chol_simulate); the ML / REML log-likelihood of the covariance parameters with its exact gradient
-(loglik, gsi_kernelcov_loglik) and maximum-likelihood fitting of a nested model on it (fit_covariance)."""
+(loglik, gsi_kernelcov_loglik) and maximum-likelihood fitting of a nested model on it (fit_covariance); leave-one-out
+and leave-group-out cross-validation on the dense factor (KernelCovCholesky.crossval, cross_validate, gsi_chol_crossval)."""
 import ctypes as C
+from collections import namedtuple
+
 import numpy as np
 
 from . import _lib
@@ -319,6 +322,69 @@ def fit_covariance(structures, sources, y, *, nugget, drift=None, reml=True, fit
     return sts, nug, info
 
 
+CrossValidation = namedtuple("CrossValidation", ["prediction", "error", "variance", "logpdf"])
+CrossValidation.__doc__ = """Cross-validation results: prediction, error = y - prediction and variance per point (n entries in
+point order, NaN at points not held out), logpdf per group (the Gaussian log-density of the group's values given the
+other points; their sum is the usual criterion for comparing models)."""
+
+
+def _groups_csr(groups, n):
+    """(ngroups, group_ptr, group_idx) of a sequence of index arrays; None: leave-one-out (NULL pointers)"""
+    if groups is None:
+        return n, None, None
+    sizes = [np.size(g) for g in groups]
+    ptr = np.zeros(len(sizes) + 1, dtype=np.int64)
+    ptr[1:] = np.cumsum(sizes)
+    idx = np.concatenate([np.asarray(g, dtype=np.int64).reshape(-1) for g in groups]) if sizes else np.zeros(0, np.int64)
+    return len(sizes), ptr, idx
+
+
+def cross_validate(structures, sources, y, *, nugget=0.0, drift=None, groups=None):
+    """Leave-one-out (groups=None) or leave-group-out cross-validation of kriging of y at the sources (d x n) under the
+    nested covariance model `structures` with observation noise `nugget` (a scalar, or n per-point values), drift None
+    (simple kriging), "constant" or an n x p array (universal kriging; the drift is re-estimated from the remaining
+    points for every group).  groups: a sequence of index arrays of 1..128 distinct points each.
+
+    Builds the covariance and its dense factor (about 8 n^2 bytes of device memory) and frees both.  The points are
+    ordered so that the held-out points come last, group by group: the sweeps then start at the held-out columns, so
+    cross-validating a few groups costs about one factorisation.  Returns a CrossValidation in the caller's point order
+    (KernelCovCholesky.crossval)."""
+    S = _f64_colmajor(sources)
+    n = S.shape[1]
+    yh = np.asarray(y, dtype=np.float64).reshape(n)
+    F = _drift_columns(drift, n)
+    if groups is None:
+        perm = np.arange(n)
+        pgroups = None
+    else:
+        gl = [np.asarray(g, dtype=np.int64).reshape(-1) for g in groups]
+        held = np.concatenate(gl) if gl else np.zeros(0, np.int64)
+        if held.size and (held.min() < 0 or held.max() >= n):
+            raise ValueError(f"cross_validate: a group index lies outside 0 .. {n - 1}")
+        if np.unique(held).size != held.size:
+            raise ValueError("cross_validate: a point is held out twice")
+        rest = np.setdiff1d(np.arange(n), held)
+        perm = np.concatenate([rest, held])
+        pgroups, k = [], rest.size
+        for g in gl:
+            pgroups.append(np.arange(k, k + g.size))
+            k += g.size
+    nug = np.asarray(nugget, dtype=np.float64)
+    per_point = nug.ndim > 0
+    A = KernelCovModelMatrix(structures, np.ascontiguousarray(S[:, perm]), 0.0 if per_point else float(nug))
+    fac = None
+    try:
+        fac = KernelCovCholesky(A, diag=nug.reshape(n)[perm] if per_point else None)
+        r = fac.crossval(yh[perm], drift=F[perm] if F.shape[1] else None, groups=pgroups)
+    finally:
+        if fac is not None:
+            fac.free()
+        A.free()
+    inv = np.empty(n, dtype=np.int64)
+    inv[perm] = np.arange(n)
+    return CrossValidation(r.prediction[inv], r.error[inv], r.variance[inv], r.logpdf)
+
+
 class KernelCovCholesky:
     """Dense Cholesky factor A = L L' of a square kernel-covariance operator A (KernelCovMatrix, GridKernelCovMatrix,
     KernelCovModelMatrix or GridKernelCovModelMatrix; exactly as built, nugget included), held on the device
@@ -444,6 +510,47 @@ class KernelCovCholesky:
                 if Zd is not None:
                     Zd.free()
         return Z
+
+    def crossval(self, y, *, drift=None, groups=None):
+        """Leave-one-out (groups=None) or leave-group-out cross-validation of kriging on this factor
+        (gsi_chol_crossval; Dubrule 1983): for every group B, the prediction of y_B from all other points with the
+        drift re-estimated by GLS from them (drift None: simple kriging, "constant" or an n x p array, p <= 32), its
+        error y_B - yhat_B, the error variance and the Gaussian log-density log p(y_B | y_-B).  groups: a sequence of
+        index arrays of 1..128 distinct points each; points in no group are not held out.
+
+        The variance is that of predicting the observation: the noise-free kriging variance plus the point's nugget
+        (or diag entry); the noise-free variance is variance - nugget_i.  Returns a CrossValidation with prediction,
+        error and variance in point order (NaN where not held out) and one logpdf per group.  A group whose drift the
+        remaining points cannot identify raises PosDefException with its 0-based index in `.group`."""
+        n = self.n
+        yh = np.ascontiguousarray(y, dtype=np.float64).reshape(-1)
+        if yh.size != n:
+            raise _lib.DimensionMismatch(_lib.ERR_DIMENSION_MISMATCH,
+                                         f"KernelCovCholesky.crossval: y has {yh.size} values, the factor is {n} x {n}")
+        F = _drift_columns(drift, n)
+        p = F.shape[1]
+        ng, ptr, idx = _groups_csr(groups, n)
+        m = n if ptr is None else int(ptr[-1])
+        err = np.empty(max(m, 1))
+        var = np.empty(max(m, 1))
+        lpd = np.empty(max(ng, 1))
+        failed = C.c_int64(0)
+        pi64 = C.POINTER(C.c_int64)
+        status = self._lib.gsi_chol_crossval(self._h, _pd(yh), _pd(F) if p else None, p, ng,
+                                             None if ptr is None else ptr.ctypes.data_as(pi64),
+                                             None if idx is None else idx.ctypes.data_as(pi64), _pd(err), _pd(var),
+                                             _pd(lpd), C.byref(failed))
+        try:
+            check(status)
+        except _lib.PosDefException as e:
+            e.group = int(failed.value) - 1 if failed.value else None
+            raise
+        points = np.arange(n) if idx is None else idx
+        out = [np.full(n, np.nan) for _ in range(3)]
+        out[1][points] = err[:m]
+        out[2][points] = var[:m]
+        out[0][points] = yh[points] - err[:m]
+        return CrossValidation(out[0], out[1], out[2], lpd[:ng])
 
     def free(self):
         if getattr(self, "_h", None) and self._h:

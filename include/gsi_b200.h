@@ -394,6 +394,31 @@ int32_t gsi_chol_simulate(gsi_chol* f, int64_t ns, const double* y, const double
  * GSI_ERR_UNSUPPORTED.                                                                                                 */
 int32_t gsi_kernelcov_loglik(gsi_op* op, const double* y, const double* F, int64_t p, int32_t reml, double* loglik_out,
                              double* beta_out, double* grad_out, int64_t* failed_column_out);
+/* Leave-one-out and leave-group-out cross-validation of kriging on a factor of gsi_kernelcov_chol or _chol_diag (a
+ * per-point diagonal is heteroscedastic noise and works as it is), Dubrule (1983).  y: the n observations; F: the drift
+ * (host column-major n x p, 0 <= p <= 32; NULL iff p = 0), re-estimated by GLS from the remaining points for every group
+ * (universal kriging as gsi_chol_krige_variance; p = 0: simple kriging).  With P = A^-1 - A^-1 F (F'A^-1 F)^-1 F'A^-1 and
+ * alpha = P y, for a held-out index set B:
+ *   err_B = y_B - yhat_B = P_BB^-1 alpha_B,   var_B = diag(P_BB^-1),
+ *   logpdf_B = log p(y_B | y_-B) = -1/2 (alpha_B' err_B + |B| log 2 pi - log det P_BB)
+ * var is the variance of predicting the OBSERVATION: the noise-free kriging variance plus the point's nugget (or diagonal
+ * entry).  Groups in CSR form: group g is group_idx[group_ptr[g] .. group_ptr[g + 1]), group_ptr[0] = 0, 1..128 points
+ * each, indices distinct and in 0..n-1; points in no group are never held out.  group_ptr = group_idx = NULL with
+ * ngroups = n is leave-one-out, the same as n singletons in index order.  err_out and var_out receive m = group_ptr[ngroups]
+ * values (n for leave-one-out) in group_idx order, logpdf_out (optional) one value per group.  Cost: about the forward
+ * sweep of a triangular inverse over the columns from the smallest held-out index on (n^3 / 3 flops for leave-one-out),
+ * plus a Gram of the held-out columns.  A group's results do not depend, bit for bit, on which other groups share the
+ * call or on their order, and they are bit-reproducible run to run.
+ *   failed_group_out  optional: 0, or the 1-based index of the lowest group whose P_BB is not positive definite
+ * Errors, before any device work: a malformed group list (group_ptr[0] != 0, a group of 0 or more than 128 points, an
+ * index out of range or held out twice, ngroups outside 1..n), p outside 0..32, F given with p = 0 or missing with p > 0,
+ * or a non-finite entry of y or F: GSI_ERR_INVALID_ARGUMENT.  Linearly dependent drift columns, or a P_BB that is not
+ * numerically positive definite (a pivot at or below 2^-36 (A^-1)_jj: the remaining points do not identify the drift, or
+ * the block is singular): GSI_ERR_NOT_POSDEF, the latter with *failed_group_out set.  Work blocks that do not fit the
+ * free device memory: GSI_ERR_UNSUPPORTED before any allocation, the message names the bytes needed.                  */
+int32_t gsi_chol_crossval(gsi_chol* f, const double* y, const double* F, int64_t p, int64_t ngroups,
+                          const int64_t* group_ptr, const int64_t* group_idx, double* err_out, double* var_out,
+                          double* logpdf_out, int64_t* failed_group_out);
 
 /* FFTRF.powerlaw_structuredgrid (src/FFTRF.jl:83-100) for a batch of fields, on the device -- the
  * sampler behind getxis(samplefield, numfields, ...) (src/GeostatInversion.jl:29-38).  dim in {2, 3};

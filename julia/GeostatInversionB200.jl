@@ -11,8 +11,8 @@
 #   positional and keyword arguments,
 # plus covsolve(C, B; rtol, maxiter, rank, seed), the dense factor covchol(C) with covchol_solve / covchol_logdet /
 # covchol_variance, krige(...; method = :cg | :cholesky, variance), covchol(C; diag), covchol_simulate, the
-# conditional / unconditional simulate(...) and the likelihood covloglik(C, y; drift, reml, grad) on the kernel-covariance
-# operators (new),
+# conditional / unconditional simulate(...), the likelihood covloglik(C, y; drift, reml, grad) and cross-validation
+# covchol_crossval(f, y; drift, groups) on the kernel-covariance operators (new),
 # for A::Matrix{Float64}, A::KernelCovMatrix (new), A::KernelCrossCovMatrix (new, not symmetric) and
 # A::LowRankCovMatrix, whose method set is
 # the one the reference's LowRankCovMatrix provides (src/lowrank.jl:38-60,115-139):
@@ -526,6 +526,43 @@ function covloglik(C::KernelCovMatrix, y::Vector{Float64}; drift=nothing, reml::
 		(Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Int32, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
 		C.h, y, p > 0 ? pointer(F) : C_NULL, p, Int32(reml), val, beta, grad ? pointer(g) : C_NULL, col))
 	return grad ? (val[], beta[1:p], g) : (val[], beta[1:p])
+end
+
+"""
+covchol_crossval(f, y; drift=nothing, groups=nothing) -> (prediction, error, variance, logpdf)
+
+Leave-one-out (groups = nothing) or leave-group-out cross-validation of kriging on the factor (gsi_chol_crossval,
+Dubrule 1983): for each group B (a vector of 1..128 distinct 1-based point indices) the prediction of y[B] from all
+other points, the drift (nothing, :constant or an n x p matrix, p <= 32) re-estimated by GLS from them, its error
+y[B] - prediction, the error variance of the observation (nugget included: the noise-free kriging variance is
+variance - nugget) and the Gaussian log-density of y[B] given the other points.  prediction, error and variance have n
+entries in point order, NaN at points not held out; logpdf one per group.  A group whose drift the other points cannot
+identify throws LinearAlgebra.PosDefException(group).
+"""
+function covchol_crossval(f::CovCholesky, y::Vector{Float64}; drift=nothing, groups=nothing)
+	n = f.n
+	length(y) == n || throw(DimensionMismatch("covchol_crossval: y has $(length(y)) values, the factor is $n x $n"))
+	F = drift === nothing ? zeros(n, 0) : drift === :constant ? ones(n, 1) : Matrix{Float64}(drift)
+	p = size(F, 2)
+	ng = groups === nothing ? n : length(groups)
+	ptr = groups === nothing ? Int64[] : vcat(0, cumsum(Int64[length(g) for g in groups]))
+	idx = groups === nothing ? Int64[] : Int64[i - 1 for g in groups for i in g]
+	m = groups === nothing ? n : Int(ptr[end])
+	err, var, lpd = zeros(max(m, 1)), zeros(max(m, 1)), zeros(max(ng, 1))
+	failed = Ref{Int64}(0)
+	status = GC.@preserve y F ptr idx err var lpd ccall((:gsi_chol_crossval, LIB), Int32,
+		(Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64},
+		 Ptr{Float64}, Ptr{Int64}),
+		f.h, y, p > 0 ? pointer(F) : C_NULL, p, ng, groups === nothing ? C_NULL : pointer(ptr),
+		groups === nothing ? C_NULL : pointer(idx), err, var, lpd, failed)
+	failed[] > 0 && throw(LinearAlgebra.PosDefException(Int(failed[])))
+	check(status)
+	pts = groups === nothing ? collect(1:n) : idx .+ 1
+	e, v = fill(NaN, n), fill(NaN, n)
+	e[pts] = err[1:m]
+	v[pts] = var[1:m]
+	pred = y .- e
+	return pred, e, v, lpd[1:ng]
 end
 
 """
